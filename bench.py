@@ -2,6 +2,7 @@
 """Benchmark of the posterior-sampling hot path (contract: task statement "Measurement").
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c5|c5h|c2|c3|c4|c3fit] [--impl native|reference]
+                    [--dump-outputs DIR]
 
 Default workload = BASELINE.json configs[4] / north_star target ("c5"): AMCMC, 10^5 chains TOTAL (sharded
 over the N GPUs: strong scaling), MLP 3->64->64->1 (P=4481), N=10^4 synthetic points, fp32.  A "step" is one
@@ -11,7 +12,9 @@ metric = chain-steps/s, whole job.  Other workloads are selectable for the recor
   c2  HMC(L=3) 1,024 chains, MLP 2->32->32->1, N=1,000            (chain-steps/s)
   c3  256-member ensemble predictive mean/var over 10^6 points, MLP 10->128->128->1   (member-points/s)
   c4  VI ELBO value+grad, 128 MC samples, same net, N=10^5        (MC-sample evals/s)
-One JSON line is printed by rank 0.
+One JSON line is printed by rank 0.  --dump-outputs DIR writes what the timed path computed in its last step to
+DIR/<name>.npy; inputs and random streams are seeded, so two builds run with the same arguments can be compared
+output for output.
 """
 import argparse
 import json
@@ -21,6 +24,8 @@ import subprocess
 import sys
 import threading
 import time
+
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree it runs from (it may be read-only)
 
 if 'reference' in sys.argv or any(a.startswith('--impl=ref') for a in sys.argv):
     # the reference arm uses every host thread; torchrun exports OMP_NUM_THREADS=1, which would also pin
@@ -373,7 +378,11 @@ def main():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-e2e', action='store_true')
     ap.add_argument('--no-extra', action='store_true', help='skip the c5h / c3 legs reported under "extra"')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the arrays the last timed step of the headline workload computed to DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     spec = workload_spec(args.workload)
     if args.chains:
         spec['K'] = args.chains
@@ -445,13 +454,25 @@ def run_native(spec, args, steps, warmup, rank, world, local, headline):
             recs[n] = ops.Recorder(st, n, store_every=0)
         units_per_step = spec['K']
         plan = prob.plan_info(Kloc, spec['sampler'] == 'hmc')
+        # what MCMCBase.run returns for the last step (quinn_b200/mcmc/mcmc.py), per chain.  The recorded MH ratio is
+        # unclipped and overflows to inf when a proposal is far more probable, so the acceptance probability
+        # min(1, ratio) that decides the step is written instead
+        outputs = lambda: (dict(theta=st.theta, mapparams=st.map_theta, maxpost=st.map_lp, naccept=st.naccept,   # noqa: E731
+                                logpost=recs[steps].logpost[:, -1], accept_prob=recs[steps].alpha[:, -1].clamp(max=1.0),
+                                accepted=recs[steps].accepted[:, -1]), {})
     elif spec['sampler'] == 'predict':
         # members stay whole on every rank; the 10^6 test points are sharded (no collective needed, SURVEY 8e)
         plo, phi = dist.shard_range(N, rank, world)
         xs = torch.as_tensor(x[plo:phi], dtype=dt, device=dev)
         th = torch.as_tensor(theta_init(spec, P, 0, spec['K']), device=dev)
         cnet = desc.to_c()
-        advance = lambda n: [ops.predict(desc, th, xs, dtype=dt, device=dev, want_out=False, want_moments=True, cnet=cnet) for _ in range(n)]  # noqa: E731
+        last = {}
+
+        def advance(n):
+            for _ in range(n):
+                last['moments'] = ops.predict(desc, th, xs, dtype=dt, device=dev, want_out=False, want_moments=True, cnet=cnet)[1:]
+        # predictive mean and variance per test point (points are sharded over ranks)
+        outputs = lambda: (dict(mean=last['moments'][0], var=last['moments'][1]), {})       # noqa: E731
         flop_per_unit, kernel_name = 2.0 * S, 'k_predict<float>'
         units_per_step = spec['K'] * N
         import ctypes as _C
@@ -472,6 +493,9 @@ def run_native(spec, args, steps, warmup, rank, world, local, headline):
             for _ in range(n):
                 trainer.epoch(epoch_no[0])
                 epoch_no[0] += 1
+        # what fit_members returns (quinn_b200/ens/batched.py), per member
+        outputs = lambda: (dict(theta=trainer.theta, best_theta=trainer.best_theta, best_loss=trainer.best_loss,     # noqa: E731
+                                loss=trainer.last_crit), {})
         F_fit = 6.0 * nsub * S - 2.0 * nsub * desc.layers[0].n_in * desc.layers[0].n_out
         flop_per_unit, kernel_name = F_fit, 'k_logpost_grad<float>'
         units_per_step = spec['K']
@@ -484,6 +508,7 @@ def run_native(spec, args, steps, warmup, rank, world, local, headline):
         rho = torch.full((P,), -4.5, dtype=dt, device=dev)
         B = N
         c_ssq = 0.5 * B / (Kloc * world * B) / spec['sigma'] ** 2
+        last = {}
 
         def advance(n):
             for i in range(n):
@@ -493,6 +518,10 @@ def run_native(spec, args, steps, warmup, rank, world, local, headline):
                 if world > 1:          # the MC samples are sharded over ranks: sum their gradient contributions (2P floats)
                     dist._allreduce(gmu)
                     dist._allreduce(grho)
+                last.update(logpost=lp, logq=logq, logprior=logp, grad_mu=gmu, grad_rho=grho)
+        # the ELBO terms per MC sample and the ELBO gradient with respect to the variational parameters
+        outputs = lambda: ({k: last[k] for k in ('logpost', 'logq', 'logprior')},                 # noqa: E731
+                           {k: last[k] for k in ('grad_mu', 'grad_rho')})
         flop_per_unit, kernel_name = F_vg, 'k_logpost_grad<float>'
         units_per_step = spec['K']
         plan = prob.plan_info(Kloc, True)
@@ -531,6 +560,11 @@ def run_native(spec, args, steps, warmup, rank, world, local, headline):
         if steps >= 2:
             lph = recs[steps].logpost
             diag['rhat_logpost'] = dist.rhat(lph.mean(1), lph.var(1, unbiased=True), steps).item()
+
+    if headline and args.dump_outputs:
+        per_unit, whole = outputs()
+        first, n_units = (plo, N) if spec['sampler'] == 'predict' else (lo, spec['K'])
+        dump_outputs(args.dump_outputs, per_unit, whole, n_units, first, rank)
 
     value = units_per_step * steps / (ms * 1e-3)
     units_local = Kloc if spec['sampler'] != 'predict' else spec['K'] * xs.shape[0]
@@ -623,6 +657,38 @@ def run_native(spec, args, steps, warmup, rank, world, local, headline):
                 cb = cpu_baseline(spec)
         line.update(clocks=clk, e2e=e2e, cpu_baseline=cb)
     return line if rank == 0 else None
+
+
+DUMP_BYTES = 60 * 10 ** 6          # array bytes of one dump; with the .npy headers the files stay under 64 MB
+
+
+def dump_outputs(path, per_unit, whole, n_units, first, rank):
+    """Write the outputs of the last timed step as path/<name>.npy, float64 where the device array is float64 or an
+    integer count, float32 otherwise.  per_unit: arrays whose first dimension is this rank's units (chains, members,
+    test points or MC samples), starting at global unit `first`; whole: arrays every rank holds in full.  When all units would
+    take more than DUMP_BYTES, a fixed seeded sample of them is written (the same units for any number of GPUs), with
+    its global indices as unit_index.npy."""
+    import torch
+    from quinn_b200 import dist
+    conv = lambda t: t.detach().double() if t.dtype in (torch.float64, torch.int64) else t.detach().float()   # noqa: E731
+    per_unit = {k: conv(t) for k, t in per_unit.items()}
+    whole = {k: conv(t) for k, t in whole.items()}
+    row_bytes = sum(math.prod(t.shape[1:]) * t.element_size() for t in per_unit.values())
+    room = DUMP_BYTES - sum(t.numel() * t.element_size() for t in whole.values())
+    keep = None
+    if n_units * row_bytes > room:
+        keep = np.sort(np.random.RandomState(0).choice(n_units, room // (row_bytes + 8), replace=False))
+        n_local = next(iter(per_unit.values())).shape[0]
+        rows = torch.as_tensor(keep[(keep >= first) & (keep < first + n_local)] - first)
+        per_unit = {k: t[rows.to(t.device)] for k, t in per_unit.items()}
+    per_unit = {k: dist.gather_to_rank0(t.contiguous()) for k, t in per_unit.items()}
+    if rank != 0:
+        return
+    os.makedirs(path, exist_ok=True)
+    for name, t in list(per_unit.items()) + list(whole.items()):
+        np.save(os.path.join(path, name + '.npy'), t.cpu().numpy())
+    if keep is not None:
+        np.save(os.path.join(path, 'unit_index.npy'), keep.astype(np.float64))
 
 
 def measured_traffic(spec, tc, units):
