@@ -259,7 +259,12 @@ int qb_fma_peak(int dtype, int variant, int64_t iters, double* flops_out_host, v
 /* Launch-plan introspection for DESIGN.md / bench.py: fills out[0..7] =
  * {tile points TM, threads per block, dynamic smem bytes, N-splits S, blocks, inplace flag,
  *  tensor-core path (0: CUDA-core kernel, 1: tcgen05 3xTF32, 2: same, software-pipelined, 3: tcgen05 gradient kernel (3xTF32),
- *  4: tcgen05 gradient kernel with fp16-split operands), tensor-memory columns}.
+ *  4: tcgen05 gradient kernel with fp16-split operands, 5: CUDA cores, weights streamed through shared memory),
+ *  tensor-memory columns}.
+ * Code 5 serves networks whose weights do not fit in shared memory next to one tile of activations (in fp64 from about
+ * 27 000 parameters): only activations stay resident and every layer's weights pass through a small shared-memory ring in
+ * chunks of output rows, in every entry point (kernels 1-4).  It is chosen only when the resident plan does not fit;
+ * a network whose activations of one tile (8 points in fp64, 16 in fp32) exceed 227 KB is refused.
  * The tensor-core VALUE path (qb_logpost, qb_amcmc_run, qb_predict) serves fp32 MLPs with <= 15 inputs, hidden widths
  * that are multiples of 16 (<= 128), <= 4 outputs and no residual layers; the tensor-core GRADIENT path
  * (qb_logpost_grad, qb_logpost_members, qb_hmc_run) serves fp32 MLPs in -> H -> H -> 1: tanh nets with H = 64 or 128 and

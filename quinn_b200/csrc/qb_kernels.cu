@@ -11,6 +11,7 @@
 #include "qb_plan.h"
 #include "qb_device.cuh"
 #include "qb_chain.cuh"
+#include "qb_stream.cuh"
 #include "qb_tc.cuh"
 #include "qb_value_tc3.h"
 #include "qb_grad_tc.h"
@@ -242,7 +243,123 @@ static long long plan_for_tm(const qb_net_t* net, int dtype, bool want_grad, int
     return P->smem_bytes;
 }
 
-struct QbLaunch { QbPlan plan; int S; long long pts_per_split; };
+// Layer-streamed plan (qb_stream.cuh) for tile size TM: fills `P`, returns its shared-memory bytes, or -1 when the
+// activations of one tile leave no room for a ring of chunks of TU rows per layer.
+static long long stream_plan_for_tm(const qb_net_t* net, int dtype, bool want_grad, int TM, QbStreamPlan* P) {
+    const int elem = dtype == QB_F64 ? 8 : 4;
+    const int TU = dtype == QB_F64 ? 4 : 8, TP = 4, VW = dtype == QB_F64 ? 2 : 4, PV = dtype == QB_F64 ? 2 : 4;
+    const int LDPAD = dtype == QB_F64 ? 2 : 4;
+    const int NT = QS_THREADS, nl = net->n_layers;
+    memset(P, 0, sizeof(*P));
+    P->n_layers = nl; P->in_dim = net->in_dim; P->out_dim = net->out_dim; P->n_params = net->n_params;
+    P->final_exp = net->final_exp; P->want_grad = want_grad ? 1 : 0;
+    P->TM = TM; P->lda = TM + LDPAD;
+    while ((TP << P->lg_pg) < TM) ++P->lg_pg;
+    int widest = net->in_dim, row = 0;
+    for (int l = 0; l < nl; ++l) {
+        const qb_layer_t& S = net->layers[l];
+        QbLayerPlan& L = P->L[l];
+        L.n_in = S.n_in; L.n_out = S.n_out; L.n_in_pad = rup(S.n_in, TU); L.n_out_pad = rup(S.n_out, TU);
+        L.w_off = S.w_off; L.b_off = S.b_off; L.act = S.act; L.res_step = S.res_step; L.has_res = S.res_step != 0.0;
+        L.n_terms = S.n_terms > 1 ? S.n_terms : 0; L.w_stride = S.w_stride; L.b_stride = S.b_stride;
+        for (int m = 0; m < QB_MAX_TERMS; ++m) L.coef[m] = S.coef[m];
+        L.wt_off = L.wr_off = L.bias_off = -1;
+        widest = std::max(widest, S.n_out);
+        L.row_in = row; row += S.n_in; L.row_out = row;
+        // weight-gradient split of qb_dw_accumulate (as in plan_for_tm)
+        const int patches = ((S.n_out + 3) / 4) * ((S.n_in + 3) / 4);
+        int C = 1;
+        while (C < 32 && patches * C * 2 <= NT && TM / (C * 2) >= PV) C *= 2;
+        L.dw_chunks = C; L.c_shift = 0;
+        while ((1 << L.c_shift) < C) ++L.c_shift;
+        L.ig_shift = -1;
+        for (int sft = 0; sft < 16; ++sft) if ((1 << sft) == (S.n_in + 3) / 4) L.ig_shift = sft;
+    }
+    row += net->layers[nl - 1].n_out;
+    P->buf_rows = widest; P->total_rows = row; P->da_rows = want_grad ? widest : 0;
+    const long long act_elems = want_grad ? (long long)(row + widest) * P->lda : 2LL * widest * P->lda;
+    const long long head = 384;          // 40 doubles of reduction scratch, then the ring's mbarriers
+    const long long avail = QB_SMEM_MAX - head - act_elems * elem;
+    if (avail <= 0) return -1;
+    const long long slot_max = avail / (QS_STAGES * elem) / 4 * 4;
+    long long slot = 0;
+    int c = 0;
+    for (int l = 0; l < nl; ++l) {
+        const QbLayerPlan& L = P->L[l];
+        QbStreamLayer& S = P->SL[l];
+        const int nterm = L.n_terms > 1 ? L.n_terms : 1;
+        S.ldw = rup(L.n_in, TU);
+        const long long rmax = slot_max / ((long long)nterm * S.ldw) / TU * TU;
+        if (rmax < TU) return -1;
+        int R = (int)std::min<long long>(rmax, rup(L.n_out, TU));
+        S.nch = (int)cdiv(L.n_out, R);
+        R = rup((int)cdiv(L.n_out, S.nch), TU);
+        S.R = R;
+        slot = std::max<long long>(slot, rup(nterm * R * S.ldw, 4));
+        const int nsub = (R / TU) * (TM / TP);
+        while (S.lg_ks < 5 && qs_items(nsub, S.lg_ks + 1) <= NT && (L.n_in >> (S.lg_ks + 1)) >= 2 * VW) ++S.lg_ks;
+        S.kl = rup((int)cdiv(L.n_in, 1 << S.lg_ks), VW);
+        const int nsub_b = (int)cdiv(L.n_in, TU) * (TM / TP);
+        while (S.lg_bks < 5 && qs_items(nsub_b, S.lg_bks + 1) <= NT && (R >> (S.lg_bks + 1)) >= 2) ++S.lg_bks;
+        S.bkl = (int)cdiv(R, 1 << S.lg_bks);
+        S.cp_dr = NT / L.n_in; S.cp_di = NT % L.n_in;
+        S.fwd_c0 = c; c += S.nch;
+        S.bwd_c0 = -1;
+    }
+    if (want_grad)
+        for (int l = nl - 1; l >= 1; --l) { P->SL[l].bwd_c0 = c; c += P->SL[l].nch; }
+    P->n_chunks = c;
+    P->slot_elems = (int)slot;
+    P->ring_off = (int)head;
+    P->act_off = P->ring_off + QS_STAGES * (int)slot * elem;
+    P->da_off = P->act_off + (want_grad ? row * P->lda * elem : 0);
+    P->act_elems = (int)act_elems;
+    P->smem_bytes = P->act_off + act_elems * elem;
+    return P->smem_bytes;
+}
+
+struct QbLaunch { QbPlan plan; int S; long long pts_per_split; bool streamed; QbStreamPlan sp; };
+
+// Networks whose weights do not fit next to one tile of activations: the layer-streamed kernels (qb_stream.cuh).
+// The tile is chosen so that the rows of one chunk times its points fill the thread tiles of the block with as little
+// split of the reduction as possible (larger tiles at equal fill: fewer passes of the weights through the ring).
+static int make_stream_launch(const qb_net_t* net, int dtype, bool want_grad, long long K, long long N, bool force_single,
+                              QbLaunch* out) {
+    const int TU = dtype == QB_F64 ? 4 : 8, TP = 4;
+    const int cands32[] = {128, 64, 32, 16}, cands64[] = {128, 64, 32, 16, 8};
+    const int* cands = dtype == QB_F64 ? cands64 : cands32;
+    const int nc = dtype == QB_F64 ? 5 : 4, mintm = cands[nc - 1];
+    const int cap = std::max(mintm, rup((int)std::min<long long>(N, 256), mintm));
+    QbStreamPlan tmp;
+    int pick = -1;
+    long long best = -1;
+    for (int c = 0; c < nc; ++c) {
+        const int TM = cands[c];
+        if (TM > cap) continue;
+        if (stream_plan_for_tm(net, dtype, want_grad, TM, &tmp) < 0) continue;
+        long long fill = (long long)QS_THREADS * TU * TP;
+        for (int l = 0; l < net->n_layers; ++l)
+            if (net->layers[l].n_out > TU) fill = std::min<long long>(fill, (long long)tmp.SL[l].R * TM);
+        if (fill > best) { best = fill; pick = TM; }
+    }
+    if (pick < 0)
+        return qb_fail("network too large for the layer-streamed path: the activations of one %s%lld-point tile exceed 227 KB of shared memory",
+                       "", mintm);
+    stream_plan_for_tm(net, dtype, want_grad, pick, &out->sp);
+    out->streamed = true;
+    const int TM = pick;
+    long long S = 1;
+    if (!force_single) {
+        // same rule as the resident kernels; with a gradient, the [K,S,P] partial rows stay under 256 MB
+        const long long target = (long long)QB_NUM_SMS * 8;
+        if (K < target) S = std::max<long long>(1, std::min(cdiv(N, 2LL * TM), cdiv(target, K)));
+        if (want_grad) S = std::min<long long>(S, std::max<long long>(1, (256LL << 20) / (K * net->n_params * (dtype == QB_F64 ? 8 : 4))));
+    }
+    long long pps = rup((int)cdiv(N, S), TM);
+    S = cdiv(N, pps);
+    out->S = (int)S; out->pts_per_split = pps;
+    return 0;
+}
 
 static int make_launch(const qb_net_t* net, int dtype, bool want_grad, long long K, long long N, bool force_single,
                        QbLaunch* out) {
@@ -287,7 +404,12 @@ static int make_launch(const qb_net_t* net, int dtype, bool want_grad, long long
             if (forced) break;
         }
     }
-    if (pick < 0) return qb_fail("network too large for the fused shared-memory path (weights + one tile exceed 227 KB)");
+    out->streamed = false;
+    if (pick < 0) {
+        if (forced) return qb_fail("network too large for the fused shared-memory path (weights + one tile exceed 227 KB)");
+        memset(&out->plan, 0, sizeof(out->plan));
+        return make_stream_launch(net, dtype, want_grad, K, N, force_single, out);
+    }
     plan_for_tm(net, dtype, want_grad, pick, &out->plan, wr_global);
     const int TM = out->plan.TM;
     long long S = 1;
@@ -424,6 +546,22 @@ __global__ void __launch_bounds__(256, 2) k_logpost_grad(const __grid_constant__
 }
 
 
+// kernels 1 and 2, layer-streamed (qb_stream.cuh): block b = chain b / S, split b % S, so the N-splits of one chain are
+// neighbours in launch order and read each weight chunk from L2 after the first of them brought it from HBM
+template <typename T, bool GRAD>
+__global__ void __launch_bounds__(QS_THREADS, 1) k_logpost_stream(const __grid_constant__ QbStreamPlan P, const EvalArgs<T> a) {
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    QsRing rg;
+    qs_ring_init(P, smem_raw, rg);
+    const long long b = blockIdx.x, k = b / a.S, s = b - k * a.S;
+    const long long n0 = s * a.pps, n1 = min(a.N, n0 + a.pps);
+    T* g = nullptr;
+    if (GRAD) g = (a.S == 1) ? a.grad + k * P.n_params : a.gpart + (k * a.S + s) * P.n_params;
+    const double ssq = qs_eval<T, GRAD>(P, smem_raw, rg, a.theta + k * P.n_params, a.x + k * a.xs, a.y + k * a.ys, n0, n1,
+                                        a.lk.inv_sigma2, g, nullptr);
+    if (threadIdx.x == 0) a.part[k * a.S + s] = ssq;
+}
+
 // kernel 1 on the tensor cores (fp32 eligible networks, see qb_tc.cuh)
 __global__ void __launch_bounds__(512, 1) k_logpost_tc(const __grid_constant__ QbTcPlan tp, const EvalArgs<float> a) {
     extern __shared__ __align__(128) unsigned char smem_tc[];
@@ -530,7 +668,16 @@ static int run_eval(const qb_net_t* net, int dtype, const void* theta, int64_t K
     a.lp = lp; a.lk = lik_dev(lik);
     a.xsplit = nullptr;
     dim3 grid((unsigned)K, (unsigned)L.S);
-    if (want_grad) {
+    if (L.streamed) {
+        const dim3 sgrid((unsigned)(K * L.S));
+        if (want_grad) {
+            if (set_smem(k_logpost_stream<T, true>, L.sp.smem_bytes)) return -2;
+            k_logpost_stream<T, true><<<sgrid, QS_THREADS, L.sp.smem_bytes, st>>>(L.sp, a);
+        } else {
+            if (set_smem(k_logpost_stream<T, false>, L.sp.smem_bytes)) return -2;
+            k_logpost_stream<T, false><<<sgrid, QS_THREADS, L.sp.smem_bytes, st>>>(L.sp, a);
+        }
+    } else if (want_grad) {
         QbTcgPlan tg;
         QbTg8Plan t8;
         if (qb_tg8_make_plan(net, dtype, &t8)) {
@@ -573,6 +720,7 @@ extern "C" size_t qb_eval_workspace_bytes(const qb_net_t* net, int dtype, int64_
     if (make_launch(net, dtype, want_grad != 0, K, N, false, &L)) return 0;
     size_t b = ((size_t)K * L.S * sizeof(double) + 255) / 256 * 256;
     if (want_grad && L.S > 1) b += (size_t)K * L.S * net->n_params * (dtype == QB_F64 ? 8 : 4);
+    if (L.streamed) return b;
     QbTcPlan tp;
     if (!want_grad && make_tc_plan(net, dtype, &tp, 1) && tp.v3) b = (b + 255) / 256 * 256 + qb_tc3_xsplit_bytes(N, tp.v3 == 1 ? 8 : 16);
     QbTcgPlan tg;
@@ -587,6 +735,11 @@ extern "C" int qb_plan_info(const qb_net_t* net, int dtype, int64_t K, int64_t N
     if (make_launch(net, dtype, want_grad != 0, K, N, false, &L)) return -1;
     out[0] = L.plan.TM; out[1] = L.plan.nthreads; out[2] = L.plan.smem_bytes; out[3] = L.S;
     out[4] = (int64_t)K * L.S; out[5] = L.plan.inplace; out[6] = 0; out[7] = 0;
+    if (L.streamed) {
+        // CUDA cores, weights streamed through shared memory (qb_stream.cuh): out[6] = 5
+        out[0] = L.sp.TM; out[1] = QS_THREADS; out[2] = L.sp.smem_bytes; out[5] = 0; out[6] = 5;
+        return 0;
+    }
     QbTcgPlan tg;
     QbTg8Plan t8;
     if (want_grad && qb_tg8_make_plan(net, dtype, &t8)) {
@@ -880,6 +1033,32 @@ k_amcmc(const __grid_constant__ QbPlan plan, const __grid_constant__ QbTcPlan tp
     if constexpr (TC) qb_tc_fini(tp, cx);
 }
 
+// kernel 3 (AMCMC), layer-streamed: one block per chain, the proposal pass uses the activation area as scratch
+template <typename T>
+__global__ void __launch_bounds__(QS_THREADS, 1)
+k_amcmc_stream(const __grid_constant__ QbStreamPlan P, const __grid_constant__ ChainArgs<T> c, const __grid_constant__ AmcmcArgs<T> a) {
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    QsRing rg;
+    qs_ring_init(P, smem_raw, rg);
+    double* red = reinterpret_cast<double*>(smem_raw);
+    T* zbuf = reinterpret_cast<T*>(smem_raw + P.act_off);
+    const long long k = blockIdx.x;
+    const int np = P.n_params;
+    QbAmcmcLocal st;
+    st.lp_cur = 0.0; st.map_lp = 0.0; st.na = 0;
+    if (!c.init_lp) { st.lp_cur = c.lp[k]; st.map_lp = c.map_lp[k]; st.na = c.naccept[k]; }
+    st.kind = a.prop_kind[k];
+    __syncthreads();
+    for (long long s = c.init_lp ? -1 : 0; s < c.nsteps; ++s) {
+        const T* evalp = (s < 0 ? c.theta : a.prop) + k * np;
+        if (s >= 0) qb_amcmc_pre<T>(c, a, np, k, s, st.kind, zbuf);
+        else __syncthreads();
+        const double ssq = qs_eval<T, false>(P, smem_raw, rg, evalp, c.x, c.y, 0, c.N, 0.0, nullptr, nullptr);
+        qb_amcmc_post<T>(c, a, np, k, s, ssq, red, st);
+    }
+    if (threadIdx.x == 0) { c.lp[k] = st.lp_cur; c.map_lp[k] = st.map_lp; c.naccept[k] = st.na; a.prop_kind[k] = st.kind; }
+}
+
 template <typename T> static int launch_amcmc_tc(const QbPlan&, const QbTcPlan&, const ChainArgs<T>&, const AmcmcArgs<T>&, long long, cudaStream_t) {
     return qb_fail("tensor-core path is fp32 only");
 }
@@ -911,6 +1090,31 @@ __global__ void __launch_bounds__(256, 2) k_hmc(const __grid_constant__ QbPlan p
     qb_hmc_body<T>(c, h, plan.n_params, S.red, eval);
 }
 
+// HMC / MALA, layer-streamed: the evaluation functor of qb_hmc_body (value + gradient + prior, as qb_full_grad)
+template <typename T> struct QbGradStream {
+    const QbStreamPlan& P; unsigned char* smem; QsRing& rg; const ChainArgs<T>& c; long long k;
+    __device__ __forceinline__ double operator()(const T* th, T* g) const {
+        const double ssq = qs_eval<T, true>(P, smem, rg, th, c.x, c.y, 0, c.N, c.lk.inv_sigma2, g, nullptr);
+        double* red = reinterpret_cast<double*>(smem);
+        double pss = 0.0;
+        if (c.lk.has_prior) {
+            pss = qb_prior_ss<T>(c.lk, th, k, P.n_params, red);
+            qb_prior_grad_add<T>(c.lk, th, k, P.n_params, g);
+        }
+        __syncthreads();
+        return qb_lp_from(c.lk, ssq, c.N, pss, P.n_params);
+    }
+};
+
+template <typename T>
+__global__ void __launch_bounds__(QS_THREADS, 1) k_hmc_stream(const __grid_constant__ QbStreamPlan P, const ChainArgs<T> c, const HmcArgs<T> h) {
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    QsRing rg;
+    qs_ring_init(P, smem_raw, rg);
+    QbGradStream<T> eval{P, smem_raw, rg, c, (long long)blockIdx.x};
+    qb_hmc_body<T>(c, h, P.n_params, reinterpret_cast<double*>(smem_raw), eval);
+}
+
 template <typename T>
 static void fill_chain_args(ChainArgs<T>& c, const qb_data_t* data, const qb_lik_t* lik, const qb_chain_t* ch,
                             const qb_rng_t* rng, const qb_record_t* rec, int64_t t_start, int64_t nsteps, int init_lp) {
@@ -939,7 +1143,7 @@ static int run_amcmc(const qb_net_t* net, int dtype, const qb_data_t* data, cons
     if (make_launch(net, dtype, false, ch->K, data->n, true, &L)) return -1;
     const int P = net->n_params;
     if (am->adapt == QB_ADAPT_FULL || am->chol_ini) {
-        const long long act_elems = (L.plan.smem_bytes - 40 * 8) / L.plan.elem_size - L.plan.w_elems;
+        const long long act_elems = L.streamed ? L.sp.act_elems : (L.plan.smem_bytes - 40 * 8) / L.plan.elem_size - L.plan.w_elems;
         if (P > act_elems) return qb_fail("full-covariance proposals need P <= tile scratch%s (P=%lld)", "", P);
     }
     ChainArgs<T> c; fill_chain_args<T>(c, data, lik, ch, rng, rec, t_start, nsteps, init_lp);
@@ -957,8 +1161,11 @@ static int run_amcmc(const qb_net_t* net, int dtype, const qb_data_t* data, cons
     if (am->adapt == QB_ADAPT_FULL && !a.chol) return qb_fail("full adaptation needs chol");
     if (!a.pscale || !a.prop_kind || !a.prop) return qb_fail("amcmc needs pscale, prop_kind and scratch");
     QbTcPlan tp;
-    const bool tc = am->adapt != QB_ADAPT_FULL && !am->chol_ini && make_tc_plan(net, dtype, &tp, 2);
-    if (tc) {
+    const bool tc = !L.streamed && am->adapt != QB_ADAPT_FULL && !am->chol_ini && make_tc_plan(net, dtype, &tp, 2);
+    if (L.streamed) {
+        if (set_smem(k_amcmc_stream<T>, L.sp.smem_bytes)) return -2;
+        k_amcmc_stream<T><<<(unsigned)ch->K, QS_THREADS, L.sp.smem_bytes, st>>>(L.sp, c, a);
+    } else if (tc) {
         if (launch_amcmc_tc<T>(L.plan, tp, c, a, ch->K, st)) return -2;
     } else {
         memset(&tp, 0, sizeof(tp));
@@ -992,7 +1199,10 @@ static int run_hmc(const qb_net_t* net, int dtype, const qb_data_t* data, const 
     h.gcur = (T*)hm->grad_cur; h.mom = (T*)hm->mom; h.prop = (T*)hm->prop; h.gprop = (T*)hm->grad_prop;
     QbTcgPlan tg;
     QbTg8Plan t8;
-    if (qb_tg8_make_plan(net, dtype, &t8)) {
+    if (L.streamed) {
+        if (set_smem(k_hmc_stream<T>, L.sp.smem_bytes)) return -2;
+        k_hmc_stream<T><<<(unsigned)ch->K, QS_THREADS, L.sp.smem_bytes, st>>>(L.sp, c, h);
+    } else if (qb_tg8_make_plan(net, dtype, &t8)) {
         if (launch_hmc_tc128<T>(t8, c, h, ch->K, st)) return -2;
         g_launches += 1;
     } else if (qb_tcg_make_plan(net, dtype, &tg)) {
@@ -1117,6 +1327,19 @@ __global__ void __launch_bounds__(512, 1) k_predict(const __grid_constant__ QbPl
     }
 }
 
+// kernel 4, layer-streamed: block b = member b / chunks, tile chunk b % chunks (a member's chunks are neighbours)
+template <typename T>
+__global__ void __launch_bounds__(QS_THREADS, 1) k_predict_stream(const __grid_constant__ QbStreamPlan P, const PredArgs<T> a,
+                                                                 long long chunks) {
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    QsRing rg;
+    qs_ring_init(P, smem_raw, rg);
+    const long long b = blockIdx.x, m = b / chunks, ch = b - m * chunks;
+    const long long n0 = ch * a.tiles_per_block * P.TM, n1 = min(a.N, n0 + a.tiles_per_block * P.TM);
+    qs_eval<T, false>(P, smem_raw, rg, a.theta + m * P.n_params, a.x, nullptr, n0, n1, 0.0, nullptr,
+                      a.out + m * a.N * P.out_dim);
+}
+
 // mean / var(ddof=1) over the leading axis of out[M, n]  (HBM-bound, coalesced over n)
 template <typename T>
 __global__ void k_moments(const T* out, long long M, long long n, T* mean, T* var) {
@@ -1161,6 +1384,28 @@ static int run_predict(const qb_net_t* net, int dtype, const void* theta, int64_
                        void* out, void* mean, void* var, cudaStream_t st) {
     QbLaunch L;
     if (make_launch(net, dtype, false, M, N, true, &L)) return -1;
+    if (L.streamed) {
+        const QbStreamPlan& SP = L.sp;
+        if (!out) return qb_fail("moments without `out` need TM*out_dim <= 4*threads; pass an `out` buffer");
+        PredArgs<T> a;
+        a.theta = (const T*)theta; a.x = (const T*)x; a.M = M; a.N = N;
+        a.out = (T*)out; a.mean = (T*)mean; a.var = (T*)var; a.fused = 0;
+        const long long tiles = cdiv(N, SP.TM);
+        long long chunks = std::max<long long>(1, std::min<long long>(tiles, cdiv((long long)QB_NUM_SMS * 2, M)));
+        a.tiles_per_block = cdiv(tiles, chunks);
+        chunks = cdiv(tiles, a.tiles_per_block);
+        if (set_smem(k_predict_stream<T>, SP.smem_bytes)) return -2;
+        k_predict_stream<T><<<(unsigned)(M * chunks), QS_THREADS, SP.smem_bytes, st>>>(SP, a, chunks);
+        QB_CUDA(cudaGetLastError());
+        g_launches += 1;
+        if (mean || var) {
+            const long long n = N * SP.out_dim;
+            k_moments<T><<<(unsigned)cdiv(n, 256), 256, 0, st>>>((const T*)out, M, n, (T*)mean, (T*)var);
+            QB_CUDA(cudaGetLastError());
+            g_launches += 1;
+        }
+        return 0;
+    }
     const QbPlan& P = L.plan;
     const long long tiles = cdiv(N, P.TM);
     const bool want_mom = mean || var;
