@@ -1,8 +1,8 @@
 #!/usr/bin/env python
-"""The reference's examples/ex_ufit.py workflow (methods amcmc / hmc / ens / vi) with quinn_b200 as a drop-in:
+"""The reference's examples/ex_ufit.py workflow (methods amcmc / hmc / ens / vi / laplace) with quinn_b200 as a drop-in:
 only the imports change.  Plotting is out of scope, so the script prints predictive moments instead.
 
-    python examples/ex_ufit_b200.py amcmc|hmc|ens|vi [nchains]
+    python examples/ex_ufit_b200.py amcmc|hmc|ens|vi|laplace [nchains]
 """
 import os
 import sys
@@ -11,7 +11,7 @@ import numpy as np
 import torch
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-from quinn_b200.solvers import NN_MCMC, NN_Ens, NN_VI      # noqa: E402  (reference: from quinn.solvers.nn_mcmc import NN_MCMC ...)
+from quinn_b200.solvers import NN_MCMC, NN_Ens, NN_VI, NN_Laplace      # noqa: E402  (reference: from quinn.solvers.nn_mcmc import NN_MCMC ...)
 from quinn_b200.nns import RNet, Poly                      # noqa: E402  (reference: from quinn.nns.rnet import RNet, Poly)
 
 
@@ -41,8 +41,12 @@ def main():
     elif meth == 'ens':
         uqnet = NN_Ens(nnet, nens=3, dfrac=0.8, verbose=True)
         uqnet.fit(xtrn, ytrn, val=[xval, yval], lrate=0.01, batch_size=2, nepochs=300)
+    elif meth == 'laplace':
+        uqnet = NN_Laplace(nnet, nens=3, la_type='full', cov_scale=1.0, datanoise=datanoise, priorsigma=1.0, dfrac=0.8,
+                           verbose=True)
+        uqnet.fit(xtrn, ytrn, val=[xval, yval], lrate=0.01, batch_size=2, nepochs=300)
     else:
-        raise SystemExit('pick among amcmc, hmc, vi, ens')
+        raise SystemExit('pick among amcmc, hmc, vi, ens, laplace')
     xgrid = np.linspace(-np.pi, np.pi, 11)[:, None]
     nsam = 3 if meth == 'ens' else 1000
     mean, var, _ = uqnet.predict_mom_sample(xgrid, msc=1, nsam=nsam)

@@ -107,6 +107,20 @@ int qb_logpost_grad(const qb_net_t* net, int dtype, const void* theta, int64_t K
                     const qb_lik_t* lik, double* lp, void* grad, void* workspace, size_t workspace_bytes,
                     void* stream);
 
+/* Kernel 5.  hv[k,:] = (d^2 lp / d theta^2) v_k at one theta[P] (lp exactly as qb_logpost_grad) for K directions.
+ * v: [K,P] dtype, or NULL for the unit directions v_k = e_{col0+k} (rows col0 .. col0+K-1 of the Hessian).
+ * Replaces NNWrap.calc_hess_full (quinn/nns/nnwrap.py:153-203).  lik->anchor_per_chain must be 0.  K == 0 does nothing.
+ * A network whose weights, one direction and the smallest tile of activations and tangents (16 points in fp32, 8 in
+ * fp64) exceed 227 KB of shared memory is refused; it is not streamed.  hv: [K,P] dtype.  Deterministic: fp64 results
+ * are bit-identical run to run. */
+size_t qb_hvp_workspace_bytes(const qb_net_t* net, int dtype, int64_t K, int64_t N);
+int qb_logpost_hvp(const qb_net_t* net, int dtype, const void* theta, const void* v, int64_t col0, int64_t K,
+                   const qb_data_t* data, const qb_lik_t* lik, void* hv, void* workspace, size_t workspace_bytes,
+                   void* stream);
+/* Launch plan of kernel 5 for K directions over N points: out[0..4] = {tile points TM, threads per block, dynamic smem
+ * bytes, N-splits S, blocks}.  Returns -1 (with qb_last_error) for a network kernel 5 refuses. */
+int qb_hvp_plan_info(const qb_net_t* net, int dtype, int64_t K, int64_t N, int64_t* out);
+
 /* ---- Batched ensemble training (SURVEY.md 8f rank 1) --------------------------------------------
  * NN_Ens.fit (quinn/solvers/nn_ens.py:51-69) trains nens members one after the other, each with
  * Learner.fit -> nnfit (quinn/ens/learner.py:59-73, quinn/nns/nnfit.py:125-166: minibatch loop, torch Adam, best

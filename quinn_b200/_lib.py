@@ -80,6 +80,10 @@ SYMBOLS = {
                                   C.POINTER(qb_lik_t), _P, _P, _P, C.c_size_t, _P]),
     'qb_logpost_members': (C.c_int, [C.POINTER(qb_net_t), C.c_int, _P, C.c_int64, C.POINTER(qb_data_t), C.c_int64, C.c_int64,
                                      C.POINTER(qb_lik_t), _P, _P, _P, C.c_size_t, _P]),
+    'qb_hvp_workspace_bytes': (C.c_size_t, [C.POINTER(qb_net_t), C.c_int, C.c_int64, C.c_int64]),
+    'qb_logpost_hvp': (C.c_int, [C.POINTER(qb_net_t), C.c_int, _P, _P, C.c_int64, C.c_int64, C.POINTER(qb_data_t),
+                                 C.POINTER(qb_lik_t), _P, _P, C.c_size_t, _P]),
+    'qb_hvp_plan_info': (C.c_int, [C.POINTER(qb_net_t), C.c_int, C.c_int64, C.c_int64, C.POINTER(C.c_int64)]),
     'qb_adam_step': (C.c_int, [C.c_int, _P, _P, _P, _P, C.c_int64, C.c_double, C.c_double, C.c_double, C.c_double,
                                C.c_double, C.c_int64, C.c_double, _P]),
     'qb_copy_rows_where': (C.c_int, [C.c_int, _P, _P, _P, C.c_int64, C.c_int64, _P]),

@@ -12,6 +12,7 @@
 #include "qb_device.cuh"
 #include "qb_chain.cuh"
 #include "qb_stream.cuh"
+#include "qb_hvp.cuh"
 #include "qb_tc.cuh"
 #include "qb_value_tc3.h"
 #include "qb_grad_tc.h"
@@ -780,6 +781,203 @@ extern "C" int qb_logpost_members(const qb_net_t* net, int dtype, const void* th
     if (x_stride < 0 || y_stride < 0) return qb_fail("negative data stride");
     if (dtype == QB_F64) return run_eval<double>(net, dtype, theta, K, data, lik, lp, grad, ws, ws_bytes, (cudaStream_t)stream, x_stride, y_stride);
     return run_eval<float>(net, dtype, theta, K, data, lik, lp, grad, ws, ws_bytes, (cudaStream_t)stream, x_stride, y_stride);
+}
+
+// =================================================================================================
+// kernel 5: Hessian-vector products (qb_hvp.cuh)
+// =================================================================================================
+// Plan for tile size TM: every layer in GEMM mode with TU x 4 thread tiles; returns the shared-memory bytes.
+static long long hvp_plan_for_tm(const qb_net_t* net, int dtype, int TM, QbHvpPlan* H) {
+    const int elem = dtype == QB_F64 ? 8 : 4;
+    const int TU = dtype == QB_F64 ? 4 : 8, LDPAD = dtype == QB_F64 ? 2 : 4, PV = dtype == QB_F64 ? 2 : 4, TP = 4;
+    const int nl = net->n_layers, PG = TM / TP;
+    memset(H, 0, sizeof(*H));
+    QbPlan* P = &H->P;
+    P->n_layers = nl; P->in_dim = net->in_dim; P->out_dim = net->out_dim;
+    P->n_params = net->n_params; P->final_exp = net->final_exp;
+    P->TM = TM; P->lda = TM + LDPAD; P->want_grad = 1; P->elem_size = elem; P->tpg = TP;
+    int woff = 0, max_items = 0, dmax = 0;
+    for (int l = 0; l < nl; ++l) {
+        const qb_layer_t& S = net->layers[l];
+        QbLayerPlan& L = P->L[l];
+        L.n_in = S.n_in; L.n_out = S.n_out; L.n_in_pad = rup(S.n_in, TU); L.n_out_pad = rup(S.n_out, TU);
+        L.w_off = S.w_off; L.b_off = S.b_off; L.act = S.act; L.res_step = S.res_step; L.has_res = S.res_step != 0.0;
+        L.n_terms = S.n_terms > 1 ? S.n_terms : 0; L.w_stride = S.w_stride; L.b_stride = S.b_stride;
+        for (int m = 0; m < QB_MAX_TERMS; ++m) L.coef[m] = S.coef[m];
+        L.mode = QB_MODE_GEMM; L.nj = 4;
+        if (L.has_res) { P->has_res = 1; dmax = std::max(dmax, L.n_out_pad); }
+        L.ug_shift = L.ugi_shift = L.ig_shift = -1;
+        for (int sft = 0; sft < 16; ++sft) {
+            if ((1 << sft) == L.n_out_pad / TU) L.ug_shift = sft;
+            if ((1 << sft) == L.n_in_pad / TU) L.ugi_shift = sft;
+            if ((1 << sft) == (S.n_in + 3) / 4) L.ig_shift = sft;
+        }
+        max_items = std::max(max_items, (L.n_out_pad / TU) * PG);
+        if (l > 0) max_items = std::max(max_items, (L.n_in_pad / TU) * PG);
+        // [W^T ; V^T], [b ; v_b], and for l > 0 [W ; V] (qb_hvp.cuh)
+        L.wt_off = woff; woff += rup((L.n_in_pad + L.n_in) * L.n_out_pad, 4);
+        L.bias_off = woff; woff += rup(2 * L.n_out_pad, 4);
+        L.wr_off = -1;
+        if (l > 0) { L.wr_off = woff; woff += rup((L.n_out_pad + L.n_out) * L.n_in_pad, 4); }
+    }
+    P->w_elems = woff;
+    const int nthreads = std::min(256, std::max(64, rup(max_items, 32)));
+    P->nthreads = nthreads;
+    // activation rows: per layer boundary the tangent rows, then the activation rows
+    int row = 0;
+    for (int b = 0; b <= nl; ++b) {
+        const int npad = b == 0 ? P->L[0].n_in_pad : P->L[b - 1].n_out_pad;
+        row += npad;                                   // tangent rows
+        if (b < nl) P->L[b].row_in = row;
+        if (b > 0) P->L[b - 1].row_out = row;
+        row += npad;
+    }
+    P->d_row = dmax ? row : -1; row += dmax;
+    H->dd_row = dmax ? row : -1; row += dmax;
+    P->total_rows = row;
+    P->buf_rows = row;
+    for (int l = 0; l < nl; ++l) {
+        QbLayerPlan& L = P->L[l];
+        const int patches = ((L.n_out + 3) / 4) * ((L.n_in + 3) / 4);
+        int C = 1;
+        while (C < 32 && patches * C * 2 <= nthreads && TM / (C * 2) >= PV) C *= 2;
+        L.dw_chunks = C;
+        L.c_shift = 0;
+        while ((1 << L.c_shift) < C) ++L.c_shift;
+        H->LA[l] = L; H->LA[l].row_out = L.row_out - L.n_out_pad;
+        H->LB[l] = L; H->LB[l].row_in = L.row_in - L.n_in_pad; H->LB[l].b_off = -1;
+    }
+    // one pad row: the double-buffered hot loop prefetches one row past the end
+    P->smem_bytes = (long long)woff * elem + (long long)(row + 1) * P->lda * elem;
+    return P->smem_bytes;
+}
+
+struct QbHvpLaunch { QbHvpPlan H; int S; long long pps; };
+
+static int make_hvp_launch(const qb_net_t* net, int dtype, long long K, long long N, QbHvpLaunch* out) {
+    if (validate_net(net)) return -1;
+    if (dtype != QB_F32 && dtype != QB_F64) return qb_fail("unknown dtype");
+    if (K < 1 || N < 1) return qb_fail("K and N must be positive");
+    const int cands32[] = {128, 64, 32, 16}, cands64[] = {64, 32, 16, 8};
+    const int* cands = dtype == QB_F64 ? cands64 : cands32;
+    const int mintm = cands[3];
+    const int cap = std::max(mintm, rup((int)std::min<long long>(N, 256), mintm));
+    // The largest tile that fits.  Measured on a B200 (DESIGN.md section 4f, profiles/r4_hessian_bench_*.json): more,
+    // smaller blocks per SM lose, e.g. fp32 config 2 at TM 16 (six 64-thread blocks per SM) reaches 0.06 of the FMA peak
+    // against 0.20 at TM 128, and fp32 config 5 at TM 16 0.07 against 0.30 at TM 128.
+    int pick = -1;
+    for (int c = 0; c < 4 && pick < 0; ++c) {
+        const int TM = cands[c];
+        if (TM <= cap && hvp_plan_for_tm(net, dtype, TM, &out->H) <= QB_SMEM_MAX) pick = TM;
+    }
+    if (pick < 0) {
+        hvp_plan_for_tm(net, dtype, mintm, &out->H);
+        return qb_fail("network too large for the Hessian-vector kernel: its weights, one direction and a %s%lld-point tile "
+                       "exceed 227 KB of shared memory (use the diagonal curvature)", "", mintm);
+    }
+    hvp_plan_for_tm(net, dtype, pick, &out->H);
+    // few directions: split the data axis as kernel 2 does; the [K,S,P] partial rows stay under 256 MB
+    long long S = 1;
+    const long long target = (long long)QB_NUM_SMS * 8;
+    if (K < target) S = std::max<long long>(1, std::min(cdiv(N, 2LL * pick), cdiv(target, K)));
+    S = std::min<long long>(S, std::max<long long>(1, (256LL << 20) / (K * net->n_params * (dtype == QB_F64 ? 8 : 4))));
+    const long long pps = rup((int)cdiv(N, S), pick);
+    out->S = (int)cdiv(N, pps); out->pps = pps;
+    return 0;
+}
+
+template <typename T> struct HvpArgs {
+    const T* theta; const T* v; long long col0;
+    const T* x; const T* y;
+    long long N; int S; long long pps;
+    T* hv;          // [K,P]
+    T* gpart;       // [K,S,P] (S > 1)
+    double inv_sigma2, prior_c;      // prior_c = prior_scale / prior_sigma^2, or 0
+};
+
+template <typename T>
+__global__ void __launch_bounds__(256, 1) k_logpost_hvp(const __grid_constant__ QbHvpPlan H, const HvpArgs<T> a) {
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    const long long k = blockIdx.x, s = blockIdx.y;
+    const int P = H.P.n_params;
+    const long long n0 = s * a.pps, n1 = min(a.N, n0 + a.pps);
+    T* g = (a.S == 1) ? a.hv + k * P : a.gpart + (k * a.S + s) * P;
+    qb_hvp_eval<T>(H, smem_raw, a.theta, a.v ? a.v + k * P : nullptr, (int)(a.col0 + k), a.x, a.y, n0, n1, a.inv_sigma2, g);
+}
+
+// hv[k,:] = sum of the N-split rows in fixed order - prior_c * v_k
+template <typename T>
+__global__ void __launch_bounds__(256) k_hvp_finalize(const HvpArgs<T> a, long long K, int P) {
+    const long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= K * P) return;
+    const long long k = e / P;
+    const int i = (int)(e - k * P);
+    T h;
+    if (a.S > 1) {
+        const T* src = a.gpart + k * a.S * (long long)P + i;
+        h = T(0);
+        for (int s = 0; s < a.S; ++s) h += src[(long long)s * P];
+    } else {
+        h = a.hv[e];
+    }
+    if (a.prior_c != 0.0) {
+        const double vi = a.v ? (double)a.v[e] : (i == a.col0 + k ? 1.0 : 0.0);
+        h = (T)((double)h - a.prior_c * vi);
+    }
+    a.hv[e] = h;
+}
+
+extern "C" size_t qb_hvp_workspace_bytes(const qb_net_t* net, int dtype, int64_t K, int64_t N) {
+    if (K == 0) return 0;
+    QbHvpLaunch L;
+    if (make_hvp_launch(net, dtype, K, N, &L)) return 0;
+    return L.S > 1 ? (size_t)K * L.S * net->n_params * (dtype == QB_F64 ? 8 : 4) : 0;
+}
+
+extern "C" int qb_hvp_plan_info(const qb_net_t* net, int dtype, int64_t K, int64_t N, int64_t* out) {
+    QbHvpLaunch L;
+    if (make_hvp_launch(net, dtype, K, N, &L)) return -1;
+    out[0] = L.H.P.TM; out[1] = L.H.P.nthreads; out[2] = L.H.P.smem_bytes; out[3] = L.S; out[4] = (int64_t)K * L.S;
+    return 0;
+}
+
+template <typename T>
+static int run_hvp(const qb_net_t* net, int dtype, const void* theta, const void* v, int64_t col0, int64_t K,
+                   const qb_data_t* data, const qb_lik_t* lik, void* hv, void* ws, size_t ws_bytes, cudaStream_t st) {
+    QbHvpLaunch L;
+    if (make_hvp_launch(net, dtype, K, data->n, &L)) return -1;
+    const size_t need = qb_hvp_workspace_bytes(net, dtype, K, data->n);
+    if (ws_bytes < need || (need && !ws)) return qb_fail("workspace too small%s (need %lld bytes)", "", (long long)need);
+    HvpArgs<T> a;
+    a.theta = (const T*)theta; a.v = (const T*)v; a.col0 = col0;
+    a.x = (const T*)data->x; a.y = (const T*)data->y;
+    a.N = data->n; a.S = L.S; a.pps = L.pps;
+    a.hv = (T*)hv; a.gpart = L.S > 1 ? (T*)ws : nullptr;
+    a.inv_sigma2 = 1.0 / (lik->sigma * lik->sigma);
+    a.prior_c = lik->prior_sigma > 0.0 ? lik->prior_scale / (lik->prior_sigma * lik->prior_sigma) : 0.0;
+    if (set_smem(k_logpost_hvp<T>, L.H.P.smem_bytes)) return -2;
+    k_logpost_hvp<T><<<dim3((unsigned)K, (unsigned)L.S), L.H.P.nthreads, L.H.P.smem_bytes, st>>>(L.H, a);
+    QB_CUDA(cudaGetLastError());
+    g_launches += 1;
+    if (L.S > 1 || a.prior_c != 0.0) {
+        const long long n = K * (long long)net->n_params;
+        k_hvp_finalize<T><<<(unsigned)cdiv(n, 256), 256, 0, st>>>(a, K, net->n_params);
+        QB_CUDA(cudaGetLastError());
+        g_launches += 1;
+    }
+    return 0;
+}
+
+extern "C" int qb_logpost_hvp(const qb_net_t* net, int dtype, const void* theta, const void* v, int64_t col0, int64_t K,
+                              const qb_data_t* data, const qb_lik_t* lik, void* hv, void* ws, size_t ws_bytes, void* stream) {
+    if (!theta || !data || !lik || (K > 0 && !hv)) return qb_fail("NULL argument to qb_logpost_hvp");
+    if (K < 0) return qb_fail("K must not be negative");
+    if (lik->anchor_per_chain) return qb_fail("qb_logpost_hvp evaluates one theta: anchor_per_chain must be 0");
+    if (!net) return qb_fail("net is NULL");
+    if (!v && (col0 < 0 || col0 + K > net->n_params)) return qb_fail("unit directions col0 .. col0+K-1 out of range");
+    if (K == 0) return 0;
+    if (dtype == QB_F64) return run_hvp<double>(net, dtype, theta, v, col0, K, data, lik, hv, ws, ws_bytes, (cudaStream_t)stream);
+    return run_hvp<float>(net, dtype, theta, v, col0, K, data, lik, hv, ws, ws_bytes, (cudaStream_t)stream);
 }
 
 // Adam (torch.optim.Adam semantics, quinn/nns/nnfit.py:92-93) on a flat array: g = grad*grad_scale + wd*theta

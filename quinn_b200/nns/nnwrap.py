@@ -1,6 +1,7 @@
 """NNWrap: the numpy <-> network seam of the reference (quinn/nns/nnwrap.py:9-150, 330-347), backed by
 the CUDA kernels: ``__call__`` / ``predict`` / ``nn_p`` run posterior-predictive kernel 4,
-``calc_loss`` / ``calc_lossgrad`` with a NegLogPost run kernels 1 / 2.  No torch-CPU evaluation."""
+``calc_loss`` / ``calc_lossgrad`` with a NegLogPost run kernels 1 / 2, ``calc_hess_full`` kernel 5.  No torch-CPU
+evaluation."""
 import numpy as np
 import torch
 
@@ -115,8 +116,12 @@ class NNWrap:
 
     # ---- diagonal Fisher (the by-product of kernel 2 that NN_Laplace uses, SURVEY.md 8f rank 4)
     def calc_fisher_diag(self, weights, loss_fn, inputs, targets, chunk=65536):
-        """Diagonal of calc_hess_diag as a vector: mean over the data points of the squared gradient of the loss
-        evaluated on one point at a time (nnwrap.py:204-229).  Kernel 2 runs with one data point per "member"
+        """Diagonal of calc_hess_diag as a numpy vector (fisher_diag_device)."""
+        return self.fisher_diag_device(weights, loss_fn, inputs, targets, chunk).cpu().numpy()
+
+    def fisher_diag_device(self, weights, loss_fn, inputs, targets, chunk=65536):
+        """Diagonal of calc_hess_diag as a float64 device vector: mean over the data points of the squared gradient of the
+        loss evaluated on one point at a time (nnwrap.py:204-229).  Kernel 2 runs with one data point per "member"
         (qb_logpost_members: member i sees x[i], y[i]; all members share theta), qb_colsq_mean reduces the squares."""
         import ctypes as C
         from .. import _lib, post
@@ -143,7 +148,18 @@ class NNWrap:
                                                   C.byref(lik), _ptr(lp), _ptr(g), _ptr(ws), ws.numel(), _stream()),
                            'qb_logpost_members')
             acc += post.fisher_diag(g) * (n / float(N))
-        return acc.cpu().numpy()
+        return acc
+
+    def hess_full_device(self, weights, loss_fn, inputs, targets):
+        """Hessian of the loss (= -d^2 lp / d theta^2) as a (P, P) device tensor: P exact Hessian-vector products of
+        unit directions in kernel 5."""
+        prob = self._problem(loss_fn, inputs, targets)
+        self.p_unflatten(weights)
+        return ops.logpost_hessian(prob, np.asarray(weights, dtype=np.float64)).neg_()
+
+    def calc_hess_full(self, weights, loss_fn, inputs, targets):
+        """(P, P) Hessian of the loss as numpy (nnwrap.py:153-203); NegLogPost -> kernel 5."""
+        return self.hess_full_device(weights, loss_fn, inputs, targets).double().cpu().numpy()
 
     def calc_hess_diag(self, weights, loss_fn, inputs, targets):
         """The reference's return value: a (P, P) matrix with the diagonal Fisher on its diagonal (nnwrap.py:229)."""

@@ -141,6 +141,54 @@ def logpost_grad(prob: Problem, theta, lp=None, grad=None):
     return lp, grad
 
 
+def hvp_plan_info(prob: Problem, K):
+    """Launch plan of kernel 5 for K directions; raises for a network the kernel refuses."""
+    out = (C.c_int64 * 8)()
+    _lib.check(_lib.load().qb_hvp_plan_info(C.byref(prob.cnet), prob.qdt, K, prob.n, out), 'qb_hvp_plan_info')
+    return dict(TM=out[0], threads=out[1], smem_bytes=out[2], splits=out[3], blocks=out[4])
+
+
+def _hvp(prob: Problem, theta, v, col0, K, out):
+    if prob.clik.anchor_per_chain:
+        raise ValueError('Hessian-vector products are taken at one theta: the prior anchor must be a single vector')
+    lib = _lib.load()
+    nbytes = lib.qb_hvp_workspace_bytes(C.byref(prob.cnet), prob.qdt, K, prob.n)
+    if nbytes == 0 and K > 0:
+        hvp_plan_info(prob, K)            # raises with the reason when the network is refused
+    ws = torch.empty(max(int(nbytes), 1), dtype=torch.uint8, device=prob.device)
+    with torch.cuda.device(prob.device):
+        rc = lib.qb_logpost_hvp(C.byref(prob.cnet), prob.qdt, _ptr(theta), _ptr(v), int(col0), int(K), C.byref(prob.cdata),
+                                C.byref(prob.clik), _ptr(out), _ptr(ws), ws.numel(), _stream())
+    _lib.check(rc, 'qb_logpost_hvp')
+    return out
+
+
+def logpost_hvp(prob: Problem, theta, v):
+    """Kernel 5: hv[K,P] = (d^2 lp / d theta^2) v_k at one theta[P], for directions v[K,P] (or v[P])."""
+    theta = prob.theta(theta)
+    if theta.shape[0] != 1:
+        raise ValueError('logpost_hvp takes a single theta')
+    v = prob.theta(v)
+    return _hvp(prob, theta, v, 0, v.shape[0], torch.empty_like(v))
+
+
+def logpost_hessian(prob: Problem, theta, block=None):
+    """Full Hessian d^2 lp / d theta^2 [P,P] on the device, filled by blocks of `block` unit directions (default: all P
+    in one launch; kernel 5 caps its N-split workspace at 256 MB)."""
+    theta = prob.theta(theta)
+    if theta.shape[0] != 1:
+        raise ValueError('logpost_hessian takes a single theta')
+    P = prob.desc.n_params
+    block = P if block is None else int(block)
+    if block < 1:
+        raise ValueError('block must be positive')
+    H = torch.empty((P, P), dtype=prob.dtype, device=prob.device)
+    for c0 in range(0, P, block):
+        K = min(block, P - c0)
+        _hvp(prob, theta, None, c0, K, H[c0:c0 + K])
+    return H
+
+
 def predict(desc: NetDesc, theta, x, dtype=torch.float32, device='cuda', want_out=True, want_moments=False,
             cnet=None):
     """Kernel 4: theta[M,P], x[N,d] -> out[M,N,o] and/or (mean[N,o], var[N,o], ddof=1)."""

@@ -20,7 +20,8 @@ class NN_RMS(NN_Ens):
 
     def fit(self, xtrn, ytrn, **kwargs):
         """Same call as the reference (nn_rms.py:33-56): per member a random subset (np.random.permutation), an anchor
-        torch.randn(P) * priorsigma and nnfit(loss_fn='logpost', datanoise, priorparams)."""
+        torch.randn(P) * priorsigma and nnfit(loss_fn='logpost', datanoise, priorparams).  The members' subsets and
+        anchors are kept as `subsets` [nens, nsub] and `anchors` [nens, P]."""
         ntrn = ytrn.shape[0]
         nsub = int(ntrn * self.dfrac)
         user = dict(kwargs)
@@ -28,13 +29,17 @@ class NN_RMS(NN_Ens):
             user.pop(k, None)
         self.batched_fit = False
         if not self._can_batch(user):
+            subsets, anchors = [], []
             for jens, learner in enumerate(self.learners):
                 print(f"======== Fitting Learner {jens + 1}/{self.nens} =======")
                 ind = np.random.permutation(ntrn)[:nsub]
+                anchor = torch.randn(size=(self.nparams,), dtype=torch.float64) * self.priorsigma
                 kw = dict(user, lhist_suffix=f'_e{jens}', loss_fn='logpost', datanoise=self.datanoise,
-                          priorparams={'sigma': self.priorsigma,
-                                       'anchor': torch.randn(size=(self.nparams,), dtype=torch.float64) * self.priorsigma})
+                          priorparams={'sigma': self.priorsigma, 'anchor': anchor})
                 learner.fit(xtrn[ind], ytrn[ind], **kw)
+                subsets.append(ind)
+                anchors.append(anchor.numpy())
+            self.subsets, self.anchors = np.stack(subsets), np.stack(anchors)
             return
         from ..ens.batched import fit_members
         print(f"======== Fitting {self.nens} anchored learners together =======")
@@ -56,7 +61,7 @@ class NN_RMS(NN_Ens):
                           logpost=dict(sigma=self.datanoise, prior_sigma=self.priorsigma, anchor=np.stack(anchors)))
         best = res['best_theta'].double().cpu().numpy()
         self.fit_info = {k: v.cpu().numpy() for k, v in res.items() if k in ('best_loss', 'best_epoch')}
-        self.anchors = np.stack(anchors)
+        self.subsets, self.anchors = np.stack(subsets), np.stack(anchors)
         self.batched_fit = True
         for k, learner in enumerate(self.learners):
             learner.best_model = copy.deepcopy(learner.nnmodel)
