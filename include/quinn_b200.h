@@ -86,7 +86,7 @@ const char* qb_last_error(void);
  * qb_version() differs from the QB_ABI_VERSION it was written against (quinn_b200/_lib.py does), and can check its
  * struct mirrors against qb_struct_sizes(): out[0..n) = sizeof of qb_layer_t, qb_net_t, qb_lik_t, qb_data_t, qb_chain_t,
  * qb_rng_t, qb_record_t, qb_amcmc_t, qb_hmc_t (declaration order); returns how many sizes exist. */
-#define QB_ABI_VERSION 201
+#define QB_ABI_VERSION 202
 int qb_version(void);
 int qb_struct_sizes(int64_t* out, int n);
 
@@ -120,6 +120,22 @@ int qb_logpost_hvp(const qb_net_t* net, int dtype, const void* theta, const void
 /* Launch plan of kernel 5 for K directions over N points: out[0..4] = {tile points TM, threads per block, dynamic smem
  * bytes, N-splits S, blocks}.  Returns -1 (with qb_last_error) for a network kernel 5 refuses. */
 int qb_hvp_plan_info(const qb_net_t* net, int dtype, int64_t K, int64_t N, int64_t* out);
+
+/* Kernel 6.  Kronecker factors of the per-point empirical Fisher of every layer at one theta[P], summed over the N points
+ * (no 1/N, no prior).  For layer l with input activations a_i and pre-activation gradients delta_i = d log p_i / d z_l of
+ * point i's data term -0.5 ||y_i - f(x_i)||^2 / sigma^2 (only lik->sigma is used):
+ *     A_l = sum_i a_i a_i^T [n_in, n_in],  s_l = sum_i a_i [n_in] (layers with a bias only),  G_l = sum_i delta_i delta_i^T
+ *     [n_out, n_out].
+ * factors: device double, [A_0 | s_0 | G_0 | A_1 | s_1 | G_1 | ...], each matrix row-major, s_l absent without a bias.
+ * Refused (error text says why): layers sharing weights (RNet Poly(0)), polynomial-in-depth weights (n_terms >= 2),
+ * networks that kernel 2 evaluates on the layer-streamed path (plan code 5), lik->anchor_per_chain != 0.
+ * N == 0 writes zero factors and launches no kernel.  Deterministic: fp64 results are bit-identical run to run. */
+size_t qb_kfac_workspace_bytes(const qb_net_t* net, int dtype, int64_t N);
+int qb_logpost_kfac(const qb_net_t* net, int dtype, const void* theta, const qb_data_t* data, const qb_lik_t* lik,
+                    double* factors, void* workspace, size_t workspace_bytes, void* stream);
+/* Launch plan of kernel 6 over N points: out[0..4] = {tile points TM, threads per block, dynamic smem bytes, N-splits S
+ * (one block each), factor elements F}.  Returns -1 (with qb_last_error) for a network kernel 6 refuses. */
+int qb_kfac_plan_info(const qb_net_t* net, int dtype, int64_t N, int64_t* out);
 
 /* ---- Batched ensemble training (SURVEY.md 8f rank 1) --------------------------------------------
  * NN_Ens.fit (quinn/solvers/nn_ens.py:51-69) trains nens members one after the other, each with

@@ -13,6 +13,7 @@
 #include "qb_chain.cuh"
 #include "qb_stream.cuh"
 #include "qb_hvp.cuh"
+#include "qb_kfac.cuh"
 #include "qb_tc.cuh"
 #include "qb_value_tc3.h"
 #include "qb_grad_tc.h"
@@ -978,6 +979,153 @@ extern "C" int qb_logpost_hvp(const qb_net_t* net, int dtype, const void* theta,
     if (K == 0) return 0;
     if (dtype == QB_F64) return run_hvp<double>(net, dtype, theta, v, col0, K, data, lik, hv, ws, ws_bytes, (cudaStream_t)stream);
     return run_hvp<float>(net, dtype, theta, v, col0, K, data, lik, hv, ws, ws_bytes, (cudaStream_t)stream);
+}
+
+// =================================================================================================
+// kernel 6: Kronecker factors of the per-point empirical Fisher (qb_kfac.cuh)
+// =================================================================================================
+// qb_dw_accumulate's split of one re-pointed factor pass (as in plan_for_tm, for the pass's own shape)
+static void kfac_dw_split(QbLayerPlan& L, int nthreads, int TM, int PV) {
+    const int patches = ((L.n_out + 3) / 4) * ((L.n_in + 3) / 4);
+    int C = 1;
+    while (C < 32 && patches * C * 2 <= nthreads && TM / (C * 2) >= PV) C *= 2;
+    L.dw_chunks = C;
+    L.c_shift = 0;
+    while ((1 << L.c_shift) < C) ++L.c_shift;
+    L.ig_shift = -1;
+    for (int sft = 0; sft < 16; ++sft)
+        if ((1 << sft) == (L.n_in + 3) / 4) L.ig_shift = sft;
+}
+
+struct QbKfacLaunch { QbKfacPlan K; int S; long long pps; };
+
+// Kernel 2's resident CUDA-core plan for one theta, the factor passes of every layer, and the N-split: one block per
+// split, the [S, F] partial rows (dtype) under 256 MB.
+static int make_kfac_launch(const qb_net_t* net, int dtype, long long N, QbKfacLaunch* out) {
+    if (validate_net(net)) return -1;
+    if (dtype != QB_F32 && dtype != QB_F64) return qb_fail("unknown dtype");
+    for (int l = 0; l < net->n_layers; ++l) {
+        const qb_layer_t& S = net->layers[l];
+        if (S.n_terms > 1)
+            return qb_fail("Kronecker factors: layer %s%lld has polynomial-in-depth weights (n_terms >= 2); every layer "
+                           "must own its weights", "", l);
+        for (int m = 0; m < l; ++m)
+            if (net->layers[m].w_off == S.w_off)
+                return qb_fail("Kronecker factors: layer %s%lld shares its weights with an earlier layer; every layer must "
+                               "own its weights", "", l);
+    }
+    QbLaunch L;
+    if (make_launch(net, dtype, true, 1, N, true, &L)) return -1;
+    if (L.streamed)
+        return qb_fail("Kronecker factors: the network's weights do not fit in shared memory next to one tile of "
+                       "activations, and the layer-streamed path (plan code 5) has no factor kernel");
+    memset(&out->K, 0, sizeof(out->K));
+    out->K.P = L.plan;
+    const QbPlan& P = out->K.P;
+    const int PV = dtype == QB_F64 ? 2 : 4;
+    int off = 0;
+    for (int l = 0; l < P.n_layers; ++l) {
+        const QbLayerPlan& B = P.L[l];
+        QbLayerPlan& A = out->K.LA[l];
+        A = B;
+        A.n_out = B.n_in; A.n_out_pad = B.n_in_pad; A.row_out = B.row_in;
+        A.n_terms = 0;
+        A.w_off = off; off += B.n_in * B.n_in;
+        A.b_off = -1;
+        if (B.b_off >= 0) { A.b_off = off; off += B.n_in; }
+        kfac_dw_split(A, P.nthreads, P.TM, PV);
+        QbLayerPlan& G = out->K.LG[l];
+        G = B;
+        G.n_in = B.n_out; G.n_in_pad = B.n_out_pad; G.row_in = B.row_out;
+        G.n_terms = 0;
+        G.w_off = off; off += B.n_out * B.n_out;
+        G.b_off = -1;
+        kfac_dw_split(G, P.nthreads, P.TM, PV);
+    }
+    out->K.n_factors = off;
+    const int TM = P.TM;
+    const long long row_bytes = (long long)off * (dtype == QB_F64 ? 8 : 4);
+    long long S = std::max<long long>(1, std::min(cdiv(N, 2LL * TM), (long long)QB_NUM_SMS * 8));
+    S = std::min<long long>(S, std::max<long long>(1, (256LL << 20) / row_bytes));
+    const long long pps = rup((int)cdiv(N, S), TM);
+    out->S = (int)cdiv(N, pps); out->pps = pps;
+    return 0;
+}
+
+template <typename T> struct KfacArgs {
+    const T* theta; const T* x; const T* y;
+    long long N; int S; long long pps;
+    T* part;            // [S, F]
+    double* factors;    // [F]
+    double inv_sigma2;
+};
+
+// fp32: one block per SM in the register budget (157 registers; at two, 128 registers spill the fp32 factor passes)
+template <typename T>
+__global__ void __launch_bounds__(256, sizeof(T) == 8 ? 2 : 1) k_logpost_kfac(const __grid_constant__ QbKfacPlan K, const KfacArgs<T> a) {
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    const QbSmem S = qb_carve<T>(K.P, smem_raw);
+    const long long s = blockIdx.x;
+    const long long n0 = s * a.pps, n1 = min(a.N, n0 + a.pps);
+    qb_kfac_eval<T>(K, S, a.theta, a.x, a.y, n0, n1, a.inv_sigma2, a.part + s * K.n_factors);
+}
+
+// factors[e] = sum of the N-split rows in fixed order, in double
+template <typename T>
+__global__ void __launch_bounds__(256) k_kfac_finalize(const KfacArgs<T> a, int F) {
+    const long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= F) return;
+    double v = 0.0;
+    for (int s = 0; s < a.S; ++s) v += (double)a.part[(long long)s * F + e];
+    a.factors[e] = v;
+}
+
+extern "C" size_t qb_kfac_workspace_bytes(const qb_net_t* net, int dtype, int64_t N) {
+    if (N <= 0) return 0;
+    QbKfacLaunch L;
+    if (make_kfac_launch(net, dtype, N, &L)) return 0;
+    return (size_t)L.S * L.K.n_factors * (dtype == QB_F64 ? 8 : 4);
+}
+
+extern "C" int qb_kfac_plan_info(const qb_net_t* net, int dtype, int64_t N, int64_t* out) {
+    QbKfacLaunch L;
+    if (make_kfac_launch(net, dtype, std::max<int64_t>(N, 1), &L)) return -1;
+    out[0] = L.K.P.TM; out[1] = L.K.P.nthreads; out[2] = L.K.P.smem_bytes; out[3] = L.S; out[4] = L.K.n_factors;
+    return 0;
+}
+
+template <typename T>
+static int run_kfac(const qb_net_t* net, int dtype, const void* theta, const qb_data_t* data, const qb_lik_t* lik,
+                    double* factors, void* ws, size_t ws_bytes, cudaStream_t st) {
+    QbKfacLaunch L;
+    if (make_kfac_launch(net, dtype, std::max<int64_t>(data->n, 1), &L)) return -1;
+    if (data->n == 0) {               // no points: zero factors, no kernel
+        QB_CUDA(cudaMemsetAsync(factors, 0, (size_t)L.K.n_factors * sizeof(double), st));
+        return 0;
+    }
+    const size_t need = (size_t)L.S * L.K.n_factors * sizeof(T);
+    if (ws_bytes < need || !ws) return qb_fail("workspace too small%s (need %lld bytes)", "", (long long)need);
+    KfacArgs<T> a;
+    a.theta = (const T*)theta; a.x = (const T*)data->x; a.y = (const T*)data->y;
+    a.N = data->n; a.S = L.S; a.pps = L.pps;
+    a.part = (T*)ws; a.factors = factors;
+    a.inv_sigma2 = 1.0 / (lik->sigma * lik->sigma);
+    if (set_smem(k_logpost_kfac<T>, L.K.P.smem_bytes)) return -2;
+    k_logpost_kfac<T><<<(unsigned)L.S, L.K.P.nthreads, L.K.P.smem_bytes, st>>>(L.K, a);
+    QB_CUDA(cudaGetLastError());
+    k_kfac_finalize<T><<<(unsigned)cdiv(L.K.n_factors, 256), 256, 0, st>>>(a, L.K.n_factors);
+    QB_CUDA(cudaGetLastError());
+    g_launches += 2;
+    return 0;
+}
+
+extern "C" int qb_logpost_kfac(const qb_net_t* net, int dtype, const void* theta, const qb_data_t* data,
+                               const qb_lik_t* lik, double* factors, void* ws, size_t ws_bytes, void* stream) {
+    if (!theta || !data || !lik || !factors) return qb_fail("NULL argument to qb_logpost_kfac");
+    if (data->n < 0) return qb_fail("N must not be negative");
+    if (lik->anchor_per_chain) return qb_fail("qb_logpost_kfac evaluates one theta: anchor_per_chain must be 0");
+    if (dtype == QB_F64) return run_kfac<double>(net, dtype, theta, data, lik, factors, ws, ws_bytes, (cudaStream_t)stream);
+    return run_kfac<float>(net, dtype, theta, data, lik, factors, ws, ws_bytes, (cudaStream_t)stream);
 }
 
 // Adam (torch.optim.Adam semantics, quinn/nns/nnfit.py:92-93) on a flat array: g = grad*grad_scale + wd*theta

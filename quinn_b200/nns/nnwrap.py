@@ -1,7 +1,7 @@
 """NNWrap: the numpy <-> network seam of the reference (quinn/nns/nnwrap.py:9-150, 330-347), backed by
 the CUDA kernels: ``__call__`` / ``predict`` / ``nn_p`` run posterior-predictive kernel 4,
-``calc_loss`` / ``calc_lossgrad`` with a NegLogPost run kernels 1 / 2, ``calc_hess_full`` kernel 5.  No torch-CPU
-evaluation."""
+``calc_loss`` / ``calc_lossgrad`` with a NegLogPost run kernels 1 / 2, ``calc_hess_full`` kernel 5, ``kfac_device``
+kernel 6.  No torch-CPU evaluation."""
 import numpy as np
 import torch
 
@@ -160,6 +160,13 @@ class NNWrap:
     def calc_hess_full(self, weights, loss_fn, inputs, targets):
         """(P, P) Hessian of the loss as numpy (nnwrap.py:153-203); NegLogPost -> kernel 5."""
         return self.hess_full_device(weights, loss_fn, inputs, targets).double().cpu().numpy()
+
+    def kfac_device(self, weights, loss_fn, inputs, targets):
+        """Kronecker factors of the per-point empirical Fisher of every Linear layer (kernel 6): a list of dicts
+        {A, s, G} of float64 device tensors, raw sums over the data points (ops.logpost_kfac)."""
+        prob = self._problem(loss_fn, inputs, targets)
+        self.p_unflatten(weights)
+        return ops.logpost_kfac(prob, np.asarray(weights, dtype=np.float64))
 
     def calc_hess_diag(self, weights, loss_fn, inputs, targets):
         """The reference's return value: a (P, P) matrix with the diagonal Fisher on its diagonal (nnwrap.py:229)."""

@@ -189,6 +189,52 @@ def logpost_hessian(prob: Problem, theta, block=None):
     return H
 
 
+def kfac_plan_info(prob: Problem):
+    """Launch plan of kernel 6 over the problem's points; raises for a network the kernel refuses."""
+    out = (C.c_int64 * 8)()
+    _lib.check(_lib.load().qb_kfac_plan_info(C.byref(prob.cnet), prob.qdt, prob.n, out), 'qb_kfac_plan_info')
+    return dict(TM=out[0], threads=out[1], smem_bytes=out[2], splits=out[3], factor_elems=out[4])
+
+
+def kfac_layout(desc: NetDesc):
+    """Per layer (n_in, n_out, has_bias, offset of A, offset of s or -1, offset of G) in kernel 6's factor row."""
+    out, off = [], 0
+    for L in desc.layers:
+        a_off = off
+        off += L.n_in * L.n_in
+        s_off = off if L.b_off >= 0 else -1
+        off += L.n_in if L.b_off >= 0 else 0
+        out.append((L.n_in, L.n_out, L.b_off >= 0, a_off, s_off, off))
+        off += L.n_out * L.n_out
+    return out
+
+
+def logpost_kfac(prob: Problem, theta):
+    """Kernel 6: per layer dict(A, s, G) of float64 device tensors at one theta[P] -- the raw sums over the data points
+    A = sum_i a_i a_i^T [n_in, n_in], s = sum_i a_i [n_in] (None without a bias), G = sum_i delta_i delta_i^T
+    [n_out, n_out], with a_i the layer's input and delta_i = d log p_i / d z of point i's data term."""
+    theta = prob.theta(theta)
+    if theta.shape[0] != 1:
+        raise ValueError('logpost_kfac takes a single theta')
+    if prob.clik.anchor_per_chain:
+        raise ValueError('Kronecker factors are taken at one theta: the prior anchor must be a single vector')
+    F = kfac_plan_info(prob)['factor_elems']            # raises with the reason when the network is refused
+    lib = _lib.load()
+    fac = torch.empty(F, dtype=torch.float64, device=prob.device)
+    nbytes = lib.qb_kfac_workspace_bytes(C.byref(prob.cnet), prob.qdt, prob.n)
+    ws = torch.empty(max(int(nbytes), 1), dtype=torch.uint8, device=prob.device)
+    with torch.cuda.device(prob.device):
+        rc = lib.qb_logpost_kfac(C.byref(prob.cnet), prob.qdt, _ptr(theta), C.byref(prob.cdata), C.byref(prob.clik),
+                                 _ptr(fac), _ptr(ws), ws.numel(), _stream())
+    _lib.check(rc, 'qb_logpost_kfac')
+    out = []
+    for n_in, n_out, bias, a_off, s_off, g_off in kfac_layout(prob.desc):
+        out.append(dict(A=fac[a_off:a_off + n_in * n_in].view(n_in, n_in),
+                        s=fac[s_off:s_off + n_in] if bias else None,
+                        G=fac[g_off:g_off + n_out * n_out].view(n_out, n_out)))
+    return out
+
+
 def predict(desc: NetDesc, theta, x, dtype=torch.float32, device='cuda', want_out=True, want_moments=False,
             cnet=None):
     """Kernel 4: theta[M,P], x[N,d] -> out[M,N,o] and/or (mean[N,o], var[N,o], ddof=1)."""
