@@ -1,7 +1,6 @@
 // quinn_b200: kernel 2 (log-posterior + gradient) and the HMC / MALA chain kernel on the tensor cores (tcgen05).
 // Device code: qb_tcg.cuh.  Separate translation unit so that it compiles in parallel with qb_kernels.cu.
 #include <cuda_runtime.h>
-#include <stdlib.h>
 #include <string.h>
 #include <algorithm>
 
@@ -12,15 +11,11 @@
 #include "qb_tc.cuh"
 #include "qb_tcg.cuh"
 #include "qb_grad_tc.h"
-
-static int tcg_env_int(const char* name, int dflt) {
-    const char* s = getenv(name);
-    return (s && *s) ? atoi(s) : dflt;
-}
+#include "qb_launch.h"
 
 bool qb_tcg_make_plan(const qb_net_t* net, int dtype, QbTcgPlan* tp) {
     memset(tp, 0, sizeof(*tp));
-    if (dtype != QB_F32 || tcg_env_int("QB_NO_TC", 0) || tcg_env_int("QB_NO_TCG", 0)) return false;
+    if (dtype != QB_F32 || qb_env_int("QB_NO_TC", 0) || qb_env_int("QB_NO_TCG", 0)) return false;
     if (net->n_layers != 3 || net->in_dim > 7 || net->out_dim != 1 || net->final_exp) return false;
     const qb_layer_t& L0 = net->layers[0];
     const qb_layer_t& L1 = net->layers[1];

@@ -1,4 +1,4 @@
-// Host interface of the tensor-core gradient translation unit (qb_grad_tc.cu); called from qb_kernels.cu.
+// Host interface of the tensor-core gradient translation unit (qb_grad_tc.cu); called from qb_kernels.cu and qb_launch.cu.
 #pragma once
 #include <cuda_runtime.h>
 #include "quinn_b200.h"

@@ -2,7 +2,6 @@
 // operands (widths 64 and 128: configs 3 / 4 / 5).  Device code: qb_tg8.cuh.  Separate translation unit so that it compiles
 // in parallel with the others.
 #include <cuda_runtime.h>
-#include <stdlib.h>
 #include <string.h>
 #include <algorithm>
 #include <map>
@@ -16,15 +15,11 @@
 #include "qb_tc.cuh"
 #include "qb_tg8.cuh"
 #include "qb_grad_tc128.h"
-
-static int tg8_env_int(const char* name, int dflt) {
-    const char* s = getenv(name);
-    return (s && *s) ? atoi(s) : dflt;
-}
+#include "qb_launch.h"
 
 bool qb_tg8_make_plan(const qb_net_t* net, int dtype, QbTg8Plan* tp) {
     memset(tp, 0, sizeof(*tp));
-    if (dtype != QB_F32 || tg8_env_int("QB_NO_TC", 0) || tg8_env_int("QB_NO_TCG", 0) || tg8_env_int("QB_NO_TG8", 0)) return false;
+    if (dtype != QB_F32 || qb_env_int("QB_NO_TC", 0) || qb_env_int("QB_NO_TCG", 0) || qb_env_int("QB_NO_TG8", 0)) return false;
     if (net->n_layers != 3 || net->in_dim > 15 || net->out_dim != 1 || net->final_exp) return false;
     const qb_layer_t& L0 = net->layers[0];
     const qb_layer_t& L1 = net->layers[1];
@@ -33,7 +28,7 @@ bool qb_tg8_make_plan(const qb_net_t* net, int dtype, QbTg8Plan* tp) {
     if (L0.n_terms > 1 || L1.n_terms > 1 || L2.n_terms > 1) return false;
     const int HR = L0.n_out;
     if ((HR != 128 && HR != 64 && HR != 32) || L1.n_out != HR) return false;
-    if (HR <= 64 && !tg8_env_int("QB_TG8_64", 1)) return false;
+    if (HR <= 64 && !qb_env_int("QB_TG8_64", 1)) return false;
     const int H = HR == 32 ? 64 : HR;                        // 32-wide nets: zero-padded units on the 64-wide instance
     if (L0.act != QB_ACT_TANH || L1.act != QB_ACT_TANH || L2.act != QB_ACT_IDENTITY) return false;
     tp->in_dim = net->in_dim; tp->n_params = net->n_params; tp->h = H; tp->hr = HR;

@@ -2,19 +2,14 @@
 //   nvcc -gencode arch=compute_100a,code=sm_100a -lineinfo -O3 --shared -Xcompiler -fPIC
 #include <cuda_runtime.h>
 #include <stdio.h>
-#include <stdlib.h>
 #include <string.h>
 #include <algorithm>
 #include <atomic>
 
 #include "quinn_b200.h"
-#include "qb_plan.h"
 #include "qb_device.cuh"
 #include "qb_chain.cuh"
-#include "qb_stream.cuh"
-#include "qb_hvp.cuh"
-#include "qb_kfac.cuh"
-#include "qb_tc.cuh"
+#include "qb_launch.h"
 #include "qb_value_tc3.h"
 #include "qb_grad_tc.h"
 #include "qb_grad_tc128.h"
@@ -27,13 +22,9 @@
 // =================================================================================================
 // error plumbing
 // =================================================================================================
-static thread_local char g_err[512] = "";
+thread_local char g_err[512] = "";          // error text of the calling thread (qb_fail, qb_launch.cu)
 static std::atomic<long long> g_launches{0};
 
-static int qb_fail(const char* fmt, const char* a = "", long long b = 0) {
-    snprintf(g_err, sizeof(g_err), fmt, a, b);
-    return -1;
-}
 #define QB_CUDA(call)                                                                                    \
     do {                                                                                                 \
         cudaError_t e_ = (call);                                                                         \
@@ -58,455 +49,7 @@ extern "C" int qb_struct_sizes(int64_t* out, int n) {
 }
 extern "C" int64_t qb_launch_count(void) { return (int64_t)g_launches.load(); }
 
-// =================================================================================================
-// launch planning (host)
-// =================================================================================================
-static inline int rup(int v, int m) { return (v + m - 1) / m * m; }
 static inline long long cdiv(long long a, long long b) { return (a + b - 1) / b; }
-static int env_int(const char* name, int dflt) {
-    const char* s = getenv(name);
-    return (s && *s) ? atoi(s) : dflt;
-}
-
-static const int QB_SMEM_MAX = 227 * 1024;
-static const int QB_SMEM_SM = 228 * 1024;    // shared memory per SM
-// SM count of the current device (148 on B200), queried once per process
-static int qb_num_sms() {
-    static int n = 0;
-    if (n == 0) {
-        int dev = 0, v = 0;
-        if (cudaGetDevice(&dev) == cudaSuccess && cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess && v > 0) n = v;
-        else n = 148;
-    }
-    return n;
-}
-#define QB_NUM_SMS (qb_num_sms())
-
-static int validate_net(const qb_net_t* net) {
-    if (!net) return qb_fail("net is NULL");
-    if (net->n_layers < 1 || net->n_layers > QB_MAX_LAYERS) return qb_fail("n_layers out of range%s (%lld)", "", net->n_layers);
-    int width = net->in_dim;
-    for (int l = 0; l < net->n_layers; ++l) {
-        const qb_layer_t& L = net->layers[l];
-        if (L.n_in != width) return qb_fail("layer %s%lld: n_in does not match the previous width", "", l);
-        if (L.n_in < 1 || L.n_out < 1) return qb_fail("layer %s%lld: empty layer", "", l);
-        if (L.act < 0 || L.act > 2) return qb_fail("layer %s%lld: unknown activation", "", l);
-        if (L.res_step != 0.0 && L.n_in != L.n_out) return qb_fail("layer %s%lld: residual layer must be square", "", l);
-        if (L.w_off < 0 || L.w_off + L.n_in * L.n_out > net->n_params) return qb_fail("layer %s%lld: weight offset out of range", "", l);
-        if (L.b_off >= 0 && L.b_off + L.n_out > net->n_params) return qb_fail("layer %s%lld: bias offset out of range", "", l);
-        if (L.n_terms < 0 || L.n_terms > QB_MAX_TERMS) return qb_fail("layer %s%lld: n_terms out of range", "", l);
-        if (L.n_terms > 1) {
-            const long long lastw = (long long)L.w_off + (long long)(L.n_terms - 1) * L.w_stride;
-            const long long lastb = (long long)L.b_off + (long long)(L.n_terms - 1) * L.b_stride;
-            if (L.w_stride < 0 || lastw + (long long)L.n_in * L.n_out > net->n_params) return qb_fail("layer %s%lld: polynomial weight terms out of range", "", l);
-            if (L.b_off >= 0 && (L.b_stride < 0 || lastb + L.n_out > net->n_params)) return qb_fail("layer %s%lld: polynomial bias terms out of range", "", l);
-        }
-        width = L.n_out;
-    }
-    if (width != net->out_dim) return qb_fail("out_dim does not match the last layer");
-    return 0;
-}
-
-// Fill `P` for tile size TM; returns smem bytes (or -1 if a constraint fails).
-static long long plan_for_tm(const qb_net_t* net, int dtype, bool want_grad, int TM, QbPlan* P, bool wr_global = false) {
-    const int elem = dtype == QB_F64 ? 8 : 4;
-    const int TU = dtype == QB_F64 ? 4 : 8, LDPAD = dtype == QB_F64 ? 2 : 4, PV = dtype == QB_F64 ? 2 : 4;
-    // gradient kernel: TU x 4 thread tiles (twice the threads per tile) when some layer is >= 64 wide, else TU x 8
-    int widest = 0;
-    for (int l = 0; l < net->n_layers; ++l) widest = std::max(widest, net->layers[l].n_out);
-    const int tpg = (dtype == QB_F64 || widest >= 64) ? 4 : 8;
-    const int TP = want_grad ? env_int("QB_TPG", tpg) : TU;
-    memset(P, 0, sizeof(*P));
-    P->n_layers = net->n_layers; P->in_dim = net->in_dim; P->out_dim = net->out_dim;
-    P->n_params = net->n_params; P->final_exp = net->final_exp;
-    P->TM = TM; P->lda = TM + LDPAD; P->want_grad = want_grad ? 1 : 0; P->elem_size = elem;
-    P->tpg = TP;
-    const int PG = TM / TP;
-    int max_items = 0, woff = 0;
-    bool any_gemm = false;
-    for (int l = 0; l < net->n_layers; ++l) {
-        const qb_layer_t& S = net->layers[l];
-        QbLayerPlan& L = P->L[l];
-        L.n_in = S.n_in; L.n_out = S.n_out; L.n_in_pad = rup(S.n_in, TU); L.n_out_pad = rup(S.n_out, TU);
-        L.w_off = S.w_off; L.b_off = S.b_off; L.act = S.act; L.res_step = S.res_step; L.has_res = S.res_step != 0.0;
-        L.n_terms = S.n_terms > 1 ? S.n_terms : 0; L.w_stride = S.w_stride; L.b_stride = S.b_stride;
-        for (int m = 0; m < QB_MAX_TERMS; ++m) L.coef[m] = S.coef[m];
-        if (L.has_res) P->has_res = 1;
-        const int UG = L.n_out_pad / TU;
-        L.ug_shift = L.ugi_shift = L.ig_shift = -1;
-        for (int sft = 0; sft < 16; ++sft) {
-            if ((1 << sft) == UG) L.ug_shift = sft;
-            if ((1 << sft) == L.n_in_pad / TU) L.ugi_shift = sft;
-            if ((1 << sft) == (S.n_in + 3) / 4) L.ig_shift = sft;
-        }
-        L.nj = S.n_out == 1 ? 1 : (S.n_out == 2 ? 2 : 4);
-        const long long cost_g = cdiv((long long)UG * PG, 256) * S.n_in * (TP * TU + 4);
-        const long long cost_d = cdiv(TM, 256) * cdiv(S.n_out, L.nj) * S.n_in * (2 * L.nj + 1);
-        L.mode = (cost_d < cost_g) ? QB_MODE_DOT : QB_MODE_GEMM;
-        if (L.mode == QB_MODE_GEMM) { any_gemm = true; max_items = std::max(max_items, UG * PG); }
-        if (want_grad && l > 0) max_items = std::max(max_items, (L.n_in_pad / TU) * PG), any_gemm = true;
-        // shared weights: reuse an identical earlier staging
-        int dup = -1;
-        for (int m = 0; m < l; ++m) {
-            const qb_layer_t& Sm = net->layers[m];
-            bool same_terms = (Sm.n_terms > 1 ? Sm.n_terms : 0) == (S.n_terms > 1 ? S.n_terms : 0);
-            if (same_terms && S.n_terms > 1)
-                for (int q = 0; q < S.n_terms; ++q) same_terms = same_terms && Sm.coef[q] == S.coef[q];
-            if (same_terms && Sm.w_off == S.w_off && Sm.b_off == S.b_off && Sm.n_in == S.n_in && Sm.n_out == S.n_out &&
-                (Sm.act == QB_ACT_TANH) == (S.act == QB_ACT_TANH) &&      // fp32 tanh layers stage W * 2log2(e)
-                P->L[m].mode == L.mode && (P->L[m].wr_off >= 0) == (want_grad && l > 0 && !wr_global)) { dup = m; break; }
-        }
-        if (dup >= 0) {
-            L.wt_off = P->L[dup].wt_off; L.bias_off = P->L[dup].bias_off; L.wr_off = P->L[dup].wr_off;
-        } else {
-            L.wt_off = woff; woff += rup(L.n_in * L.n_out_pad, 4);
-            L.bias_off = woff; woff += rup(L.n_out_pad, 4);
-            L.wr_off = -1;
-            if (want_grad && l > 0 && !wr_global) { L.wr_off = woff; woff += rup(L.n_out * L.n_in_pad, 4); }
-        }
-    }
-    P->w_elems = woff;
-    int nthreads = any_gemm ? max_items : TM;
-    nthreads = std::min(want_grad ? 256 : 512, std::max(64, rup(nthreads, 32)));
-    nthreads = env_int("QB_THREADS", nthreads);
-    P->nthreads = nthreads;
-    // value kernel: in place when every GEMM layer is a single pass and DOT layers are single-chunk
-    int inplace = 1, buf_rows = rup(net->in_dim, TU);
-    for (int l = 0; l < net->n_layers; ++l) {
-        QbLayerPlan& L = P->L[l];
-        buf_rows = std::max(buf_rows, std::max(L.n_in_pad, L.n_out_pad));
-        if (L.mode == QB_MODE_GEMM && (L.n_out_pad / TU) * PG > nthreads) inplace = 0;
-        if (L.mode == QB_MODE_DOT && L.n_out > L.nj) inplace = 0;
-        // dW split-K chunks for narrow layers
-        const int patches = ((L.n_out + 3) / 4) * ((L.n_in + 3) / 4);
-        int C = 1;
-        while (C < 32 && patches * C * 2 <= nthreads && TM / (C * 2) >= PV) C *= 2;
-        L.dw_chunks = C;
-        L.c_shift = 0;
-        while ((1 << L.c_shift) < C) ++L.c_shift;
-    }
-    if (env_int("QB_NO_INPLACE", 0)) inplace = 0;
-    // Warp-synchronous value kernel: when every GEMM layer's unit groups divide a warp, one warp can own WP
-    // consecutive points for ALL layers (its lanes cover every unit of those points), so the tile loop needs
-    // no block barrier and warps drift apart (MUFU / FMA / LDS phases of different warps overlap).
-    P->ws = 0; P->WP = 0;
-    if (!want_grad && any_gemm && !env_int("QB_NO_WS", 0)) {
-        int ugmax = 0; bool ok = true;
-        for (int l = 0; l < net->n_layers; ++l) {
-            const QbLayerPlan& L = P->L[l];
-            if (L.mode == QB_MODE_GEMM) {
-                const int UG = L.n_out_pad / TU;
-                if (UG > 32 || 32 % UG) ok = false;
-                ugmax = std::max(ugmax, UG);
-            } else if (L.n_out > L.nj) ok = false;
-        }
-        if (ok) {
-            const int WP = (32 / ugmax) * TP;
-            if (TM % WP == 0 && TM / WP >= 1 && TM / WP <= 16) {
-                P->ws = 1; P->WP = WP; inplace = 1;
-                nthreads = 32 * (TM / WP);
-                P->nthreads = nthreads;
-            }
-        }
-    }
-    P->inplace = inplace; P->buf_rows = buf_rows;
-    // fused tail: ... -> GEMM hidden layer -> narrow linear output layer (identity, no residual, n_out <= 4)
-    P->fuse_tail = 0;
-    // (off by default: the first implementation made ptxas keep the accumulators in local memory -- 8x slower,
-    //  profiles/r1_notes.md; kept behind QB_TAIL=1 for the next round)
-    if (P->ws && net->n_layers >= 2 && env_int("QB_TAIL", 0)) {
-        const QbLayerPlan& Lh = P->L[net->n_layers - 2];
-        const QbLayerPlan& Lo = P->L[net->n_layers - 1];
-        if (Lh.mode == QB_MODE_GEMM && Lo.mode == QB_MODE_DOT && Lo.n_out <= 4 && Lo.act == QB_ACT_IDENTITY &&
-            !Lo.has_res && Lh.ug_shift >= 0)
-            P->fuse_tail = 1;
-    }
-    long long act_elems;
-    if (!want_grad) {
-        act_elems = (long long)(inplace ? 1 : 2) * buf_rows * P->lda;
-        P->total_rows = buf_rows; P->d_row = -1;
-    } else {
-        int row = 0, dmax = 0;
-        for (int l = 0; l < net->n_layers; ++l) {
-            QbLayerPlan& L = P->L[l];
-            L.row_in = row;
-            row += (l == 0) ? rup(net->in_dim, TU) : P->L[l - 1].n_out_pad;
-            if (L.has_res) dmax = std::max(dmax, L.n_out_pad);
-        }
-        for (int l = 0; l < net->n_layers; ++l) P->L[l].row_out = (l + 1 < net->n_layers) ? P->L[l + 1].row_in : row;
-        row += P->L[net->n_layers - 1].n_out_pad;
-        P->d_row = dmax ? row : -1;
-        row += dmax;
-        P->total_rows = row;
-        act_elems = (long long)row * P->lda;
-    }
-    act_elems += P->lda;      // one pad row: the double-buffered hot loop prefetches one row past the end
-    P->smem_bytes = 40 * 8 + (long long)woff * elem + act_elems * elem;
-    return P->smem_bytes;
-}
-
-// Layer-streamed plan (qb_stream.cuh) for tile size TM: fills `P`, returns its shared-memory bytes, or -1 when the
-// activations of one tile leave no room for a ring of chunks of TU rows per layer.
-static long long stream_plan_for_tm(const qb_net_t* net, int dtype, bool want_grad, int TM, QbStreamPlan* P) {
-    const int elem = dtype == QB_F64 ? 8 : 4;
-    const int TU = dtype == QB_F64 ? 4 : 8, TP = 4, VW = dtype == QB_F64 ? 2 : 4, PV = dtype == QB_F64 ? 2 : 4;
-    const int LDPAD = dtype == QB_F64 ? 2 : 4;
-    const int NT = QS_THREADS, nl = net->n_layers;
-    memset(P, 0, sizeof(*P));
-    P->n_layers = nl; P->in_dim = net->in_dim; P->out_dim = net->out_dim; P->n_params = net->n_params;
-    P->final_exp = net->final_exp; P->want_grad = want_grad ? 1 : 0;
-    P->TM = TM; P->lda = TM + LDPAD;
-    while ((TP << P->lg_pg) < TM) ++P->lg_pg;
-    int widest = net->in_dim, row = 0;
-    for (int l = 0; l < nl; ++l) {
-        const qb_layer_t& S = net->layers[l];
-        QbLayerPlan& L = P->L[l];
-        L.n_in = S.n_in; L.n_out = S.n_out; L.n_in_pad = rup(S.n_in, TU); L.n_out_pad = rup(S.n_out, TU);
-        L.w_off = S.w_off; L.b_off = S.b_off; L.act = S.act; L.res_step = S.res_step; L.has_res = S.res_step != 0.0;
-        L.n_terms = S.n_terms > 1 ? S.n_terms : 0; L.w_stride = S.w_stride; L.b_stride = S.b_stride;
-        for (int m = 0; m < QB_MAX_TERMS; ++m) L.coef[m] = S.coef[m];
-        L.wt_off = L.wr_off = L.bias_off = -1;
-        widest = std::max(widest, S.n_out);
-        L.row_in = row; row += S.n_in; L.row_out = row;
-        // weight-gradient split of qb_dw_accumulate (as in plan_for_tm)
-        const int patches = ((S.n_out + 3) / 4) * ((S.n_in + 3) / 4);
-        int C = 1;
-        while (C < 32 && patches * C * 2 <= NT && TM / (C * 2) >= PV) C *= 2;
-        L.dw_chunks = C; L.c_shift = 0;
-        while ((1 << L.c_shift) < C) ++L.c_shift;
-        L.ig_shift = -1;
-        for (int sft = 0; sft < 16; ++sft) if ((1 << sft) == (S.n_in + 3) / 4) L.ig_shift = sft;
-    }
-    row += net->layers[nl - 1].n_out;
-    P->buf_rows = widest; P->total_rows = row; P->da_rows = want_grad ? widest : 0;
-    const long long act_elems = want_grad ? (long long)(row + widest) * P->lda : 2LL * widest * P->lda;
-    const long long head = 384;          // 40 doubles of reduction scratch, then the ring's mbarriers
-    const long long avail = QB_SMEM_MAX - head - act_elems * elem;
-    if (avail <= 0) return -1;
-    const long long slot_max = avail / (QS_STAGES * elem) / 4 * 4;
-    long long slot = 0;
-    int c = 0;
-    for (int l = 0; l < nl; ++l) {
-        const QbLayerPlan& L = P->L[l];
-        QbStreamLayer& S = P->SL[l];
-        const int nterm = L.n_terms > 1 ? L.n_terms : 1;
-        S.ldw = rup(L.n_in, TU);
-        const long long rmax = slot_max / ((long long)nterm * S.ldw) / TU * TU;
-        if (rmax < TU) return -1;
-        int R = (int)std::min<long long>(rmax, rup(L.n_out, TU));
-        S.nch = (int)cdiv(L.n_out, R);
-        R = rup((int)cdiv(L.n_out, S.nch), TU);
-        S.R = R;
-        slot = std::max<long long>(slot, rup(nterm * R * S.ldw, 4));
-        const int nsub = (R / TU) * (TM / TP);
-        while (S.lg_ks < 5 && qs_items(nsub, S.lg_ks + 1) <= NT && (L.n_in >> (S.lg_ks + 1)) >= 2 * VW) ++S.lg_ks;
-        S.kl = rup((int)cdiv(L.n_in, 1 << S.lg_ks), VW);
-        const int nsub_b = (int)cdiv(L.n_in, TU) * (TM / TP);
-        while (S.lg_bks < 5 && qs_items(nsub_b, S.lg_bks + 1) <= NT && (R >> (S.lg_bks + 1)) >= 2) ++S.lg_bks;
-        S.bkl = (int)cdiv(R, 1 << S.lg_bks);
-        S.cp_dr = NT / L.n_in; S.cp_di = NT % L.n_in;
-        S.fwd_c0 = c; c += S.nch;
-        S.bwd_c0 = -1;
-    }
-    if (want_grad)
-        for (int l = nl - 1; l >= 1; --l) { P->SL[l].bwd_c0 = c; c += P->SL[l].nch; }
-    P->n_chunks = c;
-    P->slot_elems = (int)slot;
-    P->ring_off = (int)head;
-    P->act_off = P->ring_off + QS_STAGES * (int)slot * elem;
-    P->da_off = P->act_off + (want_grad ? row * P->lda * elem : 0);
-    P->act_elems = (int)act_elems;
-    P->smem_bytes = P->act_off + act_elems * elem;
-    return P->smem_bytes;
-}
-
-struct QbLaunch { QbPlan plan; int S; long long pts_per_split; bool streamed; QbStreamPlan sp; };
-
-// Networks whose weights do not fit next to one tile of activations: the layer-streamed kernels (qb_stream.cuh).
-// The tile is chosen so that the rows of one chunk times its points fill the thread tiles of the block with as little
-// split of the reduction as possible (larger tiles at equal fill: fewer passes of the weights through the ring).
-static int make_stream_launch(const qb_net_t* net, int dtype, bool want_grad, long long K, long long N, bool force_single,
-                              QbLaunch* out) {
-    const int TU = dtype == QB_F64 ? 4 : 8, TP = 4;
-    const int cands32[] = {128, 64, 32, 16}, cands64[] = {128, 64, 32, 16, 8};
-    const int* cands = dtype == QB_F64 ? cands64 : cands32;
-    const int nc = dtype == QB_F64 ? 5 : 4, mintm = cands[nc - 1];
-    const int cap = std::max(mintm, rup((int)std::min<long long>(N, 256), mintm));
-    QbStreamPlan tmp;
-    int pick = -1;
-    long long best = -1;
-    for (int c = 0; c < nc; ++c) {
-        const int TM = cands[c];
-        if (TM > cap) continue;
-        if (stream_plan_for_tm(net, dtype, want_grad, TM, &tmp) < 0) continue;
-        long long fill = (long long)QS_THREADS * TU * TP;
-        for (int l = 0; l < net->n_layers; ++l)
-            if (net->layers[l].n_out > TU) fill = std::min<long long>(fill, (long long)tmp.SL[l].R * TM);
-        if (fill > best) { best = fill; pick = TM; }
-    }
-    if (pick < 0)
-        return qb_fail("network too large for the layer-streamed path: the activations of one %s%lld-point tile exceed 227 KB of shared memory",
-                       "", mintm);
-    stream_plan_for_tm(net, dtype, want_grad, pick, &out->sp);
-    out->streamed = true;
-    const int TM = pick;
-    long long S = 1;
-    if (!force_single) {
-        // same rule as the resident kernels; with a gradient, the [K,S,P] partial rows stay under 256 MB
-        const long long target = (long long)QB_NUM_SMS * 8;
-        if (K < target) S = std::max<long long>(1, std::min(cdiv(N, 2LL * TM), cdiv(target, K)));
-        if (want_grad) S = std::min<long long>(S, std::max<long long>(1, (256LL << 20) / (K * net->n_params * (dtype == QB_F64 ? 8 : 4))));
-    }
-    long long pps = rup((int)cdiv(N, S), TM);
-    S = cdiv(N, pps);
-    out->S = (int)S; out->pts_per_split = pps;
-    return 0;
-}
-
-static int make_launch(const qb_net_t* net, int dtype, bool want_grad, long long K, long long N, bool force_single,
-                       QbLaunch* out) {
-    if (validate_net(net)) return -1;
-    if (dtype != QB_F32 && dtype != QB_F64) return qb_fail("unknown dtype");
-    if (K < 1 || N < 1) return qb_fail("K and N must be positive");
-    const int cands32[] = {256, 128, 64, 32}, cands64[] = {128, 64, 32, 16};
-    const int* cands = dtype == QB_F64 ? cands64 : cands32;
-    const int mintm = cands[3];
-    const int cap = std::max(mintm, rup((int)std::min<long long>(N, 256), mintm));
-    int forced = env_int("QB_TM", 0);
-    // Score every tile size by resident warps per SM (limited by shared memory, 128 registers/thread and 2048
-    // threads); ties go to more, smaller blocks for the value kernel (their MUFU / FMA phases overlap better,
-    // measured on config 5) and to larger tiles for the gradient kernel (fewer block barriers per point).
-    // Gradient only: if nothing fits, drop the shared copy of W used by back-propagation (read from global).
-    int pick = -1, best_score = -1;
-    bool wr_global = false;
-    QbPlan tmp;
-    bool any_poly = false;
-    for (int l = 0; l < net->n_layers; ++l) any_poly = any_poly || net->layers[l].n_terms > 1;
-    for (int g = (want_grad && env_int("QB_WR_GLOBAL", 0)) ? 1 : 0; g < 2 && pick < 0; ++g) {
-        if (g == 1 && (!want_grad || any_poly)) break;      // the global-W fallback reads theta directly: no polynomial terms
-        for (int c = 0; c < 4; ++c) {
-            int TM = cands[c];
-            if (forced) TM = forced;
-            else if (TM > cap) continue;
-            const long long b = plan_for_tm(net, dtype, want_grad, TM, &tmp, g == 1);
-            if (b <= QB_SMEM_MAX) {
-                const int by_smem = (int)(QB_SMEM_SM / (b + 1024));
-                const int by_regs = 512 / tmp.nthreads;
-                const int blocks = std::max(1, std::min(std::min(by_smem, by_regs), 16));
-                int score;
-                if (want_grad) {
-                    // gradient kernel (block barriers per layer): the largest tile that still leaves two blocks per SM,
-                    // else the largest tile that fits at all
-                    score = (blocks >= 2 ? 1000 : 0) + (3 - c);
-                } else {
-                    score = blocks * (tmp.nthreads / 32) * 16 + std::min(blocks, 8);
-                }
-                if (score > best_score) { best_score = score; pick = TM; wr_global = (g == 1); }
-            }
-            if (forced) break;
-        }
-    }
-    out->streamed = false;
-    if (pick < 0) {
-        if (forced) return qb_fail("network too large for the fused shared-memory path (weights + one tile exceed 227 KB)");
-        memset(&out->plan, 0, sizeof(out->plan));
-        return make_stream_launch(net, dtype, want_grad, K, N, force_single, out);
-    }
-    plan_for_tm(net, dtype, want_grad, pick, &out->plan, wr_global);
-    const int TM = out->plan.TM;
-    long long S = 1;
-    if (!force_single) {
-        // few chains: split the data axis so that the grid is >= 8 waves of one block per SM (tail effect < 10 %),
-        // keeping at least two tiles per block; partial sums / gradients are combined in fixed order by k_finalize
-        const long long target = (long long)QB_NUM_SMS * 8;
-        if (K < target) S = std::max<long long>(1, std::min(cdiv(N, 2LL * TM), cdiv(target, K)));
-        S = env_int("QB_SPLIT", (int)S);
-        if (S < 1) S = 1;
-    }
-    long long pps = rup((int)cdiv(N, S), TM);
-    S = cdiv(N, pps);
-    out->S = (int)S; out->pts_per_split = pps;
-    return 0;
-}
-
-
-// Tensor-core (tcgen05 3xTF32) plan for the value path; returns false when the network is not eligible:
-// fp32, >= 3 layers, no residual layers, n_in <= 15, hidden widths multiples of 16 (<= 128), <= 4 outputs.
-// allow_v3: 1 = the caller can run the warp-specialised kernels (qb_value_tc3.cu); 2 = the chain kernel (hidden width 64
-// only, with room for the chain state, 3 P floats, in shared memory); 3 = kernel 4
-static bool make_tc_plan(const qb_net_t* net, int dtype, QbTcPlan* tp, int allow_v3 = 0) {
-    memset(tp, 0, sizeof(*tp));
-    if (dtype != QB_F32 || env_int("QB_NO_TC", 0)) return false;
-    const int nl = net->n_layers;
-    if (nl < 3 || net->in_dim > 15 || net->out_dim > 4) return false;
-    int kmax = 0, nmax = 0;
-    for (int l = 0; l < nl; ++l) {
-        const qb_layer_t& S = net->layers[l];
-        if (S.res_step != 0.0 || S.n_terms > 1) return false;
-        if (l < nl - 1 && (S.n_out % 16 != 0 || S.n_out < 16 || S.n_out > 128)) return false;
-        if (l >= 1 && l < nl - 1) { kmax = std::max(kmax, S.n_in); nmax = std::max(nmax, S.n_out); }
-    }
-    const bool pipe = nl == 3 && net->layers[0].act == net->layers[1].act &&
-                      (net->layers[0].act == QB_ACT_TANH || net->layers[0].act == QB_ACT_RELU) && !env_int("QB_NO_PIPE", 0);
-    const int grp = std::max(kmax, nmax) > 64 ? 4 : 2;       // column groups = warps per quarter of the tile
-    const int cols = 2 * kmax + (pipe ? 2 : 1) * nmax;       // pipelined path: the accumulator is double-buffered
-    if (cols > 512) return false;
-    tp->n_layers = nl; tp->in_dim = net->in_dim; tp->out_dim = net->out_dim; tp->n_params = net->n_params;
-    tp->ni = (net->in_dim < 4 && !(pipe && grp == 4)) ? 4 : 16;
-    if (pipe && grp == 4 && net->in_dim <= 11 && net->layers[0].act == QB_ACT_TANH) tp->ni = 12;   // config 3: 10 inputs + bias
-    tp->h0 = net->layers[0].n_out; tp->kl = net->layers[nl - 1].n_in;
-    tp->act0 = net->layers[0].act; tp->act_last = net->layers[nl - 1].act; tp->final_exp = net->final_exp;
-    tp->w0_off = net->layers[0].w_off; tp->b0_off = net->layers[0].b_off;
-    tp->wl_off = net->layers[nl - 1].w_off; tp->bl_off = net->layers[nl - 1].b_off;
-    tp->a_lo_col = kmax; tp->d_col = 2 * kmax;
-    tp->pipe = pipe ? grp : 0;
-    tp->tmem_cols = cols <= 32 ? 32 : cols <= 64 ? 64 : cols <= 128 ? 128 : cols <= 256 ? 256 : 512;
-    int off = QB_TC_HDR_BYTES;
-    for (int l = 1; l < nl - 1; ++l) {
-        const qb_layer_t& S = net->layers[l];
-        QbTcLayer& L = tp->L[l];
-        L.n_in = S.n_in; L.n_out = S.n_out; L.w_off = S.w_off; L.b_off = S.b_off; L.act = S.act;
-        L.bhi = off; off += S.n_in * S.n_out * 4;
-        L.blo = off; off += S.n_in * S.n_out * 4;
-    }
-    tp->fl_base = off;
-    int f = 0;
-    tp->w0 = f; f += tp->h0 * tp->ni;
-    for (int l = 1; l < nl - 1; ++l) { tp->L[l].bias = f; f += rup(tp->L[l].n_out, 4); }
-    tp->wl = f; f += rup(tp->out_dim * tp->kl, 4);
-    tp->bl = f; f += 4;
-    long long bytes = (long long)off + (long long)f * 4;
-    bytes = (bytes + 15) / 16 * 16;
-    tp->ybuf = (int)bytes; bytes += 2 * 3 * 4 * 128 * 4;
-    tp->nthreads = tp->pipe ? 128 * tp->pipe : 128;
-    if (bytes > QB_SMEM_MAX) return false;
-    // tensor memory is 512 columns per SM: request enough shared memory that no more blocks than 512/tmem_cols
-    // become resident (a further block would spin in tcgen05.alloc)
-    const int max_blocks = 512 / tp->tmem_cols;
-    const long long floor_bytes = QB_SMEM_SM / (max_blocks + 1) + 1;
-    tp->smem_bytes = (int)std::min<long long>(QB_SMEM_MAX, std::max(bytes, floor_bytes));
-    const int v3h = allow_v3 ? qb_tc_v3_shape(*tp) : 0;
-    if (v3h && net->layers[1].act == QB_ACT_TANH && !env_int("QB_NO_V3", 0) && !(allow_v3 == 2 && v3h != 64)) {
-        // warp-specialised path (qb_tc3.cuh): 4 H/32 compute warps + 1 issue warp, 4 H tensor-memory columns, own layout
-        const int H = v3h, K0 = H == 64 ? 8 : 16, G = H / 32;
-        tp->v3 = H == 64 ? 1 : 2; tp->nthreads = 128 * G + 32; tp->tmem_cols = 4 * H;
-        int o = QB_TC_HDR_BYTES;
-        tp->v3_w1 = o; o += 3 * H * H * 2;
-        tp->v3_w0 = o; o += 2 * H * K0 * 4;
-        tp->v3_x = o; o += 3 * 2 * 128 * K0 * 4;
-        tp->fl_base = o;
-        tp->L[1].bias = 0; tp->wl = H; tp->bl = 2 * H; tp->v3_c1 = 2 * H + 4;
-        o += (2 * H + 8) * 4;
-        tp->ybuf = o; o += 4 * (G - 1) * 128 * 4;
-        tp->v3_xbar = o; o += 32;
-        tp->v3_state = o;
-        if (allow_v3 == 2) o += 3 * ((net->n_params + 3) / 4 * 4) * 4;
-        const int max_blocks3 = 512 / tp->tmem_cols;
-        tp->smem_bytes = (int)std::max<long long>(o, QB_SMEM_SM / (max_blocks3 + 1) + 1);
-        if (tp->smem_bytes > (QB_SMEM_SM - 1024 * max_blocks3) / max_blocks3) return make_tc_plan(net, dtype, tp, 0);     // the blocks must fit
-    }
-    return true;
-}
 
 template <typename K>
 static int set_smem(K kernel, long long bytes) {
@@ -656,21 +199,19 @@ static int run_eval(const qb_net_t* net, int dtype, const void* theta, int64_t K
                     int64_t x_stride = 0, int64_t y_stride = 0) {
     const bool want_grad = grad != nullptr;
     QbLaunch L;
-    if (make_launch(net, dtype, want_grad, K, data->n, false, &L)) return -1;
-    const size_t need = qb_eval_workspace_bytes(net, dtype, K, data->n, want_grad);
-    if (ws_bytes < need || (need && !ws)) return qb_fail("workspace too small%s (need %lld bytes)", "", (long long)need);
+    if (plan_eval(net, dtype, want_grad, K, data->n, false, &L)) return -1;
+    if (ws_bytes < L.ws_bytes || (L.ws_bytes && !ws)) return qb_fail("workspace too small%s (need %lld bytes)", "", (long long)L.ws_bytes);
     EvalArgs<T> a;
     a.theta = (const T*)theta; a.x = (const T*)data->x; a.y = (const T*)data->y;
     a.xs = x_stride; a.ys = y_stride;
     a.K = K; a.N = data->n; a.S = L.S; a.pps = L.pts_per_split;
     a.part = (double*)ws;
     a.grad = (T*)grad;
-    const size_t part_bytes = ((size_t)K * L.S * sizeof(double) + 255) / 256 * 256;
-    a.gpart = (L.S > 1 && want_grad) ? (T*)((char*)ws + part_bytes) : nullptr;
+    a.gpart = (L.S > 1 && want_grad) ? (T*)((char*)ws + L.gpart_off) : nullptr;
     a.lp = lp; a.lk = lik_dev(lik);
     a.xsplit = nullptr;
     dim3 grid((unsigned)K, (unsigned)L.S);
-    if (L.streamed) {
+    if (L.path == QB_PATH_STREAM) {
         const dim3 sgrid((unsigned)(K * L.S));
         if (want_grad) {
             if (set_smem(k_logpost_stream<T, true>, L.sp.smem_bytes)) return -2;
@@ -679,29 +220,22 @@ static int run_eval(const qb_net_t* net, int dtype, const void* theta, int64_t K
             if (set_smem(k_logpost_stream<T, false>, L.sp.smem_bytes)) return -2;
             k_logpost_stream<T, false><<<sgrid, QS_THREADS, L.sp.smem_bytes, st>>>(L.sp, a);
         }
+    } else if (L.path == QB_PATH_TG8) {
+        // tanh nets of width 64 / 128: fp16-split operands, scaled with max |x|, max |y| (the workspace's tail scratch)
+        if (launch_grad_tc128<T>(L.t8, a, (char*)ws + L.tail_off, grid, st)) return -2;
+        g_launches += 1;
+    } else if (L.path == QB_PATH_TCG) {
+        if (launch_grad_tc<T>(L.tg, a, grid, st)) return -2;
+    } else if (L.path != QB_PATH_CUDA) {
+        // hot shape with shared data: x goes to the kernel as ready-made operand tiles in the workspace's tail scratch
+        if (L.tp.v3 && x_stride == 0) a.xsplit = (const T*)((char*)ws + L.tail_off);
+        if (launch_logpost_tc<T>(L.tp, a, grid, st)) return -2;
     } else if (want_grad) {
-        QbTcgPlan tg;
-        QbTg8Plan t8;
-        if (qb_tg8_make_plan(net, dtype, &t8)) {
-            // tanh nets of width 64 / 128: fp16-split operands, scaled with max |x|, max |y| (8 bytes at the end of the workspace)
-            if (launch_grad_tc128<T>(t8, a, (char*)ws + need - QB_TG8_SCRATCH_BYTES, grid, st)) return -2;
-            g_launches += 1;
-        } else if (qb_tcg_make_plan(net, dtype, &tg)) {
-            if (launch_grad_tc<T>(tg, a, grid, st)) return -2;
-        } else {
-            if (set_smem(k_logpost_grad<T>, L.plan.smem_bytes)) return -2;
-            k_logpost_grad<T><<<grid, L.plan.nthreads, L.plan.smem_bytes, st>>>(L.plan, a);
-        }
+        if (set_smem(k_logpost_grad<T>, L.plan.smem_bytes)) return -2;
+        k_logpost_grad<T><<<grid, L.plan.nthreads, L.plan.smem_bytes, st>>>(L.plan, a);
     } else {
-        QbTcPlan tp;
-        if (make_tc_plan(net, dtype, &tp, 1)) {
-            // hot shape with shared data: x goes to the kernel as ready-made operand tiles at the end of the workspace
-            if (tp.v3 && x_stride == 0) a.xsplit = (const T*)((char*)ws + need - qb_tc3_xsplit_bytes(data->n, tp.v3 == 1 ? 8 : 16));
-            if (launch_logpost_tc<T>(tp, a, grid, st)) return -2;
-        } else {
-            if (set_smem(k_logpost<T>, L.plan.smem_bytes)) return -2;
-            k_logpost<T><<<grid, L.plan.nthreads, L.plan.smem_bytes, st>>>(L.plan, a);
-        }
+        if (set_smem(k_logpost<T>, L.plan.smem_bytes)) return -2;
+        k_logpost<T><<<grid, L.plan.nthreads, L.plan.smem_bytes, st>>>(L.plan, a);
     }
     QB_CUDA(cudaGetLastError());
     int fin_mode = want_grad ? 1 : 0;
@@ -714,49 +248,6 @@ static int run_eval(const qb_net_t* net, int dtype, const void* theta, int64_t K
     k_finalize<T><<<(unsigned)K, 128, 0, st>>>(a, net->n_params, fin_mode);
     QB_CUDA(cudaGetLastError());
     g_launches += 2;
-    return 0;
-}
-
-extern "C" size_t qb_eval_workspace_bytes(const qb_net_t* net, int dtype, int64_t K, int64_t N, int want_grad) {
-    QbLaunch L;
-    if (make_launch(net, dtype, want_grad != 0, K, N, false, &L)) return 0;
-    size_t b = ((size_t)K * L.S * sizeof(double) + 255) / 256 * 256;
-    if (want_grad && L.S > 1) b += (size_t)K * L.S * net->n_params * (dtype == QB_F64 ? 8 : 4);
-    if (L.streamed) return b;
-    QbTcPlan tp;
-    if (!want_grad && make_tc_plan(net, dtype, &tp, 1) && tp.v3) b = (b + 255) / 256 * 256 + qb_tc3_xsplit_bytes(N, tp.v3 == 1 ? 8 : 16);
-    QbTcgPlan tg;
-    QbTg8Plan t8;
-    (void)tg;
-    if (want_grad && qb_tg8_make_plan(net, dtype, &t8)) b = (b + 255) / 256 * 256 + QB_TG8_SCRATCH_BYTES;
-    return b;
-}
-
-extern "C" int qb_plan_info(const qb_net_t* net, int dtype, int64_t K, int64_t N, int want_grad, int64_t* out) {
-    QbLaunch L;
-    if (make_launch(net, dtype, want_grad != 0, K, N, false, &L)) return -1;
-    out[0] = L.plan.TM; out[1] = L.plan.nthreads; out[2] = L.plan.smem_bytes; out[3] = L.S;
-    out[4] = (int64_t)K * L.S; out[5] = L.plan.inplace; out[6] = 0; out[7] = 0;
-    if (L.streamed) {
-        // CUDA cores, weights streamed through shared memory (qb_stream.cuh): out[6] = 5
-        out[0] = L.sp.TM; out[1] = QS_THREADS; out[2] = L.sp.smem_bytes; out[5] = 0; out[6] = 5;
-        return 0;
-    }
-    QbTcgPlan tg;
-    QbTg8Plan t8;
-    if (want_grad && qb_tg8_make_plan(net, dtype, &t8)) {
-        // gradient path on the tensor cores, fp16-split operands (qb_tg8.cuh: tanh nets of width 64 / 128): out[6] = 4
-        out[0] = 128; out[1] = t8.nthreads; out[2] = t8.smem_bytes; out[5] = 0; out[6] = 4; out[7] = t8.tmem_cols;
-    } else if (want_grad && qb_tcg_make_plan(net, dtype, &tg)) {
-        // gradient path on the tensor cores, 3xTF32 (qb_tcg.cuh: widths 32 / 64, tanh / relu): out[6] = 3
-        out[0] = 128; out[1] = tg.nthreads; out[2] = tg.smem_bytes; out[5] = 0; out[6] = 3; out[7] = tg.tmem_cols;
-    }
-    QbTcPlan tp;
-    if (!want_grad && make_tc_plan(net, dtype, &tp, 1)) {
-        // value path on the tensor cores: 128-point tiles, 128 or 256 threads, out[6] = 1 + pipelined flag,
-        // out[7] = tensor-memory columns per block
-        out[0] = 128; out[1] = tp.nthreads; out[2] = tp.smem_bytes; out[5] = 0; out[6] = tp.pipe ? 2 : 1; out[7] = tp.tmem_cols;
-    }
     return 0;
 }
 
@@ -787,106 +278,6 @@ extern "C" int qb_logpost_members(const qb_net_t* net, int dtype, const void* th
 // =================================================================================================
 // kernel 5: Hessian-vector products (qb_hvp.cuh)
 // =================================================================================================
-// Plan for tile size TM: every layer in GEMM mode with TU x 4 thread tiles; returns the shared-memory bytes.
-static long long hvp_plan_for_tm(const qb_net_t* net, int dtype, int TM, QbHvpPlan* H) {
-    const int elem = dtype == QB_F64 ? 8 : 4;
-    const int TU = dtype == QB_F64 ? 4 : 8, LDPAD = dtype == QB_F64 ? 2 : 4, PV = dtype == QB_F64 ? 2 : 4, TP = 4;
-    const int nl = net->n_layers, PG = TM / TP;
-    memset(H, 0, sizeof(*H));
-    QbPlan* P = &H->P;
-    P->n_layers = nl; P->in_dim = net->in_dim; P->out_dim = net->out_dim;
-    P->n_params = net->n_params; P->final_exp = net->final_exp;
-    P->TM = TM; P->lda = TM + LDPAD; P->want_grad = 1; P->elem_size = elem; P->tpg = TP;
-    int woff = 0, max_items = 0, dmax = 0;
-    for (int l = 0; l < nl; ++l) {
-        const qb_layer_t& S = net->layers[l];
-        QbLayerPlan& L = P->L[l];
-        L.n_in = S.n_in; L.n_out = S.n_out; L.n_in_pad = rup(S.n_in, TU); L.n_out_pad = rup(S.n_out, TU);
-        L.w_off = S.w_off; L.b_off = S.b_off; L.act = S.act; L.res_step = S.res_step; L.has_res = S.res_step != 0.0;
-        L.n_terms = S.n_terms > 1 ? S.n_terms : 0; L.w_stride = S.w_stride; L.b_stride = S.b_stride;
-        for (int m = 0; m < QB_MAX_TERMS; ++m) L.coef[m] = S.coef[m];
-        L.mode = QB_MODE_GEMM; L.nj = 4;
-        if (L.has_res) { P->has_res = 1; dmax = std::max(dmax, L.n_out_pad); }
-        L.ug_shift = L.ugi_shift = L.ig_shift = -1;
-        for (int sft = 0; sft < 16; ++sft) {
-            if ((1 << sft) == L.n_out_pad / TU) L.ug_shift = sft;
-            if ((1 << sft) == L.n_in_pad / TU) L.ugi_shift = sft;
-            if ((1 << sft) == (S.n_in + 3) / 4) L.ig_shift = sft;
-        }
-        max_items = std::max(max_items, (L.n_out_pad / TU) * PG);
-        if (l > 0) max_items = std::max(max_items, (L.n_in_pad / TU) * PG);
-        // [W^T ; V^T], [b ; v_b], and for l > 0 [W ; V] (qb_hvp.cuh)
-        L.wt_off = woff; woff += rup((L.n_in_pad + L.n_in) * L.n_out_pad, 4);
-        L.bias_off = woff; woff += rup(2 * L.n_out_pad, 4);
-        L.wr_off = -1;
-        if (l > 0) { L.wr_off = woff; woff += rup((L.n_out_pad + L.n_out) * L.n_in_pad, 4); }
-    }
-    P->w_elems = woff;
-    const int nthreads = std::min(256, std::max(64, rup(max_items, 32)));
-    P->nthreads = nthreads;
-    // activation rows: per layer boundary the tangent rows, then the activation rows
-    int row = 0;
-    for (int b = 0; b <= nl; ++b) {
-        const int npad = b == 0 ? P->L[0].n_in_pad : P->L[b - 1].n_out_pad;
-        row += npad;                                   // tangent rows
-        if (b < nl) P->L[b].row_in = row;
-        if (b > 0) P->L[b - 1].row_out = row;
-        row += npad;
-    }
-    P->d_row = dmax ? row : -1; row += dmax;
-    H->dd_row = dmax ? row : -1; row += dmax;
-    P->total_rows = row;
-    P->buf_rows = row;
-    for (int l = 0; l < nl; ++l) {
-        QbLayerPlan& L = P->L[l];
-        const int patches = ((L.n_out + 3) / 4) * ((L.n_in + 3) / 4);
-        int C = 1;
-        while (C < 32 && patches * C * 2 <= nthreads && TM / (C * 2) >= PV) C *= 2;
-        L.dw_chunks = C;
-        L.c_shift = 0;
-        while ((1 << L.c_shift) < C) ++L.c_shift;
-        H->LA[l] = L; H->LA[l].row_out = L.row_out - L.n_out_pad;
-        H->LB[l] = L; H->LB[l].row_in = L.row_in - L.n_in_pad; H->LB[l].b_off = -1;
-    }
-    // one pad row: the double-buffered hot loop prefetches one row past the end
-    P->smem_bytes = (long long)woff * elem + (long long)(row + 1) * P->lda * elem;
-    return P->smem_bytes;
-}
-
-struct QbHvpLaunch { QbHvpPlan H; int S; long long pps; };
-
-static int make_hvp_launch(const qb_net_t* net, int dtype, long long K, long long N, QbHvpLaunch* out) {
-    if (validate_net(net)) return -1;
-    if (dtype != QB_F32 && dtype != QB_F64) return qb_fail("unknown dtype");
-    if (K < 1 || N < 1) return qb_fail("K and N must be positive");
-    const int cands32[] = {128, 64, 32, 16}, cands64[] = {64, 32, 16, 8};
-    const int* cands = dtype == QB_F64 ? cands64 : cands32;
-    const int mintm = cands[3];
-    const int cap = std::max(mintm, rup((int)std::min<long long>(N, 256), mintm));
-    // The largest tile that fits.  Measured on a B200 (DESIGN.md section 4f, profiles/r4_hessian_bench_*.json): more,
-    // smaller blocks per SM lose, e.g. fp32 config 2 at TM 16 (six 64-thread blocks per SM) reaches 0.06 of the FMA peak
-    // against 0.20 at TM 128, and fp32 config 5 at TM 16 0.07 against 0.30 at TM 128.
-    int pick = -1;
-    for (int c = 0; c < 4 && pick < 0; ++c) {
-        const int TM = cands[c];
-        if (TM <= cap && hvp_plan_for_tm(net, dtype, TM, &out->H) <= QB_SMEM_MAX) pick = TM;
-    }
-    if (pick < 0) {
-        hvp_plan_for_tm(net, dtype, mintm, &out->H);
-        return qb_fail("network too large for the Hessian-vector kernel: its weights, one direction and a %s%lld-point tile "
-                       "exceed 227 KB of shared memory (use the diagonal curvature)", "", mintm);
-    }
-    hvp_plan_for_tm(net, dtype, pick, &out->H);
-    // few directions: split the data axis as kernel 2 does; the [K,S,P] partial rows stay under 256 MB
-    long long S = 1;
-    const long long target = (long long)QB_NUM_SMS * 8;
-    if (K < target) S = std::max<long long>(1, std::min(cdiv(N, 2LL * pick), cdiv(target, K)));
-    S = std::min<long long>(S, std::max<long long>(1, (256LL << 20) / (K * net->n_params * (dtype == QB_F64 ? 8 : 4))));
-    const long long pps = rup((int)cdiv(N, S), pick);
-    out->S = (int)cdiv(N, pps); out->pps = pps;
-    return 0;
-}
-
 template <typename T> struct HvpArgs {
     const T* theta; const T* v; long long col0;
     const T* x; const T* y;
@@ -928,27 +319,12 @@ __global__ void __launch_bounds__(256) k_hvp_finalize(const HvpArgs<T> a, long l
     a.hv[e] = h;
 }
 
-extern "C" size_t qb_hvp_workspace_bytes(const qb_net_t* net, int dtype, int64_t K, int64_t N) {
-    if (K == 0) return 0;
-    QbHvpLaunch L;
-    if (make_hvp_launch(net, dtype, K, N, &L)) return 0;
-    return L.S > 1 ? (size_t)K * L.S * net->n_params * (dtype == QB_F64 ? 8 : 4) : 0;
-}
-
-extern "C" int qb_hvp_plan_info(const qb_net_t* net, int dtype, int64_t K, int64_t N, int64_t* out) {
-    QbHvpLaunch L;
-    if (make_hvp_launch(net, dtype, K, N, &L)) return -1;
-    out[0] = L.H.P.TM; out[1] = L.H.P.nthreads; out[2] = L.H.P.smem_bytes; out[3] = L.S; out[4] = (int64_t)K * L.S;
-    return 0;
-}
-
 template <typename T>
 static int run_hvp(const qb_net_t* net, int dtype, const void* theta, const void* v, int64_t col0, int64_t K,
                    const qb_data_t* data, const qb_lik_t* lik, void* hv, void* ws, size_t ws_bytes, cudaStream_t st) {
     QbHvpLaunch L;
     if (make_hvp_launch(net, dtype, K, data->n, &L)) return -1;
-    const size_t need = qb_hvp_workspace_bytes(net, dtype, K, data->n);
-    if (ws_bytes < need || (need && !ws)) return qb_fail("workspace too small%s (need %lld bytes)", "", (long long)need);
+    if (ws_bytes < L.ws_bytes || (L.ws_bytes && !ws)) return qb_fail("workspace too small%s (need %lld bytes)", "", (long long)L.ws_bytes);
     HvpArgs<T> a;
     a.theta = (const T*)theta; a.v = (const T*)v; a.col0 = col0;
     a.x = (const T*)data->x; a.y = (const T*)data->y;
@@ -984,74 +360,6 @@ extern "C" int qb_logpost_hvp(const qb_net_t* net, int dtype, const void* theta,
 // =================================================================================================
 // kernel 6: Kronecker factors of the per-point empirical Fisher (qb_kfac.cuh)
 // =================================================================================================
-// qb_dw_accumulate's split of one re-pointed factor pass (as in plan_for_tm, for the pass's own shape)
-static void kfac_dw_split(QbLayerPlan& L, int nthreads, int TM, int PV) {
-    const int patches = ((L.n_out + 3) / 4) * ((L.n_in + 3) / 4);
-    int C = 1;
-    while (C < 32 && patches * C * 2 <= nthreads && TM / (C * 2) >= PV) C *= 2;
-    L.dw_chunks = C;
-    L.c_shift = 0;
-    while ((1 << L.c_shift) < C) ++L.c_shift;
-    L.ig_shift = -1;
-    for (int sft = 0; sft < 16; ++sft)
-        if ((1 << sft) == (L.n_in + 3) / 4) L.ig_shift = sft;
-}
-
-struct QbKfacLaunch { QbKfacPlan K; int S; long long pps; };
-
-// Kernel 2's resident CUDA-core plan for one theta, the factor passes of every layer, and the N-split: one block per
-// split, the [S, F] partial rows (dtype) under 256 MB.
-static int make_kfac_launch(const qb_net_t* net, int dtype, long long N, QbKfacLaunch* out) {
-    if (validate_net(net)) return -1;
-    if (dtype != QB_F32 && dtype != QB_F64) return qb_fail("unknown dtype");
-    for (int l = 0; l < net->n_layers; ++l) {
-        const qb_layer_t& S = net->layers[l];
-        if (S.n_terms > 1)
-            return qb_fail("Kronecker factors: layer %s%lld has polynomial-in-depth weights (n_terms >= 2); every layer "
-                           "must own its weights", "", l);
-        for (int m = 0; m < l; ++m)
-            if (net->layers[m].w_off == S.w_off)
-                return qb_fail("Kronecker factors: layer %s%lld shares its weights with an earlier layer; every layer must "
-                               "own its weights", "", l);
-    }
-    QbLaunch L;
-    if (make_launch(net, dtype, true, 1, N, true, &L)) return -1;
-    if (L.streamed)
-        return qb_fail("Kronecker factors: the network's weights do not fit in shared memory next to one tile of "
-                       "activations, and the layer-streamed path (plan code 5) has no factor kernel");
-    memset(&out->K, 0, sizeof(out->K));
-    out->K.P = L.plan;
-    const QbPlan& P = out->K.P;
-    const int PV = dtype == QB_F64 ? 2 : 4;
-    int off = 0;
-    for (int l = 0; l < P.n_layers; ++l) {
-        const QbLayerPlan& B = P.L[l];
-        QbLayerPlan& A = out->K.LA[l];
-        A = B;
-        A.n_out = B.n_in; A.n_out_pad = B.n_in_pad; A.row_out = B.row_in;
-        A.n_terms = 0;
-        A.w_off = off; off += B.n_in * B.n_in;
-        A.b_off = -1;
-        if (B.b_off >= 0) { A.b_off = off; off += B.n_in; }
-        kfac_dw_split(A, P.nthreads, P.TM, PV);
-        QbLayerPlan& G = out->K.LG[l];
-        G = B;
-        G.n_in = B.n_out; G.n_in_pad = B.n_out_pad; G.row_in = B.row_out;
-        G.n_terms = 0;
-        G.w_off = off; off += B.n_out * B.n_out;
-        G.b_off = -1;
-        kfac_dw_split(G, P.nthreads, P.TM, PV);
-    }
-    out->K.n_factors = off;
-    const int TM = P.TM;
-    const long long row_bytes = (long long)off * (dtype == QB_F64 ? 8 : 4);
-    long long S = std::max<long long>(1, std::min(cdiv(N, 2LL * TM), (long long)QB_NUM_SMS * 8));
-    S = std::min<long long>(S, std::max<long long>(1, (256LL << 20) / row_bytes));
-    const long long pps = rup((int)cdiv(N, S), TM);
-    out->S = (int)cdiv(N, pps); out->pps = pps;
-    return 0;
-}
-
 template <typename T> struct KfacArgs {
     const T* theta; const T* x; const T* y;
     long long N; int S; long long pps;
@@ -1080,20 +388,6 @@ __global__ void __launch_bounds__(256) k_kfac_finalize(const KfacArgs<T> a, int 
     a.factors[e] = v;
 }
 
-extern "C" size_t qb_kfac_workspace_bytes(const qb_net_t* net, int dtype, int64_t N) {
-    if (N <= 0) return 0;
-    QbKfacLaunch L;
-    if (make_kfac_launch(net, dtype, N, &L)) return 0;
-    return (size_t)L.S * L.K.n_factors * (dtype == QB_F64 ? 8 : 4);
-}
-
-extern "C" int qb_kfac_plan_info(const qb_net_t* net, int dtype, int64_t N, int64_t* out) {
-    QbKfacLaunch L;
-    if (make_kfac_launch(net, dtype, std::max<int64_t>(N, 1), &L)) return -1;
-    out[0] = L.K.P.TM; out[1] = L.K.P.nthreads; out[2] = L.K.P.smem_bytes; out[3] = L.S; out[4] = L.K.n_factors;
-    return 0;
-}
-
 template <typename T>
 static int run_kfac(const qb_net_t* net, int dtype, const void* theta, const qb_data_t* data, const qb_lik_t* lik,
                     double* factors, void* ws, size_t ws_bytes, cudaStream_t st) {
@@ -1103,8 +397,7 @@ static int run_kfac(const qb_net_t* net, int dtype, const void* theta, const qb_
         QB_CUDA(cudaMemsetAsync(factors, 0, (size_t)L.K.n_factors * sizeof(double), st));
         return 0;
     }
-    const size_t need = (size_t)L.S * L.K.n_factors * sizeof(T);
-    if (ws_bytes < need || !ws) return qb_fail("workspace too small%s (need %lld bytes)", "", (long long)need);
+    if (ws_bytes < L.ws_bytes || !ws) return qb_fail("workspace too small%s (need %lld bytes)", "", (long long)L.ws_bytes);
     KfacArgs<T> a;
     a.theta = (const T*)theta; a.x = (const T*)data->x; a.y = (const T*)data->y;
     a.N = data->n; a.S = L.S; a.pps = L.pps;
@@ -1536,23 +829,21 @@ static int run_hmc(const qb_net_t* net, int dtype, const qb_data_t* data, const 
                    qb_hmc_t* hm, const qb_rng_t* rng, const qb_record_t* rec, int64_t t_start, int64_t nsteps,
                    int init_lp, cudaStream_t st) {
     QbLaunch L;
-    if (make_launch(net, dtype, true, ch->K, data->n, true, &L)) return -1;
+    if (plan_eval(net, dtype, true, ch->K, data->n, true, &L)) return -1;
     if (!hm->grad_cur || !hm->mom || !hm->prop || !hm->grad_prop) return qb_fail("hmc state has NULL arrays");
     if (hm->method == 0 && hm->L < 1) return qb_fail("HMC needs L >= 1");
     ChainArgs<T> c; fill_chain_args<T>(c, data, lik, ch, rng, rec, t_start, nsteps, init_lp);
     HmcArgs<T> h;
     h.method = hm->method; h.L = hm->L; h.eps = hm->epsilon;
     h.gcur = (T*)hm->grad_cur; h.mom = (T*)hm->mom; h.prop = (T*)hm->prop; h.gprop = (T*)hm->grad_prop;
-    QbTcgPlan tg;
-    QbTg8Plan t8;
-    if (L.streamed) {
+    if (L.path == QB_PATH_STREAM) {
         if (set_smem(k_hmc_stream<T>, L.sp.smem_bytes)) return -2;
         k_hmc_stream<T><<<(unsigned)ch->K, QS_THREADS, L.sp.smem_bytes, st>>>(L.sp, c, h);
-    } else if (qb_tg8_make_plan(net, dtype, &t8)) {
-        if (launch_hmc_tc128<T>(t8, c, h, ch->K, st)) return -2;
+    } else if (L.path == QB_PATH_TG8) {
+        if (launch_hmc_tc128<T>(L.t8, c, h, ch->K, st)) return -2;
         g_launches += 1;
-    } else if (qb_tcg_make_plan(net, dtype, &tg)) {
-        if (launch_hmc_tc<T>(tg, c, h, ch->K, st)) return -2;
+    } else if (L.path == QB_PATH_TCG) {
+        if (launch_hmc_tc<T>(L.tg, c, h, ch->K, st)) return -2;
     } else {
         if (set_smem(k_hmc<T>, L.plan.smem_bytes)) return -2;
         k_hmc<T><<<(unsigned)ch->K, L.plan.nthreads, L.plan.smem_bytes, st>>>(L.plan, c, h);
@@ -1736,10 +1027,7 @@ static int run_predict(const qb_net_t* net, int dtype, const void* theta, int64_
         PredArgs<T> a;
         a.theta = (const T*)theta; a.x = (const T*)x; a.M = M; a.N = N;
         a.out = (T*)out; a.mean = (T*)mean; a.var = (T*)var; a.fused = 0;
-        const long long tiles = cdiv(N, SP.TM);
-        long long chunks = std::max<long long>(1, std::min<long long>(tiles, cdiv((long long)QB_NUM_SMS * 2, M)));
-        a.tiles_per_block = cdiv(tiles, chunks);
-        chunks = cdiv(tiles, a.tiles_per_block);
+        const long long chunks = qb_tile_chunks(cdiv(N, SP.TM), (long long)qb_num_sms() * 2, M, &a.tiles_per_block);
         if (set_smem(k_predict_stream<T>, SP.smem_bytes)) return -2;
         k_predict_stream<T><<<(unsigned)(M * chunks), QS_THREADS, SP.smem_bytes, st>>>(SP, a, chunks);
         QB_CUDA(cudaGetLastError());
@@ -1764,10 +1052,7 @@ static int run_predict(const qb_net_t* net, int dtype, const void* theta, int64_
     QbTcPlan tp;
     if (!fused && out && make_tc_plan(net, dtype, &tp, 3)) {
         // tensor-core forward (qb_tc.cuh / qb_tc3.cuh): 128-point tiles, weights staged once per block, >= 8 waves of blocks
-        const long long t128 = cdiv(N, 128);
-        long long ch = std::max<long long>(1, std::min<long long>(t128, cdiv((long long)QB_NUM_SMS * 2 * 8, M)));
-        a.tiles_per_block = cdiv(t128, ch);
-        ch = cdiv(t128, a.tiles_per_block);
+        const long long ch = qb_tile_chunks(cdiv(N, 128), (long long)qb_num_sms() * 2 * 8, M, &a.tiles_per_block);
         if (launch_predict_tc<T>(tp, a, dim3((unsigned)M, (unsigned)ch), st)) return -2;
         QB_CUDA(cudaGetLastError());
         g_launches += 1;
@@ -1782,11 +1067,7 @@ static int run_predict(const qb_net_t* net, int dtype, const void* theta, int64_
     if (set_smem(k_predict<T>, P.smem_bytes)) return -2;
     long long chunks = tiles;
     a.tiles_per_block = 1;
-    if (!fused) {
-        chunks = std::max<long long>(1, std::min<long long>(tiles, cdiv((long long)QB_NUM_SMS * 8, M)));
-        a.tiles_per_block = cdiv(tiles, chunks);
-        chunks = cdiv(tiles, a.tiles_per_block);
-    }
+    if (!fused) chunks = qb_tile_chunks(tiles, (long long)qb_num_sms() * 8, M, &a.tiles_per_block);
     dim3 grid(fused ? (unsigned)chunks : (unsigned)M, fused ? 1u : (unsigned)chunks);
     k_predict<T><<<grid, P.nthreads, P.smem_bytes, st>>>(P, a);
     QB_CUDA(cudaGetLastError());
@@ -1950,7 +1231,7 @@ __global__ void __launch_bounds__(256, 2) k_fma2_peak(long long iters, float* si
 
 extern "C" int qb_fma_peak(int dtype, int variant, int64_t iters, double* flops_out_host, void* sink, void* stream) {
     cudaStream_t st = (cudaStream_t)stream;
-    const int blocks = QB_NUM_SMS * 8, threads = 256;
+    const int blocks = qb_num_sms() * 8, threads = 256;
     if (dtype == QB_F32 && variant == 2) {
         k_fma2_peak<<<blocks, threads, 0, st>>>(iters, (float*)sink);
         QB_CUDA(cudaGetLastError());

@@ -1,4 +1,4 @@
-// Host interface of the warp-specialised hot-shape value path (qb_value_tc3.cu); called from qb_kernels.cu.
+// Host interface of the warp-specialised hot-shape value path (qb_value_tc3.cu); called from qb_kernels.cu and qb_launch.cu.
 #pragma once
 #include <cuda_runtime.h>
 #include "quinn_b200.h"
