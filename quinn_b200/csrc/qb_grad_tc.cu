@@ -57,11 +57,8 @@ bool qb_tcg_make_plan(const qb_net_t* net, int dtype, QbTcgPlan* tp) {
     tp->c_dw1 = 6 * H; tp->c_db1 = 7 * H; tp->c_dw0 = 7 * H + 8;
     const int cols = 7 * H + 16;
     tp->tmem_cols = cols <= 256 ? 256 : 512;
-    if (off > 227 * 1024) return false;
-    // tensor memory is 512 columns per SM: request enough shared memory that no more blocks than 512/tmem_cols become resident
-    const int max_blocks = 512 / tp->tmem_cols;
-    const long long floor_bytes = 228 * 1024 / (max_blocks + 1) + 1;
-    tp->smem_bytes = (int)std::min<long long>(227 * 1024, std::max<long long>(off, floor_bytes));
+    if (off > QB_SMEM_MAX) return false;
+    tp->smem_bytes = (int)std::min<long long>(QB_SMEM_MAX, std::max<long long>(off, qb_tmem_smem_floor(tp->tmem_cols)));
     return true;
 }
 
@@ -76,7 +73,7 @@ __global__ void __launch_bounds__(H * 8, H == 32 ? 2 : 1) k_logpost_grad_tc(cons
     qb_tcg_stage(tp, smem_g, a.theta + k * tp.n_params);
     const double ssq = qb_tcg_eval<H, NI, ACT>(tp, cx, smem_g, a.x + k * a.xs, a.y + k * a.ys, n0, n1, (float)a.lk.inv_sigma2, g);
     if (threadIdx.x == 0) a.part[k * a.S + s] = ssq;
-    qb_tcg_fini(tp, cx);
+    qb_tc_stop(cx.tmem, (uint32_t)tp.tmem_cols);
 }
 
 template <int H, int NI, int ACT> struct QbGradTc {
@@ -105,7 +102,7 @@ __global__ void __launch_bounds__(H * 8, H == 32 ? 2 : 1) k_hmc_tc(const __grid_
     qb_tcg_init(tp, smem_g, cx);
     QbGradTc<H, NI, ACT> eval{tp, cx, smem_g, c, (long long)blockIdx.x};
     qb_hmc_body<float>(c, h, tp.n_params, reinterpret_cast<double*>(smem_g), eval);
-    qb_tcg_fini(tp, cx);
+    qb_tc_stop(cx.tmem, (uint32_t)tp.tmem_cols);
 }
 
 template <int H, int NI, int ACT>

@@ -53,11 +53,8 @@ bool qb_tg8_make_plan(const qb_net_t* net, int dtype, QbTg8Plan* tp) {
     const int cols = 3 * H + 32;
     tp->tmem_cols = cols <= 256 ? 256 : 512;
     tp->nthreads = 4 * H + 32;
-    if (off > 227 * 1024) return false;
-    // tensor memory is 512 columns per SM: request enough shared memory that no more blocks than 512/tmem_cols become resident
-    const int max_blocks = 512 / tp->tmem_cols;
-    const long long floor_bytes = 228 * 1024 / (max_blocks + 1) + 1;
-    tp->smem_bytes = (int)std::min<long long>(227 * 1024, std::max<long long>(off, floor_bytes));
+    if (off > QB_SMEM_MAX) return false;
+    tp->smem_bytes = (int)std::min<long long>(QB_SMEM_MAX, std::max<long long>(off, qb_tmem_smem_floor(tp->tmem_cols)));
     return true;
 }
 
@@ -94,7 +91,7 @@ __global__ void __launch_bounds__(4 * H + 32, H == 64 ? 2 : 1) k_logpost_grad_tc
     qb_tg8_stage<H>(tp, smem_g, a.theta + k * tp.n_params, absmax, is2);
     const double ssq = qb_tg8_eval<H>(tp, tmem, smem_g, a.x + k * a.xs, a.y + k * a.ys, n0, n1, is2, g);
     if (threadIdx.x == 0) a.part[k * a.S + s] = ssq;
-    qb_tg8_fini(tp, tmem);
+    qb_tc_stop(tmem, (uint32_t)tp.tmem_cols);
 }
 
 template <int H> struct QbGradTg8 {
@@ -123,7 +120,7 @@ __global__ void __launch_bounds__(4 * H + 32, H == 64 ? 2 : 1) k_hmc_tc128(const
     const uint32_t tmem = qb_tg8_init<H>(tp, smem_g);
     QbGradTg8<H> eval{tp, tmem, smem_g, c, absmax, (long long)blockIdx.x};
     qb_hmc_body<float>(c, h, tp.n_params, reinterpret_cast<double*>(smem_g), eval);
-    qb_tg8_fini(tp, tmem);
+    qb_tc_stop(tmem, (uint32_t)tp.tmem_cols);
 }
 
 template <int H>

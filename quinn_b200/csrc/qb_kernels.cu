@@ -118,7 +118,7 @@ __global__ void __launch_bounds__(512, 1) k_logpost_tc(const __grid_constant__ Q
     __syncthreads();
     const double ssq = qb_tc_eval<false>(tp, cx, smem_tc, a.x + k * a.xs, a.y + k * a.ys, n0, n1);
     if (threadIdx.x == 0) a.part[k * a.S + s] = ssq;
-    qb_tc_fini(tp, cx);
+    qb_tc_stop(cx.tmem, (uint32_t)tp.tmem_cols);
 }
 
 template <typename T> static int launch_logpost_tc(const QbTcPlan&, const EvalArgs<T>&, dim3, cudaStream_t) { return qb_fail("tensor-core path is fp32 only"); }
@@ -669,7 +669,7 @@ k_amcmc(const __grid_constant__ QbPlan plan, const __grid_constant__ QbTcPlan tp
         else qb_amcmc_post<T>(c, a, P, k, s, ssq, S.red, st);
     }
     if (threadIdx.x == 0) { c.lp[k] = st.lp_cur; c.map_lp[k] = st.map_lp; c.naccept[k] = st.na; a.prop_kind[k] = st.kind; }
-    if constexpr (TC) qb_tc_fini(tp, cx);
+    if constexpr (TC) qb_tc_stop(cx.tmem, (uint32_t)tp.tmem_cols);
 }
 
 // kernel 3 (AMCMC), layer-streamed: one block per chain, the proposal pass uses the activation area as scratch
@@ -1003,7 +1003,7 @@ __global__ void __launch_bounds__(512, 1) k_predict_tc(const __grid_constant__ Q
     qb_tc_stage(tp, smem_tc, a.theta + m * tp.n_params);
     __syncthreads();
     qb_tc_predict(tp, cx, smem_tc, a.x, a.out + m * a.N * tp.out_dim, n0, n1);
-    qb_tc_fini(tp, cx);
+    qb_tc_stop(cx.tmem, (uint32_t)tp.tmem_cols);
 }
 template <typename T> static int launch_predict_tc(const QbTcPlan&, const PredArgs<T>&, dim3, cudaStream_t) { return qb_fail("tensor-core path is fp32 only"); }
 template <> int launch_predict_tc<float>(const QbTcPlan& tp, const PredArgs<float>& a, dim3 grid, cudaStream_t st) {

@@ -26,9 +26,6 @@ int qb_env_int(const char* name, int dflt) {
 static inline int rup(int v, int m) { return (v + m - 1) / m * m; }
 static inline long long cdiv(long long a, long long b) { return (a + b - 1) / b; }
 
-static const int QB_SMEM_MAX = 227 * 1024;
-static const int QB_SMEM_SM = 228 * 1024;    // shared memory per SM
-
 int qb_num_sms() {
     static int n = 0;
     if (n == 0) {
@@ -457,11 +454,7 @@ bool make_tc_plan(const qb_net_t* net, int dtype, QbTcPlan* tp, int allow_v3) {
     tp->ybuf = (int)bytes; bytes += 2 * 3 * 4 * 128 * 4;
     tp->nthreads = tp->pipe ? 128 * tp->pipe : 128;
     if (bytes > QB_SMEM_MAX) return false;
-    // tensor memory is 512 columns per SM: request enough shared memory that no more blocks than 512/tmem_cols
-    // become resident (a further block would spin in tcgen05.alloc)
-    const int max_blocks = 512 / tp->tmem_cols;
-    const long long floor_bytes = QB_SMEM_SM / (max_blocks + 1) + 1;
-    tp->smem_bytes = (int)std::min<long long>(QB_SMEM_MAX, std::max(bytes, floor_bytes));
+    tp->smem_bytes = (int)std::min<long long>(QB_SMEM_MAX, std::max(bytes, qb_tmem_smem_floor(tp->tmem_cols)));
     const int v3h = allow_v3 ? qb_tc_v3_shape(*tp) : 0;
     if (v3h && net->layers[1].act == QB_ACT_TANH && !qb_env_int("QB_NO_V3", 0) && !(allow_v3 == 2 && v3h != 64)) {
         // warp-specialised path (qb_tc3.cuh): 4 H/32 compute warps + 1 issue warp, 4 H tensor-memory columns, own layout
@@ -479,7 +472,7 @@ bool make_tc_plan(const qb_net_t* net, int dtype, QbTcPlan* tp, int allow_v3) {
         tp->v3_state = o;
         if (allow_v3 == 2) o += 3 * ((net->n_params + 3) / 4 * 4) * 4;
         const int max_blocks3 = 512 / tp->tmem_cols;
-        tp->smem_bytes = (int)std::max<long long>(o, QB_SMEM_SM / (max_blocks3 + 1) + 1);
+        tp->smem_bytes = (int)std::max<long long>(o, qb_tmem_smem_floor(tp->tmem_cols));
         if (tp->smem_bytes > (QB_SMEM_SM - 1024 * max_blocks3) / max_blocks3) return make_tc_plan(net, dtype, tp, 0);     // the blocks must fit
     }
     return true;

@@ -9,6 +9,13 @@
 #include "qb_tcg.cuh"
 #include "qb_tg8_plan.h"
 
+constexpr int QB_SMEM_MAX = 227 * 1024;    // shared memory of one block
+constexpr int QB_SMEM_SM = 228 * 1024;     // shared memory per SM
+// Tensor memory has 512 columns per SM, and a block whose tcgen05.alloc cannot be met spins until another block frees
+// its columns.  A kernel that allocates tmem_cols columns asks for at least this much shared memory, so that no more
+// than 512 / tmem_cols of its blocks become resident on one SM.
+inline long long qb_tmem_smem_floor(int tmem_cols) { return QB_SMEM_SM / (512 / tmem_cols + 1) + 1; }
+
 // sets the thread's error text (format: a string, then an integer) and returns -1
 int qb_fail(const char* fmt, const char* a = "", long long b = 0);
 // an environment variable as an integer, dflt when unset or empty (read on every call)

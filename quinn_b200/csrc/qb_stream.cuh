@@ -13,6 +13,7 @@
 // xor-shuffle tree, so fp64 results are the same bits run to run.
 #pragma once
 #include "qb_device.cuh"
+#include "qb_tcgen05.cuh"
 
 #define QS_THREADS 256
 #define QS_STAGES 3
@@ -56,40 +57,21 @@ struct QsRing {
     long long used;         // chunks consumed by earlier evaluations of this block (slot / parity bookkeeping)
 };
 
-__device__ __forceinline__ uint32_t qs_smem(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
 __device__ __forceinline__ void qs_ring_init(const QbStreamPlan& P, unsigned char* smem, QsRing& rg) {
     rg.slots = smem + P.ring_off;
     rg.bar = reinterpret_cast<uint64_t*>(smem + 40 * sizeof(double));
     rg.used = 0;
     if (threadIdx.x < QS_STAGES)
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(qs_smem(rg.bar + threadIdx.x)), "r"(QS_THREADS) : "memory");
+        qb_mbar_init(qb_smem_u32(rg.bar + threadIdx.x), QS_THREADS);
     __syncthreads();
 }
 
 template <typename T> __device__ __forceinline__ void qs_cp(T* dst, const T* src);
 template <> __device__ __forceinline__ void qs_cp<float>(float* dst, const float* src) {
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" :: "r"(qs_smem(dst)), "l"(src) : "memory");
+    asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" :: "r"(qb_smem_u32(dst)), "l"(src) : "memory");
 }
 template <> __device__ __forceinline__ void qs_cp<double>(double* dst, const double* src) {
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" :: "r"(qs_smem(dst)), "l"(src) : "memory");
-}
-
-// bounded like qb_mbar_wait (qb_tc.cuh): a protocol bug ends the kernel with an error instead of hanging the GPU
-__device__ __forceinline__ void qs_wait(uint64_t* bar, uint32_t parity) {
-    unsigned long long t0 = 0;
-    for (uint32_t it = 0;; ++it) {
-        uint32_t ok;
-        asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.b32 %0, 1, 0, p; }"
-                     : "=r"(ok) : "r"(qs_smem(bar)), "r"(parity) : "memory");
-        if (ok) return;
-        if ((it & 1023u) == 1023u) {
-            unsigned long long now;
-            asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(now));
-            if (t0 == 0) t0 = now;
-            else if (now - t0 > 20000000000ULL) __trap();
-        }
-    }
+    asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" :: "r"(qb_smem_u32(dst)), "l"(src) : "memory");
 }
 
 // chunk c of the per-tile schedule -> layer, first row, direction
@@ -124,14 +106,14 @@ __device__ __forceinline__ void qs_fetch(const QbStreamPlan& P, const QsRing& rg
             if (i >= n_in) { i -= n_in; ++r; }
         }
     }
-    asm volatile("cp.async.mbarrier.arrive.noinc.shared::cta.b64 [%0];" :: "r"(qs_smem(rg.bar + slot)) : "memory");
+    asm volatile("cp.async.mbarrier.arrive.noinc.shared::cta.b64 [%0];" :: "r"(qb_smem_u32(rg.bar + slot)) : "memory");
 }
 
 // wait for chunk g; on return every thread has finished with chunk g-1, so its slot is refilled with chunk g+NST-1
 template <typename T>
 __device__ __forceinline__ T* qs_acquire(const QbStreamPlan& P, const QsRing& rg, const T* theta, long long g, long long g_end) {
     const int slot = (int)(g % QS_STAGES);
-    qs_wait(rg.bar + slot, (uint32_t)((g / QS_STAGES) & 1));
+    qb_mbar_wait_timed<false>(qb_smem_u32(rg.bar + slot), (uint32_t)((g / QS_STAGES) & 1));
     __syncthreads();
     if (g + QS_STAGES - 1 < g_end) qs_fetch<T>(P, rg, theta, g + QS_STAGES - 1);
     T* w = reinterpret_cast<T*>(rg.slots) + (size_t)slot * P.slot_elems;

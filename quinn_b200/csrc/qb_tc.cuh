@@ -21,6 +21,7 @@
 #pragma once
 #include <stdint.h>
 #include "qb_plan.h"
+#include "qb_tcgen05.cuh"
 
 struct QbTcLayer {
     int n_in, n_out, w_off, b_off, act;
@@ -55,76 +56,14 @@ enum { QB_TC_RED_BYTES = 320, QB_TC_BAR_OFF = 320, QB_TC_SLOT_OFF = 328, QB_TC_A
 
 struct QbTcCtx { uint32_t tmem, bar, phase, abar, aphase, hbar, hphase; };
 
-__device__ __forceinline__ uint32_t qb_smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-#define QB_R16(v) "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]), \
-                  "r"(v[8]), "r"(v[9]), "r"(v[10]), "r"(v[11]), "r"(v[12]), "r"(v[13]), "r"(v[14]), "r"(v[15])
-#define QB_W16(v) "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), \
-                  "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-#define QB_RW16(v) "+r"(v[0]), "+r"(v[1]), "+r"(v[2]), "+r"(v[3]), "+r"(v[4]), "+r"(v[5]), "+r"(v[6]), "+r"(v[7]), \
-                   "+r"(v[8]), "+r"(v[9]), "+r"(v[10]), "+r"(v[11]), "+r"(v[12]), "+r"(v[13]), "+r"(v[14]), "+r"(v[15])
-
-__device__ __forceinline__ void qb_tmem_st16(uint32_t taddr, const uint32_t (&v)[16]) {
-    asm volatile("tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16};"
-                 :: "r"(taddr), QB_R16(v) : "memory");
-}
-__device__ __forceinline__ void qb_tmem_ld16(uint32_t taddr, uint32_t (&v)[16]) {
-    asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-                 : QB_W16(v) : "r"(taddr) : "memory");
-}
-// the registers are operands of the wait so that no use of them can be scheduled before it
-__device__ __forceinline__ void qb_tmem_ld_wait16(uint32_t (&v)[16]) {
-    asm volatile("tcgen05.wait::ld.sync.aligned;" : QB_RW16(v) :: "memory");
-}
-__device__ __forceinline__ void qb_tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
-__device__ __forceinline__ void qb_tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void qb_tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-
-// bounded wait: a lost arrival traps after 20 s of wall-clock time (globaltimer, so that a context that is merely
-// preempted / time-sliced for a while does not trip it) instead of hanging the GPU
-__device__ __forceinline__ void qb_mbar_wait(uint32_t bar, uint32_t parity) {
-    unsigned long long t0 = 0;
-    for (uint32_t it = 0;; ++it) {
-        uint32_t ok;
-        asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3; selp.b32 %0, 1, 0, p; }"
-                     : "=r"(ok) : "r"(bar), "r"(parity), "r"(20000u) : "memory");       // suspend-time hint: 20 us
-        if (ok) return;
-        if ((it & 1023u) == 1023u) {
-            unsigned long long now;
-            asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(now));
-            if (t0 == 0) t0 = now;
-            else if (now - t0 > 20000000000ULL) __trap();
-        }
-    }
-}
-
-// all threads; allocates tensor memory and initialises the mbarrier
+// all threads; allocates tensor memory and initialises the mbarriers
 __device__ __forceinline__ void qb_tc_init(const QbTcPlan& tp, unsigned char* smem, QbTcCtx& cx) {
-    if ((threadIdx.x >> 5) == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
-                     :: "r"(qb_smem_u32(smem + QB_TC_SLOT_OFF)), "r"((uint32_t)tp.tmem_cols) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    if (threadIdx.x == 0) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(qb_smem_u32(smem + QB_TC_BAR_OFF)), "r"(1u) : "memory");
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(qb_smem_u32(smem + QB_TC_ABAR_OFF)), "r"((uint32_t)blockDim.x) : "memory");
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(qb_smem_u32(smem + QB_TC_HBAR_OFF)), "r"(1u) : "memory");
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    qb_tc_fence_before();
-    __syncthreads();
-    qb_tc_fence_after();
-    cx.tmem = *reinterpret_cast<volatile uint32_t*>(smem + QB_TC_SLOT_OFF);
+    const uint32_t bars[3] = {QB_TC_BAR_OFF, QB_TC_ABAR_OFF, QB_TC_HBAR_OFF}, counts[3] = {1u, QB_MBAR_BLOCK, 1u};
+    cx.tmem = qb_tc_start(smem, QB_TC_SLOT_OFF, (uint32_t)tp.tmem_cols, bars, counts);
     cx.bar = qb_smem_u32(smem + QB_TC_BAR_OFF);
     cx.abar = qb_smem_u32(smem + QB_TC_ABAR_OFF);
     cx.hbar = qb_smem_u32(smem + QB_TC_HBAR_OFF);
     cx.phase = 0; cx.aphase = 0; cx.hphase = 0;
-}
-__device__ __forceinline__ void qb_tc_fini(const QbTcPlan& tp, const QbTcCtx& cx) {
-    qb_tc_fence_before();
-    __syncthreads();
-    if ((threadIdx.x >> 5) == 0)
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(cx.tmem), "r"((uint32_t)tp.tmem_cols) : "memory");
 }
 
 __device__ __forceinline__ float qb_tf32_hi(float w) { return __uint_as_float(__float_as_uint(w) & 0xFFFFE000u); }
@@ -169,8 +108,7 @@ __device__ __forceinline__ void qb_tc_stage(const QbTcPlan& tp, unsigned char* s
         for (int e = tid; e < tp.out_dim * tp.kl; e += nt) F[tp.wl + e] = theta[tp.wl_off + e] * sl;
         for (int j = tid; j < tp.out_dim; j += nt) F[tp.bl + j] = tp.bl_off >= 0 ? theta[tp.bl_off + j] * sl : 0.0f;
     }
-    // the tensor core reads shared memory through the async proxy
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    qb_fence_proxy_async();
 }
 
 // tanh of four pre-activations that were already multiplied by 2*log2(e): tanh = 1 - 2/(1 + 2^z'), with ONE
@@ -211,9 +149,7 @@ __device__ __forceinline__ void qb_tanh4_prescaled(float2& a, float2& b) {
 template <int KS, bool HALF = false>
 __device__ __forceinline__ void qb_tc_issue_ks(uint32_t d, uint32_t a_hi, uint32_t a_lo, uint32_t bhi, uint32_t blo,
                                                uint32_t dhi, uint32_t idesc, uint32_t bar, uint32_t hbar = 0) {
-    uint32_t elected;
-    asm volatile("{ .reg .pred p; elect.sync _|p, 0xffffffff; selp.b32 %0, 1, 0, p; }" : "=r"(elected) :: "memory");
-    if (elected) {
+    if (qb_elect()) {
 #pragma unroll
         for (int half = 0; half < (HALF ? 2 : 1); ++half) {
             constexpr int S0 = 0, SN = HALF ? KS / 2 : KS;
@@ -224,18 +160,13 @@ __device__ __forceinline__ void qb_tc_issue_ks(uint32_t d, uint32_t a_hi, uint32
                     const int s = ss + half * SN;
                     const uint32_t a = (pass == 0 ? a_lo : a_hi) + (uint32_t)s * 8u;
                     const uint32_t bl = (pass == 1 ? blo : bhi) + (uint32_t)s * 16u;   // +256 bytes, in 16-byte units
-                    if (half == 0 && pass == 0 && ss == 0)
-                        asm volatile("{ .reg .pred p; .reg .b64 dd; setp.ne.b32 p, 0, 0; mov.b64 dd, {%2, %3}; tcgen05.mma.cta_group::1.kind::tf32 [%0], [%1], dd, %4, p; }"
-                                     :: "r"(d), "r"(a), "r"(bl), "r"(dhi), "r"(idesc) : "memory");
-                    else
-                        asm volatile("{ .reg .pred p; .reg .b64 dd; setp.eq.b32 p, 0, 0; mov.b64 dd, {%2, %3}; tcgen05.mma.cta_group::1.kind::tf32 [%0], [%1], dd, %4, p; }"
-                                     :: "r"(d), "r"(a), "r"(bl), "r"(dhi), "r"(idesc) : "memory");
+                    if (half == 0 && pass == 0 && ss == 0) qb_mma_ts<false, false>(d, a, bl, dhi, idesc);
+                    else qb_mma_ts<false, true>(d, a, bl, dhi, idesc);
                 }
             }
-            if (HALF && half == 0)
-                asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" :: "r"(hbar) : "memory");
+            if (HALF && half == 0) qb_commit(hbar);
         }
-        asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" :: "r"(bar) : "memory");
+        qb_commit(bar);
     }
     __syncwarp();
 }
@@ -245,9 +176,9 @@ __device__ __forceinline__ void qb_tc_issue_warp(const QbTcPlan& tp, const QbTcL
                                                  uint32_t d_off) {
     const uint32_t K = L.n_in, N = L.n_out;
     const uint32_t idesc = (1u << 4) | (2u << 7) | (2u << 10) | ((N >> 3) << 17) | ((128u >> 4) << 24);
-    const uint32_t dhi = ((128u * (K >> 2)) >> 4) | (1u << 14);
-    const uint32_t bhi = ((qb_smem_u32(smem + L.bhi) >> 4) & 0x3FFFu) | ((128u >> 4) << 16);
-    const uint32_t blo = ((qb_smem_u32(smem + L.blo) >> 4) & 0x3FFFu) | ((128u >> 4) << 16);
+    const uint32_t dhi = qb_desc_hi(128u * (K >> 2), 0u);
+    const uint32_t bhi = qb_desc_lo(qb_smem_u32(smem + L.bhi), 128u);
+    const uint32_t blo = qb_desc_lo(qb_smem_u32(smem + L.blo), 128u);
     const uint32_t d = cx.tmem + tp.d_col + d_off, a_hi = cx.tmem, a_lo = cx.tmem + tp.a_lo_col;
     if constexpr (HALF) {        // K == 8*KSH: 64 (two column groups) or 128 (four)
         qb_tc_issue_ks<KSH, true>(d, a_hi, a_lo, bhi, blo, dhi, idesc, cx.bar, cx.hbar);
@@ -263,10 +194,6 @@ __device__ __forceinline__ void qb_tc_issue_warp(const QbTcPlan& tp, const QbTcL
         case 14: qb_tc_issue_ks<14>(d, a_hi, a_lo, bhi, blo, dhi, idesc, cx.bar); break;
         default: qb_tc_issue_ks<16>(d, a_hi, a_lo, bhi, blo, dhi, idesc, cx.bar); break;
     }
-}
-
-__device__ __forceinline__ void qb_mbar_arrive(uint32_t bar) {
-    asm volatile("{ .reg .b64 st; mbarrier.arrive.shared::cta.b64 st, [%0]; }" :: "r"(bar) : "memory");
 }
 
 template <int ACT> __device__ __forceinline__ void qb_tc_act4(float2& a, float2& b) {
@@ -430,7 +357,7 @@ __device__ __forceinline__ void qb_tc_forward_tile(const QbTcPlan& tp, QbTcCtx& 
             qb_tc_fence_after();
             qb_tc_issue_warp(tp, L, cx, smem, 0u);
         }
-        qb_mbar_wait(cx.bar, cx.phase);
+        qb_mbar_wait_timed(cx.bar, cx.phase);
         cx.phase ^= 1u;
         qb_tc_fence_after();
         if (l < last_tc) {
@@ -548,7 +475,7 @@ __device__ __forceinline__ Sink qb_tc_pipe_run(const QbTcPlan& tp, QbTcCtx& cx, 
         qb_tc_fence_before();
         qb_mbar_arrive(cx.abar);
         if (threadIdx.x < 32) {
-            qb_mbar_wait(cx.abar, cx.aphase);
+            qb_mbar_wait_timed(cx.abar, cx.aphase);
             qb_tc_fence_after();
             qb_tc_issue_warp<HALFK, 4 * G>(tp, L, cx, smem, 0u);
         }
@@ -560,7 +487,7 @@ __device__ __forceinline__ Sink qb_tc_pipe_run(const QbTcPlan& tp, QbTcCtx& cx, 
         float sv[OD];
         if (grp == 0) sink.template prefetch<OD>(pc, pc < n1, sv);
         if constexpr (HALFK) {
-            qb_mbar_wait(cx.hbar, cx.hphase);                        // first K-half of tile t done: A columns [0,32) are free
+            qb_mbar_wait_timed(cx.hbar, cx.hphase);                        // first K-half of tile t done: A columns [0,32) are free
             cx.hphase ^= 1u;
             qb_tc_fence_after();
             if (more) {
@@ -570,7 +497,7 @@ __device__ __forceinline__ Sink qb_tc_pipe_run(const QbTcPlan& tp, QbTcCtx& cx, 
                 qb_tc_split_store(tl + grp * 16, tl + tp.a_lo_col + grp * 16, h);
             }
         }
-        qb_mbar_wait(cx.bar, cx.phase);                              // MMAs of tile t complete: A is free, D[t&1] is ready
+        qb_mbar_wait_timed(cx.bar, cx.phase);                              // MMAs of tile t complete: A is free, D[t&1] is ready
         cx.phase ^= 1u;
         qb_tc_fence_after();
         // finish tile t-1 (the partner warps published their partial sums one epilogue ago); these reads come before
@@ -605,7 +532,7 @@ __device__ __forceinline__ Sink qb_tc_pipe_run(const QbTcPlan& tp, QbTcCtx& cx, 
             qb_tc_fence_before();
             qb_mbar_arrive(cx.abar);
             if (threadIdx.x < 32) {
-                qb_mbar_wait(cx.abar, cx.aphase);
+                qb_mbar_wait_timed(cx.abar, cx.aphase);
                 qb_tc_fence_after();
                 qb_tc_issue_warp<HALFK, 4 * G>(tp, L, cx, smem, (uint32_t)((t + 1) & 1) * (uint32_t)N);
             }

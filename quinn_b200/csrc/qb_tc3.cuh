@@ -30,6 +30,7 @@
 // registers first thing and releases it at once.
 #pragma once
 #include "qb_tc.cuh"
+#include "qb_tcgen05.cuh"
 
 #ifdef __CUDACC__
 // Development aid (-DQB3_TRACE, scripts/tc3_trace.py): SM-clock stamps of the phases of every compute warp.
@@ -51,73 +52,22 @@ template <int H> struct Qb3Dim {
     static constexpr int COL_AHI = 2 * H, COL_ALO = 2 * H + H / 2, COL_D1 = 3 * H;
 };
 
-// mbarrier wait of the tile loops: try_wait suspends the thread until the phase completes or the 20 us hint expires, so a
-// plain counted loop is a bounded wait (2^20 x 20 us, then trap) with no state beyond its counter -- the timer-based
-// loop of qb_mbar_wait, inlined or called, made ptxas shuffle the live register arrays around it
-__device__ __forceinline__ void qb3_wait(uint32_t bar, uint32_t parity) {
-#pragma unroll 1
-    for (int it = 0; it < (1 << 20); ++it) {
-        uint32_t ok;
-        asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3; selp.b32 %0, 1, 0, p; }"
-                     : "=r"(ok) : "r"(bar), "r"(parity), "r"(20000u) : "memory");
-        if (ok) return;
-    }
-    __trap();
-}
-
 // all threads; tensor-memory allocation (the mbarriers are (re)initialised by every evaluation)
 template <int H>
 __device__ __forceinline__ void qb_tc3_init(const QbTcPlan& tp, unsigned char* smem, QbTcCtx& cx) {
     constexpr uint32_t QB3_NCOMPUTE = Qb3Dim<H>::NCOMP;
-    if ((threadIdx.x >> 5) == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
-                     :: "r"(qb_smem_u32(smem + QB_TC_SLOT_OFF)), "r"((uint32_t)tp.tmem_cols) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    if (threadIdx.x == 0) {
-        const uint32_t b = qb_smem_u32(smem);
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(b + QB3_D0F), "r"(1u) : "memory");
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(b + QB3_ARDY), "r"((uint32_t)QB3_NCOMPUTE) : "memory");
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(b + QB3_D1F), "r"(1u) : "memory");
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(b + QB3_D1FREE), "r"((uint32_t)QB3_NCOMPUTE) : "memory");
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(b + QB3_D0F1), "r"(1u) : "memory");
-        for (int i = 0; i < 3; ++i)          // x_full[3]: initialised once, their phases run across evaluations
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(b + (uint32_t)tp.v3_xbar + 8u * i), "r"(1u) : "memory");
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    qb_tc_fence_before();
-    __syncthreads();
-    qb_tc_fence_after();
-    cx.tmem = *reinterpret_cast<volatile uint32_t*>(smem + QB_TC_SLOT_OFF);
+    const uint32_t x = (uint32_t)tp.v3_xbar;
+    const uint32_t bars[8] = {QB3_D0F, QB3_ARDY, QB3_D1F, QB3_D1FREE, QB3_D0F1, x, x + 8u, x + 16u};
+    const uint32_t counts[8] = {1u, QB3_NCOMPUTE, 1u, QB3_NCOMPUTE, 1u, 1u, 1u, 1u};   // x_full[3]: their phases run across evaluations
+    cx.tmem = qb_tc_start(smem, QB_TC_SLOT_OFF, (uint32_t)tp.tmem_cols, bars, counts);
     cx.bar = cx.abar = cx.hbar = 0; cx.phase = cx.aphase = cx.hphase = 0;
 }
-// thread 0, between two block barriers: every phase of the previous evaluation has completed, start again at parity 0
+// between evaluations (thread 0): the five barriers of the tile loop start again at parity 0
 template <int H>
 __device__ __forceinline__ void qb_tc3_reset_barriers(unsigned char* smem) {
-    constexpr uint32_t QB3_NCOMPUTE = Qb3Dim<H>::NCOMP;
-    const uint32_t b = qb_smem_u32(smem);
-    const uint32_t off[5] = {QB3_D0F, QB3_ARDY, QB3_D1F, QB3_D1FREE, QB3_D0F1};
-#pragma unroll
-    for (int i = 0; i < 5; ++i) {
-        asm volatile("mbarrier.inval.shared::cta.b64 [%0];" :: "r"(b + off[i]) : "memory");
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(b + off[i]), "r"((i == 0 || i == 2 || i == 4) ? 1u : (uint32_t)QB3_NCOMPUTE) : "memory");
-    }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-}
-
-__device__ __forceinline__ uint32_t qb3_pack_f16(float lo_elem, float hi_elem) {
-    uint32_t r;
-    asm("cvt.rn.f16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi_elem), "f"(lo_elem));
-    return r;
-}
-// (x0, x1) -> fp16 pair `hi` (round to nearest) and the fp16 pair of the NEGATED remainders hi - x (the mixed-precision
-// subtract takes the fp16 operand first; the sign is absorbed by a negated copy of the other operand's hi tile)
-__device__ __forceinline__ void qb3_split_f16(float x0, float x1, uint32_t& hi, uint32_t& nlo) {
-    hi = qb3_pack_f16(x0, x1);
-    float d0, d1;       // hi - x, exactly: one instruction per element
-    asm("{ .reg .b16 a, b; mov.b32 {a, b}, %2; sub.rn.f32.f16 %0, a, %3; sub.rn.f32.f16 %1, b, %4; }"
-        : "=f"(d0), "=f"(d1) : "r"(hi), "f"(x0), "f"(x1));
-    nlo = qb3_pack_f16(d0, d1);
+    const uint32_t bars[5] = {QB3_D0F, QB3_ARDY, QB3_D1F, QB3_D1FREE, QB3_D0F1};
+    const uint32_t counts[5] = {1u, (uint32_t)Qb3Dim<H>::NCOMP, 1u, (uint32_t)Qb3Dim<H>::NCOMP, 1u};
+    qb_mbar_reset(smem, bars, counts);
 }
 
 // flat theta (global) -> shared operands of the three layers.  All threads of the block; ends with the async-proxy fence.
@@ -179,7 +129,7 @@ __device__ __forceinline__ void qb_tc3_stage(const QbTcPlan& tp, unsigned char* 
                 const int k = (lane + 32 * jj) * 2;
                 const float w0 = theta[L.w_off + n * H + k], w1 = theta[L.w_off + n * H + k + 1];
                 uint32_t h2, l2;
-                qb3_split_f16(w0 * wscale, w1 * wscale, h2, l2);
+                qb_split_f16_nlo(w0 * wscale, w1 * wscale, h2, l2);
                 const int idx = (((n >> 3) * (H / 8) + (k >> 3)) * 64 + (n & 7) * 8 + (k & 7)) >> 1;      // 32-bit word index
                 hi[idx] = h2; lo[idx] = l2 ^ 0x80008000u; nhi[idx] = h2 ^ 0x80008000u;
                 s += w0 + w1;
@@ -205,12 +155,7 @@ __device__ __forceinline__ void qb_tc3_stage(const QbTcPlan& tp, unsigned char* 
             F[tp.v3_c1] = __uint_as_float((uint32_t)(127 - 14 - sW) << 23);
         }
     }
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-}
-
-__device__ __forceinline__ void qb_tmem_st8(uint32_t taddr, const uint32_t (&v)[8]) {
-    asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};"
-                 :: "r"(taddr), "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]) : "memory");
+    qb_fence_proxy_async();
 }
 
 // 2^14 / (1 + 2^z) for EIGHT pre-activations with ONE reciprocal (the MUFU pipe, 16 results/clk/SM, is the first
@@ -236,28 +181,6 @@ __device__ __forceinline__ void qb3_sig8(float2 (&v)[4]) {
     const float2 i01 = __fmul2_rn(rq, p23), i23 = __fmul2_rn(rq, p01);      // 1/p01, 1/p23
     v[0] = __fmul2_rn(i01, d[1]); v[1] = __fmul2_rn(i01, d[0]);
     v[2] = __fmul2_rn(i23, d[3]); v[3] = __fmul2_rn(i23, d[2]);
-}
-
-// one tcgen05.mma (issued by the elected lane); ACC: accumulate into D
-template <bool ACC>
-__device__ __forceinline__ void qb3_mma_tf32_ss(uint32_t d, uint32_t a_lo32, uint32_t b_lo32, uint32_t dhi, uint32_t idesc) {
-    asm volatile("{ .reg .pred p; .reg .b64 da, db; setp.ne.b32 p, %5, 0; mov.b64 da, {%1, %3}; mov.b64 db, {%2, %3};\n\t"
-                 "tcgen05.mma.cta_group::1.kind::tf32 [%0], da, db, %4, p; }"
-                 :: "r"(d), "r"(a_lo32), "r"(b_lo32), "r"(dhi), "r"(idesc), "n"(ACC ? 1 : 0) : "memory");
-}
-template <bool ACC>
-__device__ __forceinline__ void qb3_mma_f16_ts(uint32_t d, uint32_t a_tmem, uint32_t b_lo32, uint32_t dhi, uint32_t idesc) {
-    asm volatile("{ .reg .pred p; .reg .b64 db; setp.ne.b32 p, %5, 0; mov.b64 db, {%2, %3};\n\t"
-                 "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], db, %4, p; }"
-                 :: "r"(d), "r"(a_tmem), "r"(b_lo32), "r"(dhi), "r"(idesc), "n"(ACC ? 1 : 0) : "memory");
-}
-__device__ __forceinline__ void qb3_commit(uint32_t bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" :: "r"(bar) : "memory");
-}
-__device__ __forceinline__ bool qb3_elect() {
-    uint32_t e;
-    asm volatile("{ .reg .pred p; elect.sync _|p, 0xffffffff; selp.b32 %0, 1, 0, p; }" : "=r"(e) :: "memory");
-    return e != 0;
 }
 
 // The issue warp's view of an x tile: lane l owns points 4l .. 4l+3
@@ -353,19 +276,18 @@ __device__ __forceinline__ Sink qb_tc3_run(const QbTcPlan& tp, QbTcCtx& cx, unsi
     if (!bulk && wid < D::ISSUER && 4 * (int)(threadIdx.x >> 7) < K0) {
         float xv[4];
         for (int u = 0; u < 2 && u < T; ++u) { xfetch(u, xv); xstage(u, xv); }
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+        qb_fence_proxy_async();
     }
     __syncthreads();
     if (T > 0 && wid == D::ISSUER) {
         // ================================ issue warp ================================
         float* xb = reinterpret_cast<float*>(smem + tp.v3_x);         // [3][hi | lo], 128 x K0 floats each
-        const uint32_t dhi0 = ((128u * (K0 / 4)) >> 4) | (1u << 14);  // tf32 operands with K = K0: SBO 128 K0/4 bytes
-        const uint32_t dhi1 = ((16u * H) >> 4) | (1u << 14);          // fp16 W1, K = H: SBO 16 H bytes
-        const uint32_t lbo = (128u >> 4) << 16;
-        const uint32_t w0hi = ((qb_smem_u32(smem + tp.v3_w0) >> 4) & 0x3FFFu) | lbo, w0lo = w0hi + ((uint32_t)(H * K0 * 4) >> 4);
-        const uint32_t w1hi = ((qb_smem_u32(smem + tp.v3_w1) >> 4) & 0x3FFFu) | lbo, w1lo = w1hi + ((uint32_t)(H * H * 2) >> 4),
+        const uint32_t dhi0 = qb_desc_hi(128u * (K0 / 4), 0u);        // tf32 operands with K = K0: SBO 128 K0/4 bytes
+        const uint32_t dhi1 = qb_desc_hi(16u * H, 0u);                // fp16 W1, K = H: SBO 16 H bytes
+        const uint32_t w0hi = qb_desc_lo(qb_smem_u32(smem + tp.v3_w0), 128u), w0lo = w0hi + ((uint32_t)(H * K0 * 4) >> 4);
+        const uint32_t w1hi = qb_desc_lo(qb_smem_u32(smem + tp.v3_w1), 128u), w1lo = w1hi + ((uint32_t)(H * H * 2) >> 4),
                        w1nhi = w1lo + ((uint32_t)(H * H * 2) >> 4);
-        const uint32_t xd = ((qb_smem_u32(xb) >> 4) & 0x3FFFu) | lbo;  // + 2 XT / 16 per ring slot, + XT / 16 for lo
+        const uint32_t xd = qb_desc_lo(qb_smem_u32(xb), 128u);        // + 2 XT / 16 per ring slot, + XT / 16 for lo
         const uint32_t id_tf32 = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(H >> 3) << 17) | ((128u >> 4) << 24);
         const uint32_t id_f16 = (1u << 4) | ((uint32_t)(H >> 3) << 17) | ((128u >> 4) << 24);
         const uint32_t d0 = cx.tmem, a_hi = cx.tmem + D::COL_AHI, a_lo = cx.tmem + D::COL_ALO;
@@ -383,7 +305,7 @@ __device__ __forceinline__ Sink qb_tc3_run(const QbTcPlan& tp, QbTcCtx& cx, unsi
         };
         auto xwait = [&](int u) {                  // all lanes: tile u has landed
             const int sl = u % 3;
-            qb3_wait(bar_x + (uint32_t)sl * 8u, (xpar >> sl) & 1u);
+            qb_mbar_wait_counted(bar_x + (uint32_t)sl * 8u, (xpar >> sl) & 1u);
             xpar ^= 1u << sl;
         };
         auto mma0 = [&](int u) {           // layer 0 of tile u: x ring slot u % 3 -> D0[u & 1]
@@ -393,18 +315,18 @@ __device__ __forceinline__ Sink qb_tc3_run(const QbTcPlan& tp, QbTcCtx& cx, unsi
 #pragma unroll
                 for (int ks = 0; ks < K0 / 8; ++ks) {
                     const uint32_t a = xa + (pass == 0 ? (XT >> 4) : 0u) + 16u * ks, b = (pass == 1 ? w0lo : w0hi) + 16u * ks;
-                    if (pass == 0 && ks == 0) qb3_mma_tf32_ss<false>(d, a, b, dhi0, id_tf32);
-                    else qb3_mma_tf32_ss<true>(d, a, b, dhi0, id_tf32);
+                    if (pass == 0 && ks == 0) qb_mma_ss<false, false>(d, a, dhi0, b, dhi0, id_tf32);
+                    else qb_mma_ss<false, true>(d, a, dhi0, b, dhi0, id_tf32);
                 }
             }
-            qb3_commit((u & 1) ? sb + QB3_D0F1 : bar_d0f);
+            qb_commit((u & 1) ? sb + QB3_D0F1 : bar_d0f);
         };
         // x tiles 0 .. 2 staged up front (unless the previous evaluation left them), layer 0 of tiles 0 and 1 started
         if (bulk && !(PRESTAGE && cx.phase) && lane == 0)
             for (int u = 0; u < 3 && u < T; ++u) xcopy(u);
         if (bulk) { xwait(0); if (T > 1) xwait(1); }
         __syncwarp();
-        if (qb3_elect()) {
+        if (qb_elect()) {
             mma0(0);
             if (T > 1) mma0(1);
         }
@@ -412,17 +334,17 @@ __device__ __forceinline__ Sink qb_tc3_run(const QbTcPlan& tp, QbTcCtx& cx, unsi
 #pragma unroll 1
         for (int t = 0; t < T; ++t) {
             if (bulk && t + 2 < T) xwait(t + 2);                                      // long since landed
-            qb3_wait(bar_ardy, (uint32_t)t & 1u);                                     // A(t) written, D0[t&1] read
+            qb_mbar_wait_counted(bar_ardy, (uint32_t)t & 1u);                                     // A(t) written, D0[t&1] read
             QB3_STAMP(t, 0);
             qb_tc_fence_after();
             __syncwarp();
-            if (t + 2 < T && qb3_elect()) mma0(t + 2);
+            if (t + 2 < T && qb_elect()) mma0(t + 2);
             __syncwarp();
             QB3_STAMP(t, 1);
-            if (t >= 1) { qb3_wait(bar_d1free, (uint32_t)(t - 1) & 1u); qb_tc_fence_after(); }   // EPI1(t-1) holds D1 in registers
+            if (t >= 1) { qb_mbar_wait_counted(bar_d1free, (uint32_t)(t - 1) & 1u); qb_tc_fence_after(); }   // EPI1(t-1) holds D1 in registers
             __syncwarp();
             QB3_STAMP(t, 2);
-            if (qb3_elect()) {
+            if (qb_elect()) {
                 const uint32_t d1 = cx.tmem + D::COL_D1;
 #pragma unroll
                 for (int pass = 0; pass < 3; ++pass) {
@@ -430,11 +352,11 @@ __device__ __forceinline__ Sink qb_tc3_run(const QbTcPlan& tp, QbTcCtx& cx, unsi
                     for (int ks = 0; ks < H / 16; ++ks) {
                         const uint32_t a = (pass == 0 ? a_lo : a_hi) + 8u * ks;
                         const uint32_t b = (pass == 0 ? w1nhi : pass == 1 ? w1lo : w1hi) + 16u * ks;
-                        if (pass == 0 && ks == 0) qb3_mma_f16_ts<false>(d1, a, b, dhi1, id_f16);
-                        else qb3_mma_f16_ts<true>(d1, a, b, dhi1, id_f16);
+                        if (pass == 0 && ks == 0) qb_mma_ts<true, false>(d1, a, b, dhi1, id_f16);
+                        else qb_mma_ts<true, true>(d1, a, b, dhi1, id_f16);
                     }
                 }
-                qb3_commit(bar_d1f);
+                qb_commit(bar_d1f);
             }
             __syncwarp();
             QB3_STAMP(t, 3);
@@ -469,7 +391,7 @@ __device__ __forceinline__ Sink qb_tc3_run(const QbTcPlan& tp, QbTcCtx& cx, unsi
             // layer 0 of tiles u >= 2 was issued BEFORE MMA1(u-2), whose commit (d1_full(u-2), waited for in EPI0(u-1))
             // covers every earlier tcgen05 operation of the issuing thread: only the first two tiles wait on d0_full
             if (u < 2) {
-                qb3_wait((u & 1) ? sb + QB3_D0F1 : bar_d0f, 0u);
+                qb_mbar_wait_counted((u & 1) ? sb + QB3_D0F1 : bar_d0f, 0u);
                 qb_tc_fence_after();
             }
             uint32_t v[2][16];
@@ -488,12 +410,12 @@ __device__ __forceinline__ Sink qb_tc3_run(const QbTcPlan& tp, QbTcCtx& cx, unsi
                     for (int i = 0; i < 4; ++i) a[i] = make_float2(__uint_as_float(v[j][8 * q + 2 * i]), __uint_as_float(v[j][8 * q + 2 * i + 1]));
                     qb3_sig8(a);
 #pragma unroll
-                    for (int i = 0; i < 4; ++i) qb3_split_f16(a[i].x, a[i].y, hi[j][4 * q + i], lo[j][4 * q + i]);
+                    for (int i = 0; i < 4; ++i) qb_split_f16_nlo(a[i].x, a[i].y, hi[j][4 * q + i], lo[j][4 * q + i]);
                 }
             }
             QB3_STAMP(u, 2);
             if (u > 0) {
-                qb3_wait(bar_d1f, (uint32_t)(u - 1) & 1u);           // MMA1(u-1) complete: A is free, D1 is ready
+                qb_mbar_wait_counted(bar_d1f, (uint32_t)(u - 1) & 1u);           // MMA1(u-1) complete: A is free, D1 is ready
                 qb_tc_fence_after();
             }
             QB3_STAMP(u, 3);
@@ -504,7 +426,7 @@ __device__ __forceinline__ Sink qb_tc3_run(const QbTcPlan& tp, QbTcCtx& cx, unsi
             }
             if (xmine && u + 2 < T) {
                 xstage(u + 2, xv);        // slot (u+2) % 3 was last read by MMA0(u-1), whose D0 this thread consumed a tile ago
-                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+                qb_fence_proxy_async();
             }
             qb_tmem_st_wait();
             qb_tc_fence_before();
@@ -575,7 +497,7 @@ __device__ __forceinline__ Sink qb_tc3_run(const QbTcPlan& tp, QbTcCtx& cx, unsi
                 }
             }
             if (t + 1 < T) epi0(t + 1);
-            else { qb3_wait(bar_d1f, (uint32_t)t & 1u); qb_tc_fence_after(); }
+            else { qb_mbar_wait_counted(bar_d1f, (uint32_t)t & 1u); qb_tc_fence_after(); }
         }
         {
             const int u = T - 1;

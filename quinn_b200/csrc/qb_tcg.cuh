@@ -32,6 +32,7 @@
 #include <stdint.h>
 #include "qb_plan.h"
 #include "qb_tc.cuh"
+#include "qb_tcgen05.cuh"
 
 struct QbTcgPlan {
     int in_dim, ni, n_params;
@@ -55,35 +56,15 @@ enum { QB_TCG_BARF = 320, QB_TCG_SLOT = 328, QB_TCG_ABAR = 336, QB_TCG_BARB = 34
 struct QbTcgCtx { uint32_t tmem, abar, barf, barb, barw, barz, ph; };   // ph: parity bits (0 abar, 1 f, 2 b, 3 w, 4 z)
 
 __device__ __forceinline__ void qb_tcg_init(const QbTcgPlan& tp, unsigned char* smem, QbTcgCtx& cx) {
-    if ((threadIdx.x >> 5) == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
-                     :: "r"(qb_smem_u32(smem + QB_TCG_SLOT)), "r"((uint32_t)tp.tmem_cols) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    if (threadIdx.x == 0) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(qb_smem_u32(smem + QB_TCG_ABAR)), "r"((uint32_t)blockDim.x) : "memory");
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(qb_smem_u32(smem + QB_TCG_BARF)), "r"(1u) : "memory");
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(qb_smem_u32(smem + QB_TCG_BARB)), "r"(1u) : "memory");
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(qb_smem_u32(smem + QB_TCG_BARW)), "r"(1u) : "memory");
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(qb_smem_u32(smem + QB_TCG_BARZ)), "r"(1u) : "memory");
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    qb_tc_fence_before();
-    __syncthreads();
-    qb_tc_fence_after();
-    cx.tmem = *reinterpret_cast<volatile uint32_t*>(smem + QB_TCG_SLOT);
+    const uint32_t bars[5] = {QB_TCG_ABAR, QB_TCG_BARF, QB_TCG_BARB, QB_TCG_BARW, QB_TCG_BARZ};
+    const uint32_t counts[5] = {QB_MBAR_BLOCK, 1u, 1u, 1u, 1u};
+    cx.tmem = qb_tc_start(smem, QB_TCG_SLOT, (uint32_t)tp.tmem_cols, bars, counts);
     cx.abar = qb_smem_u32(smem + QB_TCG_ABAR);
     cx.barf = qb_smem_u32(smem + QB_TCG_BARF);
     cx.barb = qb_smem_u32(smem + QB_TCG_BARB);
     cx.barw = qb_smem_u32(smem + QB_TCG_BARW);
     cx.barz = qb_smem_u32(smem + QB_TCG_BARZ);
     cx.ph = 0;
-}
-__device__ __forceinline__ void qb_tcg_fini(const QbTcgPlan& tp, const QbTcgCtx& cx) {
-    qb_tc_fence_before();
-    __syncthreads();
-    if ((threadIdx.x >> 5) == 0)
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(cx.tmem), "r"((uint32_t)tp.tmem_cols) : "memory");
 }
 
 // flat theta (global) -> shared: layer-0 rows (paired units, bias in slot in_dim), W1 (scaled for tanh) and W1^T (unscaled),
@@ -133,7 +114,7 @@ __device__ __forceinline__ void qb_tcg_stage(const QbTcgPlan& tp, unsigned char*
         F[tp.wl + j] = theta[tp.wl_off + j];
     }
     if (tid == 0) F[tp.bl] = tp.bl_off >= 0 ? theta[tp.bl_off] : 0.0f;
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    qb_fence_proxy_async();
 }
 
 template <int ACT> __device__ __forceinline__ float qb_tcg_dact(float a) {
@@ -167,28 +148,6 @@ __device__ __forceinline__ void qb_tcg_store_mn(unsigned char* bhi, unsigned cha
 }
 
 // ---- MMA issue (one elected lane of warp 0).  Descriptors are {lo, hi} 32-bit halves; k-steps add a constant to lo.
-__device__ __forceinline__ void qb_tcg_mma_ts(uint32_t d, uint32_t a, uint32_t blo, uint32_t bhi, uint32_t idesc, uint32_t acc) {
-    asm volatile("{ .reg .pred p; .reg .b64 db; setp.ne.b32 p, %5, 0; mov.b64 db, {%2, %3}; "
-                 "tcgen05.mma.cta_group::1.kind::tf32 [%0], [%1], db, %4, p; }"
-                 :: "r"(d), "r"(a), "r"(blo), "r"(bhi), "r"(idesc), "r"(acc) : "memory");
-}
-__device__ __forceinline__ void qb_tcg_mma_ss(uint32_t d, uint32_t alo, uint32_t ahi, uint32_t blo, uint32_t bhi, uint32_t idesc,
-                                              uint32_t acc) {
-    asm volatile("{ .reg .pred p; .reg .b64 da, db; setp.ne.b32 p, %6, 0; mov.b64 da, {%1, %2}; mov.b64 db, {%3, %4}; "
-                 "tcgen05.mma.cta_group::1.kind::tf32 [%0], da, db, %5, p; }"
-                 :: "r"(d), "r"(alo), "r"(ahi), "r"(blo), "r"(bhi), "r"(idesc), "r"(acc) : "memory");
-}
-__device__ __forceinline__ void qb_tcg_commit(uint32_t bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" :: "r"(bar) : "memory");
-}
-__device__ __forceinline__ bool qb_elect() {
-    uint32_t e;
-    asm volatile("{ .reg .pred p; elect.sync _|p, 0xffffffff; selp.b32 %0, 1, 0, p; }" : "=r"(e) :: "memory");
-    return e != 0;
-}
-__device__ __forceinline__ uint32_t qb_desc_lo(uint32_t saddr, uint32_t lbo) { return ((saddr >> 4) & 0x3FFFu) | ((lbo >> 4) << 16); }
-__device__ __forceinline__ uint32_t qb_desc_hi(uint32_t sbo, uint32_t layout) { return (sbo >> 4) | (1u << 14) | (layout << 29); }
-
 // A (tensor memory, hi at column ahi_col, lo at alo_col) x B (K-major weights): 3 passes x KS k-steps, then commit
 template <int KS>
 __device__ __forceinline__ void qb_tcg_issue_ts(uint32_t d, uint32_t ahi_col, uint32_t alo_col, uint32_t bhi_lo, uint32_t blo_lo,
@@ -199,10 +158,10 @@ __device__ __forceinline__ void qb_tcg_issue_ts(uint32_t d, uint32_t ahi_col, ui
         for (int s = 0; s < KS; ++s) {
             const uint32_t a = (pass == 0 ? alo_col : ahi_col) + 8u * s;
             const uint32_t b = (pass == 1 ? blo_lo : bhi_lo) + 16u * s;
-            qb_tcg_mma_ts(d, a, b, b_hi, idesc, (pass == 0 && s == 0) ? 0u : 1u);
+            qb_mma_ts<false>(d, a, b, b_hi, idesc, (pass == 0 && s == 0) ? 0u : 1u);
         }
     }
-    qb_tcg_commit(bar);
+    qb_commit(bar);
 }
 // A (smem, MN-major point buffer) x B (smem): 3 passes x 16 k-steps (128 points); `acc0`: accumulate into D from the start
 __device__ __forceinline__ void qb_tcg_issue_ss(uint32_t d, uint32_t ahi_lo, uint32_t alo_lo, uint32_t a_hi, uint32_t a_step,
@@ -214,7 +173,7 @@ __device__ __forceinline__ void qb_tcg_issue_ss(uint32_t d, uint32_t ahi_lo, uin
         for (int s = 0; s < 16; ++s) {
             const uint32_t a = (pass == 0 ? alo_lo : ahi_lo) + a_step * s;
             const uint32_t b = (pass == 1 ? blo_lo : bhi_lo) + b_step * s;
-            qb_tcg_mma_ss(d, a, a_hi, b, b_hi, idesc, (pass == 0 && s == 0) ? acc0 : 1u);
+            qb_mma_ss<false>(d, a, a_hi, b, b_hi, idesc, (pass == 0 && s == 0) ? acc0 : 1u);
         }
     }
 }
@@ -222,12 +181,12 @@ __device__ __forceinline__ void qb_tcg_issue_ss(uint32_t d, uint32_t ahi_lo, uin
 // everybody: my stores (tensor memory and shared memory) are visible to the tensor core; returns after arriving
 __device__ __forceinline__ void qb_tcg_publish(QbTcgCtx& cx) {
     qb_tmem_st_wait();
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    qb_fence_proxy_async();
     qb_tc_fence_before();
     qb_mbar_arrive(cx.abar);
 }
 __device__ __forceinline__ void qb_tcg_wait(uint32_t bar, QbTcgCtx& cx, int bit) {
-    qb_mbar_wait(bar, (cx.ph >> bit) & 1u);
+    qb_mbar_wait_timed(bar, (cx.ph >> bit) & 1u);
     cx.ph ^= 1u << bit;
     qb_tc_fence_after();
 }
@@ -347,7 +306,7 @@ __device__ __forceinline__ double qb_tcg_eval(const QbTcgPlan& tp, QbTcgCtx& cx,
         park_to_smem(tp.c_a0hi, tp.c_a0lo, a0hi, a0lo, (uint32_t)tp.a0_sbo);
         qb_tcg_publish(cx);
         if (warp == 0) {
-            qb_mbar_wait(cx.abar, cx.ph & 1u);
+            qb_mbar_wait_timed(cx.abar, cx.ph & 1u);
             qb_tc_fence_after();
             if (qb_elect())
                 qb_tcg_issue_ts<KS>(cx.tmem + tp.c_d1, cx.tmem + tp.c_a0hi, cx.tmem + tp.c_a0lo, w1hi_lo, w1lo_lo, w_hi, id_fwd, cx.barf);
@@ -407,7 +366,7 @@ __device__ __forceinline__ double qb_tcg_eval(const QbTcgPlan& tp, QbTcgCtx& cx,
         }
         qb_tcg_publish(cx);
         if (warp == 0) {
-            qb_mbar_wait(cx.abar, cx.ph & 1u);
+            qb_mbar_wait_timed(cx.abar, cx.ph & 1u);
             qb_tc_fence_after();
             if (qb_elect()) {
                 qb_tcg_issue_ts<KS>(cx.tmem + tp.c_d0, cx.tmem + tp.c_zhi, cx.tmem + tp.c_zlo, w1thi_lo, w1tlo_lo, w_hi, id_fwd, cx.barb);
@@ -416,7 +375,7 @@ __device__ __forceinline__ double qb_tcg_eval(const QbTcgPlan& tp, QbTcgCtx& cx,
                 const uint32_t xs = qb_smem_u32(smem + tp.xt + (t & 1) * QB_TCG_XT_TILE);
                 qb_tcg_issue_ss(cx.tmem + tp.c_db1, zhi_lo, zlo_lo, z_hi, z_step, qb_desc_lo(xs, 144u),
                                 qb_desc_lo(xs + QB_TCG_XT_HALF, 144u), x_hi, 18u, id_dx, acc0);
-                qb_tcg_commit(cx.barw);
+                qb_commit(cx.barw);
             }
             __syncwarp();
         }
@@ -450,7 +409,7 @@ __device__ __forceinline__ double qb_tcg_eval(const QbTcgPlan& tp, QbTcgCtx& cx,
         if (more) park_to_smem(tp.c_a0hi, tp.c_a0lo, a0hi, a0lo, (uint32_t)tp.a0_sbo);
         qb_tcg_publish(cx);
         if (warp == 0) {
-            qb_mbar_wait(cx.abar, cx.ph & 1u);
+            qb_mbar_wait_timed(cx.abar, cx.ph & 1u);
             qb_tc_fence_after();
             if (qb_elect()) {
                 if (more)
@@ -458,7 +417,7 @@ __device__ __forceinline__ double qb_tcg_eval(const QbTcgPlan& tp, QbTcgCtx& cx,
                 const uint32_t xs = qb_smem_u32(smem + tp.xt + (t & 1) * QB_TCG_XT_TILE);
                 qb_tcg_issue_ss(cx.tmem + tp.c_dw0, zhi_lo, zlo_lo, z_hi, z_step, qb_desc_lo(xs, 144u),
                                 qb_desc_lo(xs + QB_TCG_XT_HALF, 144u), x_hi, 18u, id_dx, t > 0 ? 1u : 0u);
-                qb_tcg_commit(cx.barz);
+                qb_commit(cx.barz);
             }
             __syncwarp();
         }

@@ -45,7 +45,7 @@
 #include <stdint.h>
 #include "qb_plan.h"
 #include "qb_tc.cuh"
-#include "qb_tc3.cuh"
+#include "qb_tcgen05.cuh"
 #include "qb_tg8_plan.h"
 
 
@@ -80,73 +80,23 @@ __device__ __forceinline__ float qb_tg8_pow2(int e) { return __uint_as_float((ui
 template <int H>
 __device__ __forceinline__ uint32_t qb_tg8_init(const QbTg8Plan& tp, unsigned char* smem) {
     using D = QbTg8Dim<H>;
-    if ((threadIdx.x >> 5) == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
-                     :: "r"(qb_smem_u32(smem + QB_TG8_SLOT)), "r"((uint32_t)tp.tmem_cols) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    if (threadIdx.x == 0) {
-        const uint32_t b = qb_smem_u32(smem);
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(b + QB_TG8_BAR_F), "r"(1u) : "memory");
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(b + QB_TG8_BAR_B), "r"(1u) : "memory");
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(b + QB_TG8_BAR_W), "r"(1u) : "memory");
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(b + QB_TG8_BAR_Z), "r"(1u) : "memory");
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(b + QB_TG8_BAR_RDY), "r"((uint32_t)D::NCOMP) : "memory");
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(b + QB_TG8_BAR_L), "r"(1u) : "memory");
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(b + QB_TG8_BAR_RDY2), "r"((uint32_t)D::NCOMP) : "memory");
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(b + QB_TG8_BAR_RDY3), "r"((uint32_t)D::NCOMP) : "memory");
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    qb_tc_fence_before();
-    __syncthreads();
-    qb_tc_fence_after();
-    return *reinterpret_cast<volatile uint32_t*>(smem + QB_TG8_SLOT);
+    const uint32_t bars[8] = {QB_TG8_BAR_F, QB_TG8_BAR_B, QB_TG8_BAR_W, QB_TG8_BAR_Z, QB_TG8_BAR_RDY, QB_TG8_BAR_L, QB_TG8_BAR_RDY2, QB_TG8_BAR_RDY3};
+    const uint32_t counts[8] = {1u, 1u, 1u, 1u, (uint32_t)D::NCOMP, 1u, (uint32_t)D::NCOMP, (uint32_t)D::NCOMP};
+    return qb_tc_start(smem, QB_TG8_SLOT, (uint32_t)tp.tmem_cols, bars, counts);
 }
-__device__ __forceinline__ void qb_tg8_fini(const QbTg8Plan& tp, uint32_t tmem) {
-    qb_tc_fence_before();
-    __syncthreads();
-    if ((threadIdx.x >> 5) == 0)
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(tmem), "r"((uint32_t)tp.tmem_cols) : "memory");
-}
-// thread 0, between two block barriers: every phase of the previous evaluation has completed, start again at parity 0
+// between evaluations (thread 0): every barrier starts again at parity 0
 template <int H>
 __device__ __forceinline__ void qb_tg8_reset_barriers(unsigned char* smem) {
     using D = QbTg8Dim<H>;
-    const uint32_t b = qb_smem_u32(smem);
-    const uint32_t off[8] = {QB_TG8_BAR_F, QB_TG8_BAR_B, QB_TG8_BAR_W, QB_TG8_BAR_Z, QB_TG8_BAR_RDY, QB_TG8_BAR_L, QB_TG8_BAR_RDY2, QB_TG8_BAR_RDY3};
-#pragma unroll
-    for (int i = 0; i < 8; ++i) {
-        asm volatile("mbarrier.inval.shared::cta.b64 [%0];" :: "r"(b + off[i]) : "memory");
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(b + off[i]), "r"((i == 4 || i >= 6) ? (uint32_t)D::NCOMP : 1u) : "memory");
-    }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-}
-
-// bounded polling wait (no suspend hint): traps after ~2^28 polls instead of hanging
-__device__ __forceinline__ void qb_tg8_spin(uint32_t bar, uint32_t parity) {
-#pragma unroll 1
-    for (int it = 0; it < (1 << 28); ++it) {
-        uint32_t ok;
-        asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.b32 %0, 1, 0, p; }"
-                     : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-        if (ok) return;
-    }
-    __trap();
-}
-__device__ __forceinline__ void qb_tg8_st4(uint32_t taddr, const uint32_t (&v)[4]) {
-    asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1,%2,%3,%4};" :: "r"(taddr), "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]) : "memory");
+    const uint32_t bars[8] = {QB_TG8_BAR_F, QB_TG8_BAR_B, QB_TG8_BAR_W, QB_TG8_BAR_Z, QB_TG8_BAR_RDY, QB_TG8_BAR_L, QB_TG8_BAR_RDY2, QB_TG8_BAR_RDY3};
+    const uint32_t counts[8] = {1u, 1u, 1u, 1u, (uint32_t)D::NCOMP, 1u, (uint32_t)D::NCOMP, (uint32_t)D::NCOMP};
+    qb_mbar_reset(smem, bars, counts);
 }
 // fp16 pair -> two floats
 __device__ __forceinline__ float2 qb_tg8_unpack(uint32_t w) {
     float a, b;
     asm("{ .reg .b16 l, h; mov.b32 {l, h}, %2; cvt.f32.f16 %0, l; cvt.f32.f16 %1, h; }" : "=f"(a), "=f"(b) : "r"(w));
     return make_float2(a, b);
-}
-// (x0, x1) -> fp16 pair hi (round to nearest) and fp16 pair lo = x - hi
-__device__ __forceinline__ void qb_tg8_split(float x0, float x1, uint32_t& hi, uint32_t& lo) {
-    uint32_t nlo;
-    qb3_split_f16(x0, x1, hi, nlo);
-    lo = nlo ^ 0x80008000u;
 }
 // S * tanh of four pre-activations that were already multiplied by 2 log2 e (one reciprocal for the four, as
 // qb_tanh4_prescaled)
@@ -256,7 +206,7 @@ __device__ __forceinline__ void qb_tg8_stage(const QbTg8Plan& tp, unsigned char*
                 else if (q + u == tp.in_dim && tp.b0_off >= 0) v[u] = theta[tp.b0_off + i] * sc0;
             }
             uint32_t h2, l2;
-            qb_tg8_split(v[0], v[1], h2, l2);
+            qb_split_f16(v[0], v[1], h2, l2);
             const int idx = ((i >> 3) * 128 + (q >> 3) * 64 + (i & 7) * 8 + (q & 7)) >> 1;
             hi[idx] = h2; lo[idx] = l2;
         }
@@ -272,7 +222,7 @@ __device__ __forceinline__ void qb_tg8_stage(const QbTg8Plan& tp, unsigned char*
             const bool real = j < hr && i < hr;
             const float w0 = real ? theta[tp.w1_off + j * hr + i] : 0.0f, w1 = real ? theta[tp.w1_off + j * hr + i + 1] : 0.0f;
             uint32_t h2, l2;
-            qb_tg8_split(w0 * wscale, w1 * wscale, h2, l2);
+            qb_split_f16(w0 * wscale, w1 * wscale, h2, l2);
             hi[cm * 32 + lane] = h2; lo[cm * 32 + lane] = l2;
         }
     }
@@ -296,17 +246,9 @@ __device__ __forceinline__ void qb_tg8_stage(const QbTg8Plan& tp, unsigned char*
         F[tp.sc + QB_TG8_S_SX] = qb_tg8_pow2(sX);
         F[tp.sc + QB_TG8_S_C0] = qb_tg8_pow2(-sX - s0);                // DL -> 2 log2 e * (W0 x + b0)
     }
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    qb_fence_proxy_async();
 }
 
-// ---- MMA issue (one elected lane of the issue warp).  Descriptors are {lo, hi} 32-bit halves; k-steps add a constant to lo.
-__device__ __forceinline__ void qb_tg8_mma(uint32_t d, uint32_t alo, uint32_t ahi, uint32_t blo, uint32_t bhi, uint32_t idesc, uint32_t acc) {
-    asm volatile("{ .reg .pred p; .reg .b64 da, db; setp.ne.b32 p, %6, 0; mov.b64 da, {%1, %2}; mov.b64 db, {%3, %4}; "
-                 "tcgen05.mma.cta_group::1.kind::f16 [%0], da, db, %5, p; }"
-                 :: "r"(d), "r"(alo), "r"(ahi), "r"(blo), "r"(bhi), "r"(idesc), "r"(acc) : "memory");
-}
-__device__ __forceinline__ uint32_t qb_tg8_dlo(uint32_t saddr, uint32_t lbo) { return ((saddr >> 4) & 0x3FFFu) | ((lbo >> 4) << 16); }
-__device__ __forceinline__ uint32_t qb_tg8_dhi(uint32_t sbo) { return (sbo >> 4) | (1u << 14); }
 // three passes (a_lo*b_hi, a_hi*b_lo, a_hi*b_hi) x KS k-steps of 16; *_img are descriptor low words of the hi / lo images;
 // idesc1: instruction descriptor of the pass that reads b_lo (DW1: the lo image of a0 has no ones block, N = 128 there)
 template <int KS>
@@ -322,7 +264,7 @@ __device__ __forceinline__ void qb_tg8_issue3(uint32_t d, uint32_t a_hi_img, uin
         for (int s = 0; s < KS; ++s) {
             const uint32_t a = (pass == 0 ? a_lo_img : a_hi_img) + a_step * s;
             const uint32_t b = (pass == 1 ? b_lo_img : b_hi_img) + b_step * s;
-            qb_tg8_mma(d, a, a_dhi, b, b_dhi, pass == 1 ? idesc1 : idesc, (pass == 0 && s == 0) ? acc0 : 1u);
+            qb_mma_ss<true>(d, a, a_dhi, b, b_dhi, pass == 1 ? idesc1 : idesc, (pass == 0 && s == 0) ? acc0 : 1u);
         }
     }
 }
@@ -358,36 +300,36 @@ __device__ __forceinline__ double qb_tg8_eval(const QbTg8Plan& tp, uint32_t tmem
         const uint32_t id_dw1 = id_unt | ((uint32_t)((H + 16) >> 3) << 17);
         const uint32_t id_dw1n = id_unt | ((uint32_t)(H >> 3) << 17);
         const uint32_t id_dw0 = id_unt | ((16u >> 3) << 17);
-        const uint32_t dh_a = qb_tg8_dhi(128u), dh_b = qb_tg8_dhi(2048u), dh_w = qb_tg8_dhi((uint32_t)D::WSBO);   // SBO 128 / 2048 / 16 H
+        const uint32_t dh_a = qb_desc_hi(128u, 0u), dh_b = qb_desc_hi(2048u, 0u), dh_w = qb_desc_hi((uint32_t)D::WSBO, 0u);   // SBO 128 / 2048 / 16 H
         const uint32_t a_img = sb + (uint32_t)tp.a_img, z_img = sb + (uint32_t)tp.z_img, w_img = sb + (uint32_t)tp.w_img,
                        w0_img = sb + (uint32_t)tp.w0_img;
         // K-major views of the point images and the MN-major view of W: LBO 2048; the other views: LBO 128
-        const uint32_t aK_hi = qb_tg8_dlo(a_img, 2048u), aK_lo = qb_tg8_dlo(a_img + D::AIMG, 2048u);
-        const uint32_t aM_hi = qb_tg8_dlo(a_img, 128u), aM_lo = qb_tg8_dlo(a_img + D::AIMG, 128u);
-        const uint32_t zK_hi = qb_tg8_dlo(z_img, 2048u), zK_lo = qb_tg8_dlo(z_img + D::IMG, 2048u);
-        const uint32_t zM_hi = qb_tg8_dlo(z_img, 128u), zM_lo = qb_tg8_dlo(z_img + D::IMG, 128u);
-        const uint32_t wK_hi = qb_tg8_dlo(w_img, 128u), wK_lo = qb_tg8_dlo(w_img + D::WIMG, 128u);
-        const uint32_t wM_hi = qb_tg8_dlo(w_img, (uint32_t)D::WSBO), wM_lo = qb_tg8_dlo(w_img + D::WIMG, (uint32_t)D::WSBO);
-        const uint32_t w0_hi = qb_tg8_dlo(w0_img, 128u), w0_lo = qb_tg8_dlo(w0_img + D::W0IMG, 128u), dh_w0 = qb_tg8_dhi(256u);
+        const uint32_t aK_hi = qb_desc_lo(a_img, 2048u), aK_lo = qb_desc_lo(a_img + D::AIMG, 2048u);
+        const uint32_t aM_hi = qb_desc_lo(a_img, 128u), aM_lo = qb_desc_lo(a_img + D::AIMG, 128u);
+        const uint32_t zK_hi = qb_desc_lo(z_img, 2048u), zK_lo = qb_desc_lo(z_img + D::IMG, 2048u);
+        const uint32_t zM_hi = qb_desc_lo(z_img, 128u), zM_lo = qb_desc_lo(z_img + D::IMG, 128u);
+        const uint32_t wK_hi = qb_desc_lo(w_img, 128u), wK_lo = qb_desc_lo(w_img + D::WIMG, 128u);
+        const uint32_t wM_hi = qb_desc_lo(w_img, (uint32_t)D::WSBO), wM_lo = qb_desc_lo(w_img + D::WIMG, (uint32_t)D::WSBO);
+        const uint32_t w0_hi = qb_desc_lo(w0_img, 128u), w0_lo = qb_desc_lo(w0_img + D::W0IMG, 128u), dh_w0 = qb_desc_hi(256u, 0u);
         // Hand-overs from the compute threads.  Two arrivals of one thread on the same mbarrier must be separated by a wait that
         // depends on the issue warp having seen the first one (else a fast thread's second arrival completes the phase while a slow
         // thread has not arrived once): the second hand-over of phase A follows the first without such a wait and has its own barrier.
         // The issue warp polls without a suspend hint: every hand-over is on the critical path of the tile loop.
         uint32_t n = 0, n2 = 0, n3 = 0;
         auto wait_rdy = [&]() {
-            qb_tg8_spin(bar_rdy, n & 1u);
+            qb_mbar_spin(bar_rdy, n & 1u);
             ++n;
             qb_tc_fence_after();
             __syncwarp();
         };
         auto wait_rdy3 = [&]() {
-            qb_tg8_spin(bar_rdy3, n3 & 1u);
+            qb_mbar_spin(bar_rdy3, n3 & 1u);
             ++n3;
             qb_tc_fence_after();
             __syncwarp();
         };
         auto wait_rdy2 = [&]() {
-            qb_tg8_spin(bar_rdy2, n2 & 1u);
+            qb_mbar_spin(bar_rdy2, n2 & 1u);
             ++n2;
             qb_tc_fence_after();
             __syncwarp();
@@ -395,17 +337,17 @@ __device__ __forceinline__ double qb_tg8_eval(const QbTg8Plan& tp, uint32_t tmem
         // layer 0 of tile u: X image (K-major view, K = 16: one k-step) x W0 image -> R1
         auto issue_l0 = [&](int u) {
             const uint32_t x_img = sb + (uint32_t)tp.x_img + (uint32_t)(u & 1) * 2u * QB_TG8_XIMG;
-            qb_tg8_issue3<1>(tmem + D::C_D1, qb_tg8_dlo(x_img, 2048u), qb_tg8_dlo(x_img + QB_TG8_XIMG, 2048u), dh_a, 0u,
+            qb_tg8_issue3<1>(tmem + D::C_D1, qb_desc_lo(x_img, 2048u), qb_desc_lo(x_img + QB_TG8_XIMG, 2048u), dh_a, 0u,
                              w0_hi, w0_lo, dh_w0, 0u, id_fwd, id_fwd, 0u);
         };
         if (T > 0) {
             wait_rdy();                                                   // X(0) is in the X image
-            if (qb3_elect()) { issue_l0(0); qb3_commit(bar_l); }
+            if (qb_elect()) { issue_l0(0); qb_commit(bar_l); }
             __syncwarp();
             wait_rdy();                                                   // a0(0) is in the a0 image
-            if (qb3_elect()) {
+            if (qb_elect()) {
                 qb_tg8_issue3<KS>(tmem + D::C_D1, aK_hi, aK_lo, dh_a, 256u, wK_hi, wK_lo, dh_w, 16u, id_fwd, id_fwd, 0u);
-                qb3_commit(bar_f);
+                qb_commit(bar_f);
             }
             __syncwarp();
         }
@@ -414,34 +356,34 @@ __device__ __forceinline__ double qb_tg8_eval(const QbTg8Plan& tp, uint32_t tmem
             const uint32_t acc0 = t > 0 ? 1u : 0u;
             if (t + 1 < T) {
                 wait_rdy3();                                              // X(t+1) is in the X image, R1 has been read (EPI1(t), first pass)
-                if (qb3_elect()) { issue_l0(t + 1); qb3_commit(bar_l); }
+                if (qb_elect()) { issue_l0(t + 1); qb_commit(bar_l); }
                 __syncwarp();
             }
             wait_rdy();                                                   // z1(t) is in the z image; R0 is free
             QB_TG8_STAMP(t, 0);
-            if (qb3_elect()) {
+            if (qb_elect()) {
                 qb_tg8_issue3<KS>(tmem + D::C_D0, zK_hi, zK_lo, dh_a, 256u, wM_hi, wM_lo, dh_a, (uint32_t)(2 * D::WSBO) >> 4, id_bwd, id_bwd, 0u);
-                qb3_commit(bar_b);
+                qb_commit(bar_b);
                 qb_tg8_issue3<8>(tmem + D::C_DW1, zM_hi, zM_lo, dh_b, 16u, aM_hi, aM_lo, dh_b, 16u, id_dw1, id_dw1n, acc0);
-                qb3_commit(bar_w);
+                qb_commit(bar_w);
             }
             __syncwarp();
             QB_TG8_STAMP(t, 1);
             if (t + 1 < T) {
                 wait_rdy();                                               // a0(t+1) is in the a0 image, R1 is free
-                if (qb3_elect()) {
+                if (qb_elect()) {
                     qb_tg8_issue3<KS>(tmem + D::C_D1, aK_hi, aK_lo, dh_a, 256u, wK_hi, wK_lo, dh_w, 16u, id_fwd, id_fwd, 0u);
-                    qb3_commit(bar_f);
+                    qb_commit(bar_f);
                 }
                 __syncwarp();
             }
             wait_rdy2();                                                  // z0(t) is in the z image
             QB_TG8_STAMP(t, 2);
-            if (qb3_elect()) {
+            if (qb_elect()) {
                 const uint32_t x_img = sb + (uint32_t)tp.x_img + (uint32_t)(t & 1) * 2u * QB_TG8_XIMG;
-                qb_tg8_issue3<8>(tmem + D::C_DW0, zM_hi, zM_lo, dh_b, 16u, qb_tg8_dlo(x_img, 128u), qb_tg8_dlo(x_img + QB_TG8_XIMG, 128u),
+                qb_tg8_issue3<8>(tmem + D::C_DW0, zM_hi, zM_lo, dh_b, 16u, qb_desc_lo(x_img, 128u), qb_desc_lo(x_img + QB_TG8_XIMG, 128u),
                                  dh_b, 16u, id_dw0, id_dw0, acc0);
-                qb3_commit(bar_z);
+                qb_commit(bar_z);
             }
             __syncwarp();
             QB_TG8_STAMP(t, 3);
@@ -465,7 +407,7 @@ __device__ __forceinline__ double qb_tg8_eval(const QbTg8Plan& tp, uint32_t tmem
         const float4* W4 = reinterpret_cast<const float4*>(F + tp.wl + c);
 
         auto publish = [&](uint32_t bar) {
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+            qb_fence_proxy_async();
             qb_tc_fence_before();
             qb_mbar_arrive(bar);
         };
@@ -502,7 +444,7 @@ __device__ __forceinline__ double qb_tg8_eval(const QbTg8Plan& tp, uint32_t tmem
         auto xstore = [&](int tt) {
             uint32_t h[D::CPG / 2], l[D::CPG / 2];
 #pragma unroll
-            for (int j = 0; j < D::CPG / 2; ++j) qb_tg8_split(xq[2 * j] * sx, xq[2 * j + 1] * sx, h[j], l[j]);
+            for (int j = 0; j < D::CPG / 2; ++j) qb_split_f16(xq[2 * j] * sx, xq[2 * j + 1] * sx, h[j], l[j]);
             unsigned char* xi = x_row + (tt & 1) * 2 * QB_TG8_XIMG;
             if constexpr (D::CPG == 4) {
                 *reinterpret_cast<uint2*>(xi) = make_uint2(h[0], h[1]);
@@ -525,8 +467,8 @@ __device__ __forceinline__ double qb_tg8_eval(const QbTg8Plan& tp, uint32_t tmem
                     float2 z0 = __fmul2_rn(make_float2(__uint_as_float(v[4 * gq]), __uint_as_float(v[4 * gq + 1])), c2);
                     float2 z1 = __fmul2_rn(make_float2(__uint_as_float(v[4 * gq + 2]), __uint_as_float(v[4 * gq + 3])), c2);
                     qb_tg8_tanh4(z0, z1, 16384.0f);
-                    qb_tg8_split(z0.x, z0.y, o[2 * gq], o[8 + 2 * gq]);
-                    qb_tg8_split(z1.x, z1.y, o[2 * gq + 1], o[8 + 2 * gq + 1]);
+                    qb_split_f16(z0.x, z0.y, o[2 * gq], o[8 + 2 * gq]);
+                    qb_split_f16(z1.x, z1.y, o[2 * gq + 1], o[8 + 2 * gq + 1]);
                 }
                 qb_tmem_st16(tl + D::C_D1 + c + 16 * hf, o);
             }
@@ -538,7 +480,7 @@ __device__ __forceinline__ double qb_tg8_eval(const QbTg8Plan& tp, uint32_t tmem
             yv = yn;
             xstore(0);
             publish(bar_rdy);
-            qb3_wait(bar_l, 0u);
+            qb_mbar_wait_counted(bar_l, 0u);
             qb_tc_fence_after();
             epil();
             qb_tmem_st_wait();
@@ -553,7 +495,7 @@ __device__ __forceinline__ double qb_tg8_eval(const QbTg8Plan& tp, uint32_t tmem
             // ---------------- phase B: EPI1(t)
             QB_TG8_STAMP(t, 0);
             if (more) fetch(t + 1);
-            qb3_wait(bar_f, (uint32_t)t & 1u);
+            qb_mbar_wait_counted(bar_f, (uint32_t)t & 1u);
             qb_tc_fence_after();
             QB_TG8_STAMP(t, 1);
             {
@@ -588,7 +530,7 @@ __device__ __forceinline__ double qb_tg8_eval(const QbTg8Plan& tp, uint32_t tmem
                 const float dy = r * is2, dyz = dy * sz1;
                 const float2 dy2 = make_float2(dy, dy), dyz2 = make_float2(dyz, dyz), one2 = make_float2(1.0f, 1.0f);
                 if (grp == 0) { ssq = fmaf(r, r, ssq); dbl += dy; }
-                if (t > 0) { qb3_wait(bar_z, (uint32_t)(t - 1) & 1u); qb_tc_fence_after(); }     // DW0(t-1) has read the z and X images
+                if (t > 0) { qb_mbar_wait_counted(bar_z, (uint32_t)(t - 1) & 1u); qb_tc_fence_after(); }     // DW0(t-1) has read the z and X images
                 QB_TG8_STAMP(t, 3);
                 if (more) {
                     xstore(t + 1);
@@ -612,8 +554,8 @@ __device__ __forceinline__ double qb_tg8_eval(const QbTg8Plan& tp, uint32_t tmem
                             const float2 z23 = __fmul2_rn(__fmul2_rn(make_float2(w.z, w.w), dyz2), __ffma2_rn(make_float2(-a23.x, -a23.y), a23, one2));
                             dwl2[8 * hf + 2 * gq] = __ffma2_rn(dy2, a01, dwl2[8 * hf + 2 * gq]);
                             dwl2[8 * hf + 2 * gq + 1] = __ffma2_rn(dy2, a23, dwl2[8 * hf + 2 * gq + 1]);
-                            qb_tg8_split(z01.x, z01.y, h[2 * g2], l[2 * g2]);
-                            qb_tg8_split(z23.x, z23.y, h[2 * g2 + 1], l[2 * g2 + 1]);
+                            qb_split_f16(z01.x, z01.y, h[2 * g2], l[2 * g2]);
+                            qb_split_f16(z23.x, z23.y, h[2 * g2 + 1], l[2 * g2 + 1]);
                         }
                         *reinterpret_cast<uint4*>(z_hi + 2048 * (2 * hf + jj)) = make_uint4(h[0], h[1], h[2], h[3]);
                         *reinterpret_cast<uint4*>(z_lo + 2048 * (2 * hf + jj)) = make_uint4(l[0], l[1], l[2], l[3]);
@@ -625,14 +567,14 @@ __device__ __forceinline__ double qb_tg8_eval(const QbTg8Plan& tp, uint32_t tmem
             // ---------------- phase A: EPIL(t+1) while BWD(t) runs, EPI0(t) while DW1(t) runs; results stay in tensor memory until
             // DW1(t) has read the images
             if (more) {
-                qb3_wait(bar_l, (uint32_t)(t + 1) & 1u);               // layer 0 of tile t+1 is in R1 (issued ahead of BWD(t))
+                qb_mbar_wait_counted(bar_l, (uint32_t)(t + 1) & 1u);               // layer 0 of tile t+1 is in R1 (issued ahead of BWD(t))
                 qb_tc_fence_after();
                 QB_TG8_STAMP(t, 10);
                 epil();
                 yv = yn;
             }
             QB_TG8_STAMP(t, 5);
-            qb3_wait(bar_b, (uint32_t)t & 1u);
+            qb_mbar_wait_counted(bar_b, (uint32_t)t & 1u);
             qb_tc_fence_after();
             QB_TG8_STAMP(t, 6);
             {
@@ -654,7 +596,7 @@ __device__ __forceinline__ double qb_tg8_eval(const QbTg8Plan& tp, uint32_t tmem
                             const float2 da = __ffma2_rn(make_float2(-a.x, -a.y), a, one);
                             const float2 d = make_float2(__uint_as_float(v[8 * jj + 2 * w]), __uint_as_float(v[8 * jj + 2 * w + 1]));
                             const float2 z = __fmul2_rn(__fmul2_rn(d, k2), da);
-                            qb_tg8_split(z.x, z.y, o[4 * jj + w], o[8 + 4 * jj + w]);
+                            qb_split_f16(z.x, z.y, o[4 * jj + w], o[8 + 4 * jj + w]);
                         }
                     }
                     qb_tmem_st16(tl + D::C_D0 + c + 16 * hf, o);      // the z image is still an operand of DW1(t)
@@ -662,7 +604,7 @@ __device__ __forceinline__ double qb_tg8_eval(const QbTg8Plan& tp, uint32_t tmem
             }
             qb_tmem_st_wait();
             QB_TG8_STAMP(t, 7);
-            qb3_wait(bar_w, (uint32_t)t & 1u);                      // DW1(t) has read the z and a0 images
+            qb_mbar_wait_counted(bar_w, (uint32_t)t & 1u);                      // DW1(t) has read the z and a0 images
             qb_tc_fence_after();
             QB_TG8_STAMP(t, 8);
             if (more) {
@@ -673,7 +615,7 @@ __device__ __forceinline__ double qb_tg8_eval(const QbTg8Plan& tp, uint32_t tmem
             publish(bar_rdy2);                                       // => DW0(t)
             QB_TG8_STAMP(t, 9);
         }
-        if (T > 0) { qb3_wait(bar_z, (uint32_t)(T - 1) & 1u); qb_tc_fence_after(); }
+        if (T > 0) { qb_mbar_wait_counted(bar_z, (uint32_t)(T - 1) & 1u); qb_tc_fence_after(); }
 
         // ---------------- gradient out: row j (G1) / i (G0).  An M = 128 accumulator keeps row m in lane m; an M = 64 one in
         // lane (m % 16) + 32 (m / 16): the first 16 lanes of every warp quarter

@@ -48,7 +48,7 @@ __device__ __forceinline__ void qb_tc3_drain(const QbTcPlan& tp, const QbTcCtx& 
     if ((threadIdx.x >> 5) == 8 && cx.phase && bulk) {
         const int T = (int)((N + 127) / 128);
         for (int u = 0; u < 3 && u < T; ++u)
-            qb_mbar_wait(qb_smem_u32(smem) + (uint32_t)tp.v3_xbar + 8u * u, (cx.hphase >> u) & 1u);
+            qb_mbar_wait_timed(qb_smem_u32(smem) + (uint32_t)tp.v3_xbar + 8u * u, (cx.hphase >> u) & 1u);
     }
 }
 
@@ -75,7 +75,7 @@ __global__ void __launch_bounds__(Qb3Dim<H>::NCOMP + 32, H == 64 ? 2 : 1) k_logp
     const float* xs = a.xsplit ? a.xsplit + (n0 >> 7) * (2 * 128 * Qb3K0<H>::value) : nullptr;
     const double ssq = qb_tc3_eval_any<H, false>(tp, cx, smem_tc, a.x + k * a.xs, a.y + k * a.ys, n0, n1, xs);
     if (threadIdx.x == 0) a.part[k * a.S + s] = ssq;
-    qb_tc_fini(tp, cx);
+    qb_tc_stop(cx.tmem, (uint32_t)tp.tmem_cols);
 }
 
 __global__ void __launch_bounds__(288, 2)
@@ -241,7 +241,7 @@ k_amcmc_tc3(const __grid_constant__ QbTcPlan tp, const __grid_constant__ ChainAr
     for (int i = tid; i < P; i += nt) { curg[i] = cur_s[i]; psg[i] = ps_s[i]; }
     if (tid == 0) { c.lp[k] = lp_cur; c.map_lp[k] = map_lp; c.naccept[k] = na; a.prop_kind[k] = kind; }
     QB3_STAMP(80, 3);
-    qb_tc_fini(tp, cx);
+    qb_tc_stop(cx.tmem, (uint32_t)tp.tmem_cols);
 }
 
 #ifdef QB3_TRACE
@@ -270,7 +270,7 @@ k_predict_tc3(const __grid_constant__ QbTcPlan tp, const float* __restrict__ the
     Qb3SinkStore sink;
     sink.out = out + m * N;
     qb_tc3_dispatch<H, false>(tp, cx, smem_tc, x, n0, n1, nullptr, sink);
-    qb_tc_fini(tp, cx);
+    qb_tc_stop(cx.tmem, (uint32_t)tp.tmem_cols);
 }
 
 cudaError_t qb_tc3_launch_logpost(const QbTcPlan& tp, const EvalArgs<float>& a, dim3 grid, cudaStream_t st) {
