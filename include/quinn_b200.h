@@ -86,7 +86,7 @@ const char* qb_last_error(void);
  * qb_version() differs from the QB_ABI_VERSION it was written against (quinn_b200/_lib.py does), and can check its
  * struct mirrors against qb_struct_sizes(): out[0..n) = sizeof of qb_layer_t, qb_net_t, qb_lik_t, qb_data_t, qb_chain_t,
  * qb_rng_t, qb_record_t, qb_amcmc_t, qb_hmc_t (declaration order); returns how many sizes exist. */
-#define QB_ABI_VERSION 202
+#define QB_ABI_VERSION 203
 int qb_version(void);
 int qb_struct_sizes(int64_t* out, int n);
 
@@ -136,6 +136,22 @@ int qb_logpost_kfac(const qb_net_t* net, int dtype, const void* theta, const qb_
 /* Launch plan of kernel 6 over N points: out[0..4] = {tile points TM, threads per block, dynamic smem bytes, N-splits S
  * (one block each), factor elements F}.  Returns -1 (with qb_last_error) for a network kernel 6 refuses. */
 int qb_kfac_plan_info(const qb_net_t* net, int dtype, int64_t N, int64_t* out);
+
+/* Kernel 7.  Network outputs and their per-point Jacobians with respect to theta[P] over x[N, in_dim] (dtype), as
+ * per-layer pairs: for output j of point n, layer l's part of d f_j(x_n) / d [W_l | b_l] is outer(d_l[j, :, n],
+ * [a_l[:, n]; 1]) with a_l the layer's input and d_l[j] = d f_j / d z_l its pre-activation gradient.  Polynomial terms
+ * (each term gets coef_m times that part) and layers sharing weights (parts summed) are left to the caller.
+ * out: [N, o] dtype, f(x_n) with final_exp applied.
+ * fac: dtype, N * F elements with F = sum_l (n_in_l + o * n_out_l), unit-major; per layer, in order,
+ *     a_l as [n_in_l, N], then d_l as [o, n_out_l, N].
+ * Refused (error text says why): networks that kernel 2 evaluates on the layer-streamed path (plan code 5), NULL
+ * arguments, N < 0.  N == 0 launches no kernel.  No reduction over the points: fp64 results are bit-identical run to
+ * run.  Replaces nothing in the reference; it feeds NN_Laplace.predict_mom_glm (DESIGN.md section 4h). */
+int qb_predict_jac(const qb_net_t* net, int dtype, const void* theta, const void* x, int64_t N, void* out, void* fac,
+                   void* stream);
+/* Launch plan of kernel 7 over N points: out[0..4] = {tile points TM, threads per block, dynamic smem bytes, blocks (runs
+ * of whole tiles, 0 for N == 0), factor rows F}.  Returns -1 (with qb_last_error) for a network kernel 7 refuses. */
+int qb_jac_plan_info(const qb_net_t* net, int dtype, int64_t N, int64_t* out);
 
 /* ---- Batched ensemble training (SURVEY.md 8f rank 1) --------------------------------------------
  * NN_Ens.fit (quinn/solvers/nn_ens.py:51-69) trains nens members one after the other, each with

@@ -64,7 +64,7 @@ class qb_hmc_t(C.Structure):
                 ('mom', C.c_void_p), ('prop', C.c_void_p), ('grad_prop', C.c_void_p)]
 
 
-QB_ABI_VERSION = 202          # include/quinn_b200.h
+QB_ABI_VERSION = 203          # include/quinn_b200.h
 ABI_STRUCTS = (qb_layer_t, qb_net_t, qb_lik_t, qb_data_t, qb_chain_t, qb_rng_t, qb_record_t, qb_amcmc_t, qb_hmc_t)
 
 # every symbol include/quinn_b200.h declares: name -> (restype, argtypes)
@@ -88,6 +88,8 @@ SYMBOLS = {
     'qb_logpost_kfac': (C.c_int, [C.POINTER(qb_net_t), C.c_int, _P, C.POINTER(qb_data_t), C.POINTER(qb_lik_t), _P, _P,
                                   C.c_size_t, _P]),
     'qb_kfac_plan_info': (C.c_int, [C.POINTER(qb_net_t), C.c_int, C.c_int64, C.POINTER(C.c_int64)]),
+    'qb_predict_jac': (C.c_int, [C.POINTER(qb_net_t), C.c_int, _P, _P, C.c_int64, _P, _P, _P]),
+    'qb_jac_plan_info': (C.c_int, [C.POINTER(qb_net_t), C.c_int, C.c_int64, C.POINTER(C.c_int64)]),
     'qb_adam_step': (C.c_int, [C.c_int, _P, _P, _P, _P, C.c_int64, C.c_double, C.c_double, C.c_double, C.c_double,
                                C.c_double, C.c_int64, C.c_double, _P]),
     'qb_copy_rows_where': (C.c_int, [C.c_int, _P, _P, _P, C.c_int64, C.c_int64, _P]),

@@ -15,7 +15,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, 'csrc')
 UNITS = ['qb_kernels.cu', 'qb_launch.cu', 'qb_grad_tc.cu', 'qb_grad_tc128.cu', 'qb_value_tc3.cu', 'qb_post.cu']
-HEADERS = ['qb_device.cuh', 'qb_chain.cuh', 'qb_stream.cuh', 'qb_hvp.cuh', 'qb_kfac.cuh', 'qb_tcgen05.cuh', 'qb_tc.cuh', 'qb_tc3.cuh', 'qb_tcg.cuh', 'qb_tg8.cuh', 'qb_tg8_plan.h', 'qb_grad_tc.h', 'qb_grad_tc128.h', 'qb_value_tc3.h', 'qb_plan.h', 'qb_launch.h']
+HEADERS = ['qb_device.cuh', 'qb_chain.cuh', 'qb_stream.cuh', 'qb_hvp.cuh', 'qb_kfac.cuh', 'qb_jac.cuh', 'qb_tcgen05.cuh', 'qb_tc.cuh', 'qb_tc3.cuh', 'qb_tcg.cuh', 'qb_tg8.cuh', 'qb_tg8_plan.h', 'qb_grad_tc.h', 'qb_grad_tc128.h', 'qb_value_tc3.h', 'qb_plan.h', 'qb_launch.h']
 DEPS = [os.path.join(CSRC, f) for f in UNITS + HEADERS] + [os.path.join(ROOT, 'include', 'quinn_b200.h')]
 OUT = os.path.join(HERE, 'lib', 'libquinn_b200.so')
 STAMP = OUT + '.srchash'

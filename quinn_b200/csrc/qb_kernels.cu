@@ -421,6 +421,50 @@ extern "C" int qb_logpost_kfac(const qb_net_t* net, int dtype, const void* theta
     return run_kfac<float>(net, dtype, theta, data, lik, factors, ws, ws_bytes, (cudaStream_t)stream);
 }
 
+// =================================================================================================
+// kernel 7: per-point output Jacobians as per-layer pairs (qb_jac.cuh)
+// =================================================================================================
+template <typename T> struct JacArgs {
+    const T* theta; const T* x;
+    long long N; long long pps;
+    T* out;             // [N, o]
+    T* fac;             // [F, N]
+};
+
+template <typename T>
+__global__ void __launch_bounds__(256, 2) k_predict_jac(const __grid_constant__ QbJacPlan J, const JacArgs<T> a) {
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    const QbSmem S = qb_carve<T>(J.P, smem_raw);
+    const long long s = blockIdx.x;
+    const long long n0 = s * a.pps, n1 = min(a.N, n0 + a.pps);
+    qb_jac_eval<T>(J, S, a.theta, a.x, a.N, n0, n1, a.out, a.fac);
+}
+
+template <typename T>
+static int run_jac(const qb_net_t* net, int dtype, const void* theta, const void* x, int64_t N, void* out, void* fac,
+                   cudaStream_t st) {
+    QbJacLaunch L;
+    if (make_jac_launch(net, dtype, std::max<int64_t>(N, 1), &L)) return -1;
+    if (N == 0) return 0;             // no points: no kernel
+    JacArgs<T> a;
+    a.theta = (const T*)theta; a.x = (const T*)x;
+    a.N = N; a.pps = L.pps;
+    a.out = (T*)out; a.fac = (T*)fac;
+    if (set_smem(k_predict_jac<T>, L.J.P.smem_bytes)) return -2;
+    k_predict_jac<T><<<(unsigned)L.S, L.J.P.nthreads, L.J.P.smem_bytes, st>>>(L.J, a);
+    QB_CUDA(cudaGetLastError());
+    g_launches += 1;
+    return 0;
+}
+
+extern "C" int qb_predict_jac(const qb_net_t* net, int dtype, const void* theta, const void* x, int64_t N, void* out,
+                              void* fac, void* stream) {
+    if (!theta || (N > 0 && (!x || !out || !fac))) return qb_fail("NULL argument to qb_predict_jac");
+    if (N < 0) return qb_fail("N must not be negative");
+    if (dtype == QB_F64) return run_jac<double>(net, dtype, theta, x, N, out, fac, (cudaStream_t)stream);
+    return run_jac<float>(net, dtype, theta, x, N, out, fac, (cudaStream_t)stream);
+}
+
 // Adam (torch.optim.Adam semantics, quinn/nns/nnfit.py:92-93) on a flat array: g = grad*grad_scale + wd*theta
 template <typename T>
 __global__ void k_adam(T* th, const T* g, T* m, T* v, long long n, double lr, double b1, double b2, double eps, double wd,

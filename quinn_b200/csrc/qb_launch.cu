@@ -677,3 +677,36 @@ extern "C" int qb_kfac_plan_info(const qb_net_t* net, int dtype, int64_t N, int6
     out[0] = L.K.P.TM; out[1] = L.K.P.nthreads; out[2] = L.K.P.smem_bytes; out[3] = L.S; out[4] = L.K.n_factors;
     return 0;
 }
+
+// =================================================================================================
+// kernel 7: per-point output Jacobians as per-layer pairs (qb_jac.cuh)
+// =================================================================================================
+// Kernel 2's resident CUDA-core plan for one theta, the factor rows of every layer, and the N-split: one block per run of
+// whole tiles.  Nothing is reduced over the points, so there are no partial rows to cap.
+int make_jac_launch(const qb_net_t* net, int dtype, long long N, QbJacLaunch* out) {
+    if (check_args(net, dtype, 1, N)) return -1;
+    QbLaunch L;
+    if (make_launch(net, dtype, true, 1, N, true, &L)) return -1;
+    if (L.streamed)
+        return qb_fail("output Jacobians: the network's weights do not fit in shared memory next to one tile of "
+                       "activations, and the layer-streamed path (plan code 5) has no Jacobian kernel");
+    memset(&out->J, 0, sizeof(out->J));
+    out->J.P = L.plan;
+    const QbPlan& P = out->J.P;
+    int row = 0;
+    for (int l = 0; l < P.n_layers; ++l) {
+        out->J.row0[l] = row;
+        row += P.L[l].n_in + P.out_dim * P.L[l].n_out;
+    }
+    out->J.n_rows = row;
+    fit_splits(N, P.TM, want_splits(N, P.TM, 1, 0), &out->S, &out->pps);
+    return 0;
+}
+
+extern "C" int qb_jac_plan_info(const qb_net_t* net, int dtype, int64_t N, int64_t* out) {
+    if (N < 0) return qb_fail("N must not be negative");
+    QbJacLaunch L;
+    if (make_jac_launch(net, dtype, std::max<int64_t>(N, 1), &L)) return -1;
+    out[0] = L.J.P.TM; out[1] = L.J.P.nthreads; out[2] = L.J.P.smem_bytes; out[3] = N > 0 ? L.S : 0; out[4] = L.J.n_rows;
+    return 0;
+}

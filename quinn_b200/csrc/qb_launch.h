@@ -5,6 +5,7 @@
 #include "qb_stream.cuh"
 #include "qb_hvp.cuh"
 #include "qb_kfac.cuh"
+#include "qb_jac.cuh"
 #include "qb_tc.cuh"
 #include "qb_tcg.cuh"
 #include "qb_tg8_plan.h"
@@ -36,12 +37,14 @@ struct QbLaunch {
 };
 struct QbHvpLaunch { QbHvpPlan H; int S; long long pps; size_t ws_bytes; };
 struct QbKfacLaunch { QbKfacPlan K; int S; long long pps; size_t ws_bytes; };
+struct QbJacLaunch { QbJacPlan J; int S; long long pps; };
 
 // the planners return -1 with the error set when they refuse; force_single: one block per chain
 int make_launch(const qb_net_t* net, int dtype, bool want_grad, long long K, long long N, bool force_single, QbLaunch* out);
 int plan_eval(const qb_net_t* net, int dtype, bool want_grad, long long K, long long N, bool force_single, QbLaunch* out);
 int make_hvp_launch(const qb_net_t* net, int dtype, long long K, long long N, QbHvpLaunch* out);
 int make_kfac_launch(const qb_net_t* net, int dtype, long long N, QbKfacLaunch* out);
+int make_jac_launch(const qb_net_t* net, int dtype, long long N, QbJacLaunch* out);
 bool make_tc_plan(const qb_net_t* net, int dtype, QbTcPlan* tp, int allow_v3 = 0);
 // kernel 4's member-parallel grid: chunks of tiles_per_block consecutive tiles, about blocks_wanted blocks over M members
 long long qb_tile_chunks(long long tiles, long long blocks_wanted, long long M, long long* tiles_per_block);

@@ -235,6 +235,46 @@ def logpost_kfac(prob: Problem, theta):
     return out
 
 
+def jac_plan_info(desc: NetDesc, N, dtype=torch.float32):
+    """Launch plan of kernel 7 over N points; raises for a network the kernel refuses.  rows = F, the factor rows of N
+    elements each."""
+    out = (C.c_int64 * 8)()
+    cnet = desc.to_c()
+    _lib.check(_lib.load().qb_jac_plan_info(C.byref(cnet), qb_dtype(dtype), int(N), out), 'qb_jac_plan_info')
+    return dict(TM=out[0], threads=out[1], smem_bytes=out[2], blocks=out[3], rows=out[4])
+
+
+def predict_jac(desc: NetDesc, theta, x, dtype=torch.float32, device='cuda'):
+    """Kernel 7: f[N, o] at one theta[P] and, per layer, dict(a=[n_in, N], d=[o, n_out, N]) with a the layer's input and
+    d[j] = d f_j / d z its pre-activation gradient (views into one buffer).  Layer l's part of d f_j(x_n) / d [W_l | b_l]
+    is outer(d[j, :, n], [a[:, n]; 1])."""
+    device = torch.device(device)
+    theta = as_device(theta, dtype, device)
+    if theta.dim() == 2 and theta.shape[0] == 1:
+        theta = theta[0]
+    x = as_device(x, dtype, device)
+    _need_cuda(theta, x)
+    if theta.dim() != 1 or theta.shape[0] != desc.n_params or x.dim() != 2 or x.shape[1] != desc.in_dim:
+        raise ValueError('predict_jac takes a single theta[P] and x[N, in_dim] that match the network')
+    N, o = x.shape[0], desc.out_dim
+    F = jac_plan_info(desc, N, dtype)['rows']          # raises with the reason when the network is refused
+    out = torch.empty((N, o), dtype=dtype, device=device)
+    fac = torch.empty(N * F, dtype=dtype, device=device)
+    cnet = desc.to_c()
+    with torch.cuda.device(device):
+        rc = _lib.load().qb_predict_jac(C.byref(cnet), qb_dtype(dtype), _ptr(theta), _ptr(x), N, _ptr(out), _ptr(fac),
+                                        _stream())
+    _lib.check(rc, 'qb_predict_jac')
+    pairs, row = [], 0
+    for L in desc.layers:
+        a = fac[row * N:(row + L.n_in) * N].view(L.n_in, N)
+        row += L.n_in
+        d = fac[row * N:(row + o * L.n_out) * N].view(o, L.n_out, N)
+        row += o * L.n_out
+        pairs.append(dict(a=a, d=d))
+    return out, pairs
+
+
 def predict(desc: NetDesc, theta, x, dtype=torch.float32, device='cuda', want_out=True, want_moments=False,
             cnet=None):
     """Kernel 4: theta[M,P], x[N,d] -> out[M,N,o] and/or (mean[N,o], var[N,o], ddof=1)."""

@@ -5,7 +5,9 @@ curvature of its NegLogPost at the MAP is taken on the device, either the exact 
 Hessian-vector product per unit direction), the diagonal Fisher of NNWrap.calc_hess_diag (la_type='diag') or the
 Kronecker-factored Fisher of every Linear layer (la_type='kron': kernel 6, DESIGN.md section 4g).  The curvature is
 factored on the device (torch.linalg.eigh, elementwise, or eigh of each layer's two factors) and the posterior draws
-theta = mu_j + H_j^{-1/2} z sqrt(cov_scale) are formed there, so predictions go straight to kernel 4."""
+theta = mu_j + H_j^{-1/2} z sqrt(cov_scale) are formed there, so predictions go straight to kernel 4.  predict_mom_glm is
+the linearised predictive instead: per-point Jacobians from kernel 7 (DESIGN.md section 4h) contracted with the same
+covariance, no sampling."""
 import copy
 import warnings
 
@@ -131,6 +133,108 @@ class NN_Laplace(NN_RMS):
         desc, thetas, dtype = self._ens_thetas(1)
         out, _, _ = ops.predict(desc, thetas, np.asarray(x), dtype=dtype)
         return out[0].double().cpu().numpy()
+
+    def predict_mom_glm(self, x, msc=0):
+        """Moments of the linearised (GLM) predictive f(x; mu_j) + J_j(x) (theta - mu_j), theta ~ N(mu_j, cov_scale
+        Sigma_j), with Sigma_j the covariance _ens_thetas samples from; members weigh equally.  Deterministic, no
+        observation noise.  Same contract as predict_mom_sample: (mean [N, o], var [N, o] for msc >= 1, cov [N, N, o]
+        for msc == 2), numpy float64.  J_j comes from kernel 7 in the solver's dtype; the contraction with Sigma_j runs
+        in float64 on the device, over chunks of points whose buffers stay under _GLM_CHUNK_BYTES each."""
+        if msc not in (0, 1, 2):
+            raise ValueError(f"msc={msc}, but needs to be 0,1, or 2.")
+        if self.means is None:
+            raise RuntimeError('predict_mom_glm needs the posterior: call fit first')
+        from .. import ops
+        desc = self._desc()
+        x = np.asarray(x)
+        N, o, P = x.shape[0], desc.out_dim, desc.n_params
+        dev = self.means.device
+        F = ops.jac_plan_info(desc, max(N, 1), self.dtype)['rows']
+        step = max(1, _GLM_CHUNK_BYTES // (8 * max(F, o * P)))
+        vsum = torch.zeros((N, o), dtype=torch.float64, device=dev)
+        csum = torch.zeros((o, N, N), dtype=torch.float64, device=dev) if msc == 2 else None
+        fmem = torch.zeros((self.nens, N, o), dtype=torch.float64, device=dev)
+        for j in range(self.nens):
+            mu = self.means[j].to(self.dtype)
+            Bs = []
+            for lo in range(0, N, step):
+                f, pairs = ops.predict_jac(desc, mu, x[lo:lo + step], dtype=self.dtype, device=dev)
+                fmem[j, lo:lo + step] = f
+                if msc == 2:
+                    Bs.append(_glm_factor(self.la_type, self._factors[j], desc, pairs))
+                elif msc == 1:
+                    vsum[lo:lo + step] += _glm_var(self.la_type, self._factors[j], desc, pairs)
+            if msc == 2 and Bs:
+                B = torch.cat(Bs)
+                csum += torch.einsum('nja,mja->jnm', B, B)
+        # law of total variance over equally weighted members, as the mean of the members' variances plus the variance of
+        # their means (the same value as mean_j(v_j + f_j^2) - mean^2, without its cancellation)
+        mean = fmem.mean(0)
+        dev_f = fmem - mean
+        var = cov = None
+        if msc == 2:
+            cv = self.cov_scale * csum / self.nens + torch.einsum('knj,kmj->jnm', dev_f, dev_f) / self.nens  # [o, N, N]
+            var = torch.diagonal(cv, dim1=1, dim2=2).T.cpu().numpy()
+            cov = cv.permute(1, 2, 0).cpu().numpy()
+        elif msc == 1:
+            var = (self.cov_scale * vsum / self.nens + (dev_f * dev_f).mean(0)).cpu().numpy()
+        return mean.cpu().numpy(), var, cov
+
+
+_GLM_CHUNK_BYTES = 1 << 30        # predict_mom_glm: the largest buffer of one chunk of points
+
+
+def assemble_jac(desc, pairs):
+    """J [n, o, P] (float64) of d f_j(x_n) / d theta from kernel 7's per-layer pairs (ops.predict_jac): layer l adds
+    coef_m * outer(d_l[j, :, n], [a_l[:, n]; 1]) at each of its terms (coef_m, w_off_m, b_off_m), so layers that share
+    weights sum their parts.  Runs wherever the pair tensors live."""
+    a0 = pairs[0]['a']
+    n, o = a0.shape[1], desc.out_dim
+    J = torch.zeros((n, o, desc.n_params), dtype=torch.float64, device=a0.device)
+    for L, p in zip(desc.layers, pairs):
+        a, d = p['a'].double(), p['d'].double()
+        gW = torch.einsum('jun,in->njui', d, a).reshape(n, o, L.n_out * L.n_in)
+        gb = d.permute(2, 0, 1)
+        for c, wo, bo in (L.terms or [(1.0, L.w_off, L.b_off)]):
+            J[:, :, wo:wo + L.n_out * L.n_in] += c * gW
+            if bo >= 0:
+                J[:, :, bo:bo + L.n_out] += c * gb
+    return J
+
+
+def _glm_factor(la_type, fac, desc, pairs):
+    """B [n, o, K] with B[n, j] B[m, j]^T = J_j(x_n) Sigma J_j(x_m)^T for one member's factors"""
+    if la_type == 'full':
+        U, isq, _ = fac
+        return assemble_jac(desc, pairs) @ (U * isq)
+    if la_type == 'diag':
+        return assemble_jac(desc, pairs) * fac[0]
+    Bs = []
+    for p, (_, UG, UA, isq, _) in zip(pairs, fac):
+        dr, ar = _kron_rotate(p, UG, UA)                     # [o, n_out, n], [n_in(+1), n]
+        B = dr.permute(2, 0, 1)[:, :, :, None] * ar.T[:, None, None, :] * isq
+        Bs.append(B.reshape(B.shape[0], B.shape[1], -1))
+    return torch.cat(Bs, 2)
+
+
+def _glm_var(la_type, fac, desc, pairs):
+    """diag of J Sigma J^T [n, o] for one member's factors ('kron': per layer sum_rc d'_r^2 a'_c^2 / lambda_rc, with
+    d' = U_G^T d and a' = U_A^T [a; 1], no assembly)"""
+    if la_type != 'kron':
+        return (_glm_factor(la_type, fac, desc, pairs) ** 2).sum(2)
+    v = 0.0
+    for p, (_, UG, UA, isq, _) in zip(pairs, fac):
+        dr, ar = _kron_rotate(p, UG, UA)
+        M = (isq * isq) @ (ar * ar)                          # [n_out, n]: sum_c a'_c^2 / lambda_rc
+        v = v + ((dr * dr) * M[None]).sum(1).T
+    return v
+
+
+def _kron_rotate(p, UG, UA):
+    a, d = p['a'].double(), p['d'].double()
+    if UA.shape[0] > a.shape[0]:                             # a layer with a bias: a~ = [a; 1]
+        a = torch.cat([a, torch.ones((1, a.shape[1]), dtype=a.dtype, device=a.device)])
+    return torch.einsum('ur,jun->jrn', UG, d), UA.T @ a
 
 
 def _check_kron_net(desc):
