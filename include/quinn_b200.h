@@ -268,6 +268,34 @@ int qb_hmc_run(const qb_net_t* net, int dtype, const qb_data_t* data, const qb_l
                qb_chain_t* chain, qb_hmc_t* hm, const qb_rng_t* rng, const qb_record_t* rec,
                int64_t t_start, int64_t nsteps, int init_lp, void* stream);
 
+/* No-U-Turn sampler (Hoffman & Gelman 2014; multinomial, iterative tree building, identity metric): nsteps transitions of
+ * K chains from absolute step t_start, on the same kernel path qb_hmc_run takes for (net, dtype, K).  A transition runs
+ * at most 2^max_depth - 1 leapfrog steps of size eps; it is divergent when H - H0 > 1000 or the log-posterior is not
+ * finite, which stops its tree and leaves the state unchanged.
+ * Step size: per-chain dual averaging (Stan's gamma 0.05, t0 10, kappa 0.75, mu = log(10 epsilon)) towards target_accept
+ * while t_start + s < n_adapt; later transitions use the averaged eps_bar (n_adapt == 0: epsilon throughout).
+ *   log_eps, log_eps_bar, h_bar: [K] double, the adaptation state, carried across calls (so a run split over calls adapts
+ *     as one call); init_lp != 0 sets them to log(epsilon), log(epsilon), 0 and evaluates the incoming theta as
+ *     qb_hmc_run does.
+ *   grad_cur: [K,P] dtype, the gradient at the current state, carried across calls.
+ *   scratch: [K, (9 + 2*max_depth) * P] dtype.
+ * rec: logpost, accepted (1 = the chain moved), samples and logpost0 as qb_hmc_run; alpha = the acceptance statistic (mean
+ * of min(1, exp(H0 - H)) over the transition's new points).  Optional per-transition records at [k*rec->ld + s] (rec is
+ * needed when one is given): rec_depth (int32 doublings), rec_n_leapfrog (int32), rec_diverging (uint8), rec_step_size
+ * (double, the eps used).
+ * Draws (Philox, keyed by seed and chain_offset + k at step t = t_start + s, so results do not depend on sharding or on
+ * how the steps are split over calls): the momentum from QB_STREAM_INCR (stream 0) as qb_hmc_run; from QB_STREAM_NUTS
+ * (stream 5) the four words of index j drive doubling j (bit 0 of word 0: 1 = forwards; word 1 as a uniform: the biased
+ * progressive choice of the new subtree), and word 0 of index 16 + n is the uniform of leapfrog n (counted from 0 over the
+ * transition) in the uniform progressive choice inside its subtree.
+ * Refused (error text says why): REPLAY rng mode, NULL arrays, max_depth outside [1, 12], target_accept outside (0, 1),
+ * epsilon <= 0 or not finite, negative n_adapt, nsteps or t_start.  K == 0 or nsteps == 0 launches nothing. */
+int qb_nuts_run(const qb_net_t* net, int dtype, const qb_data_t* data, const qb_lik_t* lik, qb_chain_t* chain,
+                const qb_rng_t* rng, const qb_record_t* rec, int64_t t_start, int64_t nsteps, int init_lp,
+                double epsilon, int max_depth, int64_t n_adapt, double target_accept, double* log_eps,
+                double* log_eps_bar, double* h_bar, void* grad_cur, void* scratch, int32_t* rec_depth,
+                int32_t* rec_n_leapfrog, uint8_t* rec_diverging, double* rec_step_size, void* stream);
+
 /* ---- Kernel 4: posterior predictive -----------------------------------------------------------
  * Replaces the M sequential forwards of nn_p (quinn/nns/nnwrap.py:330-347), NN_MCMC.predict_ens
  * (nn_mcmc.py:180-200), NN_Ens.predict_ens (nn_ens.py:85-110), QUiNNBase.predict_ens /

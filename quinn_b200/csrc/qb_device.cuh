@@ -973,7 +973,7 @@ __device__ __forceinline__ uint4 qb_philox(uint4 c, uint2 k) {
     }
     return c;
 }
-enum { QB_STREAM_INCR = 0, QB_STREAM_Z0 = 1, QB_STREAM_UNIF = 2, QB_STREAM_VI = 3, QB_STREAM_SWAG = 4 };
+enum { QB_STREAM_INCR = 0, QB_STREAM_Z0 = 1, QB_STREAM_UNIF = 2, QB_STREAM_VI = 3, QB_STREAM_SWAG = 4, QB_STREAM_NUTS = 5 };
 
 __device__ __forceinline__ uint4 qb_rand4(uint64_t seed, int64_t chain, int64_t step, int stream, uint32_t idx4) {
     // seed and chain live in DIFFERENT words (key = seed, counter = chain/step/index): two (seed, chain) pairs never share

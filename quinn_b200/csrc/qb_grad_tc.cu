@@ -8,6 +8,7 @@
 #include "qb_plan.h"
 #include "qb_device.cuh"
 #include "qb_chain.cuh"
+#include "qb_nuts.cuh"
 #include "qb_tc.cuh"
 #include "qb_tcg.cuh"
 #include "qb_grad_tc.h"
@@ -106,6 +107,17 @@ __global__ void __launch_bounds__(H * 8, H == 32 ? 2 : 1) k_hmc_tc(const __grid_
 }
 
 template <int H, int NI, int ACT>
+__global__ void __launch_bounds__(H * 8, H == 32 ? 2 : 1) k_nuts_tc(const __grid_constant__ QbTcgPlan tp, const __grid_constant__ ChainArgs<float> c,
+                                                      const __grid_constant__ NutsArgs<float> a) {
+    extern __shared__ __align__(1024) unsigned char smem_g[];
+    QbTcgCtx cx;
+    qb_tcg_init(tp, smem_g, cx);
+    QbGradTc<H, NI, ACT> eval{tp, cx, smem_g, c, (long long)blockIdx.x};
+    qb_nuts_body<float>(c, a, tp.n_params, reinterpret_cast<double*>(smem_g), eval);
+    qb_tc_stop(cx.tmem, (uint32_t)tp.tmem_cols);
+}
+
+template <int H, int NI, int ACT>
 static cudaError_t launch_eval_t(const QbTcgPlan& tp, const EvalArgs<float>& a, dim3 grid, cudaStream_t st) {
     cudaError_t e = cudaFuncSetAttribute(k_logpost_grad_tc<H, NI, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, tp.smem_bytes);
     if (e != cudaSuccess) return e;
@@ -117,6 +129,14 @@ static cudaError_t launch_hmc_t(const QbTcgPlan& tp, const ChainArgs<float>& c, 
     cudaError_t e = cudaFuncSetAttribute(k_hmc_tc<H, NI, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, tp.smem_bytes);
     if (e != cudaSuccess) return e;
     k_hmc_tc<H, NI, ACT><<<(unsigned)K, tp.nthreads, tp.smem_bytes, st>>>(tp, c, h);
+    return cudaGetLastError();
+}
+
+template <int H, int NI, int ACT>
+static cudaError_t launch_nuts_t(const QbTcgPlan& tp, const ChainArgs<float>& c, const NutsArgs<float>& a, long long K, cudaStream_t st) {
+    cudaError_t e = cudaFuncSetAttribute(k_nuts_tc<H, NI, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, tp.smem_bytes);
+    if (e != cudaSuccess) return e;
+    k_nuts_tc<H, NI, ACT><<<(unsigned)K, tp.nthreads, tp.smem_bytes, st>>>(tp, c, a);
     return cudaGetLastError();
 }
 
@@ -134,4 +154,7 @@ cudaError_t qb_tcg_launch_eval(const QbTcgPlan& tp, const EvalArgs<float>& a, di
 }
 cudaError_t qb_tcg_launch_hmc(const QbTcgPlan& tp, const ChainArgs<float>& c, const HmcArgs<float>& h, long long K, cudaStream_t st) {
     QB_TCG_DISPATCH(launch_hmc_t, tp, c, h, K, st);
+}
+cudaError_t qb_tcg_launch_nuts(const QbTcgPlan& tp, const ChainArgs<float>& c, const NutsArgs<float>& a, long long K, cudaStream_t st) {
+    QB_TCG_DISPATCH(launch_nuts_t, tp, c, a, K, st);
 }

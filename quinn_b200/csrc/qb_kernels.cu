@@ -9,6 +9,7 @@
 #include "quinn_b200.h"
 #include "qb_device.cuh"
 #include "qb_chain.cuh"
+#include "qb_nuts.cuh"
 #include "qb_launch.h"
 #include "qb_value_tc3.h"
 #include "qb_grad_tc.h"
@@ -152,6 +153,16 @@ template <> int launch_hmc_tc128<float>(const QbTg8Plan& tg, const ChainArgs<flo
 template <typename T> static int launch_hmc_tc(const QbTcgPlan&, const ChainArgs<T>&, const HmcArgs<T>&, long long, cudaStream_t) { return qb_fail("tensor-core path is fp32 only"); }
 template <> int launch_hmc_tc<float>(const QbTcgPlan& tg, const ChainArgs<float>& c, const HmcArgs<float>& h, long long K, cudaStream_t st) {
     QB_CUDA(qb_tcg_launch_hmc(tg, c, h, K, st));
+    return 0;
+}
+template <typename T> static int launch_nuts_tc128(const QbTg8Plan&, const ChainArgs<T>&, const NutsArgs<T>&, long long, cudaStream_t) { return qb_fail("tensor-core path is fp32 only"); }
+template <> int launch_nuts_tc128<float>(const QbTg8Plan& tg, const ChainArgs<float>& c, const NutsArgs<float>& a, long long K, cudaStream_t st) {
+    QB_CUDA(qb_tg8_launch_nuts(tg, c, a, K, st));
+    return 0;
+}
+template <typename T> static int launch_nuts_tc(const QbTcgPlan&, const ChainArgs<T>&, const NutsArgs<T>&, long long, cudaStream_t) { return qb_fail("tensor-core path is fp32 only"); }
+template <> int launch_nuts_tc<float>(const QbTcgPlan& tg, const ChainArgs<float>& c, const NutsArgs<float>& a, long long K, cudaStream_t st) {
+    QB_CUDA(qb_tcg_launch_nuts(tg, c, a, K, st));
     return 0;
 }
 
@@ -798,6 +809,24 @@ __global__ void __launch_bounds__(QS_THREADS, 1) k_hmc_stream(const __grid_const
     qb_hmc_body<T>(c, h, P.n_params, reinterpret_cast<double*>(smem_raw), eval);
 }
 
+// NUTS (qb_nuts.cuh) on the same evaluation functors as k_hmc / k_hmc_stream
+template <typename T>
+__global__ void __launch_bounds__(256, 1) k_nuts(const __grid_constant__ QbPlan plan, const ChainArgs<T> c, const NutsArgs<T> a) {
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    const QbSmem S = qb_carve<T>(plan, smem_raw);
+    QbGradSimt<T> eval{plan, S, c, (long long)blockIdx.x};
+    qb_nuts_body<T>(c, a, plan.n_params, S.red, eval);
+}
+
+template <typename T>
+__global__ void __launch_bounds__(QS_THREADS, 1) k_nuts_stream(const __grid_constant__ QbStreamPlan P, const ChainArgs<T> c, const NutsArgs<T> a) {
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    QsRing rg;
+    qs_ring_init(P, smem_raw, rg);
+    QbGradStream<T> eval{P, smem_raw, rg, c, (long long)blockIdx.x};
+    qb_nuts_body<T>(c, a, P.n_params, reinterpret_cast<double*>(smem_raw), eval);
+}
+
 template <typename T>
 static void fill_chain_args(ChainArgs<T>& c, const qb_data_t* data, const qb_lik_t* lik, const qb_chain_t* ch,
                             const qb_rng_t* rng, const qb_record_t* rec, int64_t t_start, int64_t nsteps, int init_lp) {
@@ -903,6 +932,70 @@ extern "C" int qb_hmc_run(const qb_net_t* net, int dtype, const qb_data_t* data,
     if (check_chain_common(data, lik, chain, rng) || !hm) return g_err[0] ? -1 : qb_fail("NULL hmc state");
     if (dtype == QB_F64) return run_hmc<double>(net, dtype, data, lik, chain, hm, rng, rec, t_start, nsteps, init_lp, (cudaStream_t)stream);
     return run_hmc<float>(net, dtype, data, lik, chain, hm, rng, rec, t_start, nsteps, init_lp, (cudaStream_t)stream);
+}
+
+template <typename T>
+static void fill_nuts_args(NutsArgs<T>& a, double epsilon, int max_depth, int64_t n_adapt, double target_accept, double* log_eps,
+                           double* log_eps_bar, double* h_bar, void* grad_cur, void* scratch, int32_t* rec_depth,
+                           int32_t* rec_n_leapfrog, uint8_t* rec_diverging, double* rec_step_size) {
+    a.eps0 = epsilon; a.target = target_accept; a.max_depth = max_depth; a.n_adapt = n_adapt;
+    a.log_eps = log_eps; a.log_eps_bar = log_eps_bar; a.h_bar = h_bar;
+    a.gcur = (T*)grad_cur; a.scratch = (T*)scratch;
+    a.rec_depth = rec_depth; a.rec_nleap = rec_n_leapfrog; a.rec_div = rec_diverging; a.rec_eps = rec_step_size;
+}
+
+template <typename T>
+static int run_nuts(const qb_net_t* net, int dtype, const qb_data_t* data, const qb_lik_t* lik, qb_chain_t* ch,
+                    const qb_rng_t* rng, const qb_record_t* rec, int64_t t_start, int64_t nsteps, int init_lp,
+                    const NutsArgs<T>& a, cudaStream_t st) {
+    QbLaunch L;
+    if (plan_eval(net, dtype, true, ch->K, data->n, true, &L)) return -1;
+    ChainArgs<T> c; fill_chain_args<T>(c, data, lik, ch, rng, rec, t_start, nsteps, init_lp);
+    if (L.path == QB_PATH_STREAM) {
+        if (set_smem(k_nuts_stream<T>, L.sp.smem_bytes)) return -2;
+        k_nuts_stream<T><<<(unsigned)ch->K, QS_THREADS, L.sp.smem_bytes, st>>>(L.sp, c, a);
+    } else if (L.path == QB_PATH_TG8) {
+        if (launch_nuts_tc128<T>(L.t8, c, a, ch->K, st)) return -2;
+        g_launches += 1;
+    } else if (L.path == QB_PATH_TCG) {
+        if (launch_nuts_tc<T>(L.tg, c, a, ch->K, st)) return -2;
+    } else {
+        if (set_smem(k_nuts<T>, L.plan.smem_bytes)) return -2;
+        k_nuts<T><<<(unsigned)ch->K, L.plan.nthreads, L.plan.smem_bytes, st>>>(L.plan, c, a);
+    }
+    QB_CUDA(cudaGetLastError());
+    g_launches += 1;
+    return 0;
+}
+
+extern "C" int qb_nuts_run(const qb_net_t* net, int dtype, const qb_data_t* data, const qb_lik_t* lik,
+                           qb_chain_t* chain, const qb_rng_t* rng, const qb_record_t* rec, int64_t t_start,
+                           int64_t nsteps, int init_lp, double epsilon, int max_depth, int64_t n_adapt,
+                           double target_accept, double* log_eps, double* log_eps_bar, double* h_bar, void* grad_cur,
+                           void* scratch, int32_t* rec_depth, int32_t* rec_n_leapfrog, uint8_t* rec_diverging,
+                           double* rec_step_size, void* stream) {
+    if (!net || !data || !lik || !chain || !rng) return qb_fail("NULL argument to chain run");
+    if (rng->mode == QB_RNG_REPLAY) return qb_fail("NUTS has no replay mode: its draws come from Philox");
+    if (!(epsilon > 0.0 && epsilon < INFINITY)) return qb_fail("NUTS needs a finite epsilon > 0");
+    if (max_depth < 1 || max_depth > QB_NUTS_MAX_DEPTH)
+        return qb_fail("NUTS needs 1 <= max_depth <= 12%s (max_depth=%lld)", "", max_depth);
+    if (!(target_accept > 0.0 && target_accept < 1.0)) return qb_fail("NUTS needs 0 < target_accept < 1");
+    if (n_adapt < 0 || nsteps < 0 || t_start < 0) return qb_fail("n_adapt, nsteps and t_start must be >= 0");
+    if (!log_eps || !log_eps_bar || !h_bar || !grad_cur || !scratch) return qb_fail("NUTS state has NULL arrays");
+    if (!rec && (rec_depth || rec_n_leapfrog || rec_diverging || rec_step_size))
+        return qb_fail("NUTS records need rec: they share its leading dimension");
+    if (chain->K == 0 || nsteps == 0) return 0;
+    if (check_chain_common(data, lik, chain, rng)) return -1;
+    if (dtype == QB_F64) {
+        NutsArgs<double> a;
+        fill_nuts_args<double>(a, epsilon, max_depth, n_adapt, target_accept, log_eps, log_eps_bar, h_bar, grad_cur, scratch,
+                               rec_depth, rec_n_leapfrog, rec_diverging, rec_step_size);
+        return run_nuts<double>(net, dtype, data, lik, chain, rng, rec, t_start, nsteps, init_lp, a, (cudaStream_t)stream);
+    }
+    NutsArgs<float> a;
+    fill_nuts_args<float>(a, epsilon, max_depth, n_adapt, target_accept, log_eps, log_eps_bar, h_bar, grad_cur, scratch,
+                          rec_depth, rec_n_leapfrog, rec_diverging, rec_step_size);
+    return run_nuts<float>(net, dtype, data, lik, chain, rng, rec, t_start, nsteps, init_lp, a, (cudaStream_t)stream);
 }
 
 // =================================================================================================

@@ -2,3 +2,4 @@ from .mcmc import MCMCBase, DeviceLogPost
 from .admcmc import AMCMC
 from .hmc import HMC
 from .mala import MALA
+from .nuts import NUTS

@@ -479,6 +479,82 @@ def hmc_run(state: ChainState, hm: HmcState, nsteps, rec: Recorder = None, seed=
     state.initialised = True
 
 
+NUTS_MAX_DEPTH = 12          # compile-time cap of qb_nuts_run
+
+
+class NutsState:
+    """NUTS settings and device state of K chains: the per-chain dual-averaging state (log eps, log eps_bar, H_bar), the
+    gradient at the current state and the tree scratch of (9 + 2 max_depth) P elements per chain (qb_nuts_run)."""
+
+    def __init__(self, state: ChainState, epsilon=0.05, max_depth=10, n_adapt=1000, target_accept=0.8):
+        if not 1 <= int(max_depth) <= NUTS_MAX_DEPTH:
+            raise ValueError(f'max_depth must lie in [1, {NUTS_MAX_DEPTH}]')
+        if not 0.0 < float(target_accept) < 1.0:
+            raise ValueError('target_accept must lie in (0, 1)')
+        if not (float(epsilon) > 0.0 and np.isfinite(float(epsilon))):
+            raise ValueError('epsilon must be finite and > 0')
+        if int(n_adapt) < 0:
+            raise ValueError('n_adapt must be >= 0')
+        self.epsilon, self.max_depth = float(epsilon), int(max_depth)
+        self.n_adapt, self.target_accept = int(n_adapt), float(target_accept)
+        K, dev = state.K, state.prob.device
+        self.log_eps = torch.full((K,), float(np.log(self.epsilon)), dtype=torch.float64, device=dev)
+        self.log_eps_bar = self.log_eps.clone()
+        self.h_bar = torch.zeros(K, dtype=torch.float64, device=dev)
+        self.grad_cur = torch.zeros_like(state.theta)
+        self.scratch = torch.empty((K, (9 + 2 * self.max_depth) * state.P), dtype=state.theta.dtype, device=dev)
+
+    _FIELDS = ('log_eps', 'log_eps_bar', 'h_bar', 'grad_cur')
+
+    def state_dict(self):
+        return {k: getattr(self, k).detach().cpu().clone() for k in self._FIELDS}
+
+    def load_state_dict(self, d):
+        for k in self._FIELDS:
+            getattr(self, k).copy_(d[k])
+
+    def step_size(self, t):
+        """[K] step sizes transition t uses (float64, on the device)."""
+        return torch.exp(self.log_eps_bar if (self.n_adapt > 0 and t >= self.n_adapt) else self.log_eps)
+
+
+class NutsRecords:
+    """Per-transition NUTS records of one run segment: tree depth, leapfrog count (int32), divergence flag (uint8) and
+    step size (float64), [K, nsteps] each."""
+
+    def __init__(self, state: ChainState, nsteps):
+        K, dev = state.K, state.prob.device
+        self.tree_depth = torch.empty((K, nsteps), dtype=torch.int32, device=dev)
+        self.n_leapfrog = torch.empty((K, nsteps), dtype=torch.int32, device=dev)
+        self.diverging = torch.empty((K, nsteps), dtype=torch.uint8, device=dev)
+        self.step_size = torch.empty((K, nsteps), dtype=torch.float64, device=dev)
+
+
+def nuts_run(state: ChainState, ns: NutsState, nsteps, rec: Recorder = None, nrec: NutsRecords = None, seed=0,
+             chain_offset=0):
+    """qb_nuts_run: advance all chains by nsteps NUTS transitions (Philox draws; there is no replay mode).  nrec needs rec
+    (the records share its leading dimension)."""
+    if nrec is not None and rec is None:
+        raise ValueError('NUTS records need a Recorder')
+    if nsteps == 0:
+        return
+    prob = state.prob
+    rng = _rng_struct(seed, chain_offset, None, None)
+    cch = state.c()
+    crec = rec.c() if rec is not None else None
+    nr = [None] * 4 if nrec is None else [_ptr(nrec.tree_depth), _ptr(nrec.n_leapfrog), _ptr(nrec.diverging),
+                                           _ptr(nrec.step_size)]
+    with torch.cuda.device(prob.device):
+        rc = _lib.load().qb_nuts_run(C.byref(prob.cnet), prob.qdt, C.byref(prob.cdata), C.byref(prob.clik), C.byref(cch),
+                                     C.byref(rng), C.byref(crec) if crec is not None else None, state.t, nsteps,
+                                     0 if state.initialised else 1, ns.epsilon, ns.max_depth, ns.n_adapt,
+                                     ns.target_accept, _ptr(ns.log_eps), _ptr(ns.log_eps_bar), _ptr(ns.h_bar),
+                                     _ptr(ns.grad_cur), _ptr(ns.scratch), *nr, _stream())
+    _lib.check(rc, 'qb_nuts_run')
+    state.t += nsteps
+    state.initialised = True
+
+
 def vi_sample(mu, rho, nsam, pi, sigma1, sigma2, eps=None, seed=0, step=0):
     """w[nsam,P] = mu + exp(rho)*eps, log q[nsam], log prior[nsam] (bnet.py:142-166)."""
     _need_cuda(mu, rho)

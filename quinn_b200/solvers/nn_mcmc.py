@@ -12,6 +12,7 @@ from .. import ops
 from ..mcmc.admcmc import AMCMC
 from ..mcmc.hmc import HMC
 from ..mcmc.mala import MALA
+from ..mcmc.nuts import NUTS
 from ..mcmc.mcmc import DeviceLogPost
 from ..netdesc import netdesc_from_module
 from ..nns.nnwrap import NNWrap, nn_p
@@ -73,6 +74,10 @@ class NN_MCMC(QUiNNBase):
             distributed=False, diag_every=None, gather=True, data_sharded=False, keep_on_device=False):
         """Sample the posterior of the flat parameters (nn_mcmc.py:100-139).
 
+        ``sampler='nuts'`` runs the No-U-Turn sampler (quinn_b200.mcmc.NUTS, sampler_params: epsilon, max_depth, n_adapt,
+        target_accept) in this process; its result dict adds ``tree_depth``, ``n_leapfrog``, ``diverging`` and
+        ``step_size`` per transition.
+
         Extensions (keyword-only): ``nchains`` / a (K,P) ``param_ini`` run K chains at once (``samples``
         becomes (K, M+1, P)); ``seed``, ``store_every``, ``replay``, ``chain_offset`` are passed to the sampler.
         With ``zflag`` the start point is refined by BFGS on -logpost using the analytic gradient of kernel 2
@@ -89,6 +94,9 @@ class NN_MCMC(QUiNNBase):
         (and gradient) is the all-reduced sum of the per-rank partial sums (the N-sharded mode for data that exceed one
         GPU; propose / accept run redundantly and identically on every rank)."""
         assert xtrn.shape[0] == ytrn.shape[0]
+        if sampler == 'nuts' and (data_sharded or distributed):
+            raise ValueError("sampler='nuts' runs in a single process: distributed=True and data_sharded=True are not "
+                             "supported with it")
         if data_sharded:
             return self._fit_data_sharded(xtrn, ytrn, datanoise, nmcmc, param_ini, sampler, sampler_params, nchains, seed,
                                           store_every)
@@ -112,8 +120,11 @@ class NN_MCMC(QUiNNBase):
         elif sampler == 'mala':                     # promised by the docstring at nn_mcmc.py:110
             mymcmc = MALA(**sampler_params)
             mymcmc.setLogPost(self.logpost, self.logpostgrad, lpinfo=self.lpinfo)
+        elif sampler == 'nuts':
+            mymcmc = NUTS(**sampler_params)
+            mymcmc.setLogPost(self.logpost, self.logpostgrad, lpinfo=self.lpinfo)
         else:
-            raise ValueError(f"sampler {sampler!r} is not one of 'amcmc', 'hmc', 'mala'")
+            raise ValueError(f"sampler {sampler!r} is not one of 'amcmc', 'hmc', 'mala', 'nuts'")
         res = mymcmc.run(param_ini=param_ini, nmcmc=nmcmc, seed=seed, store_every=store_every, replay=replay,
                          chain_offset=chain_offset, verbose=self.verbose, keep_on_device=keep_on_device)
         self.sampler_obj, self.mcmc_results = mymcmc, res
