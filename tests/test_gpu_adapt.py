@@ -4,7 +4,7 @@
   counter-based streams restated in numpy, pinned to the Random123 known-answer vectors) and the oracle's run_chain, both
   for the diagonal adaptation (the repo's scalable deviation, DESIGN.md section 5) and for the initial rank-1 + diagonal
   proposal; chain, decisions, running mean / covariance and proposal scales must agree.
-* fp32 tensor-core kernels k_amcmc<float,1> (config-5 shape) and k_amcmc<float,2> (other eligible shapes): replay mode
+* fp32 tensor-core kernels k_amcmc_tc3 (config-5 shape) and k_amcmc<float,2> (other eligible shapes): replay mode
   across adaptation points against the oracle recursion, and Philox mode against the CUDA-core kernel run from the same
   seed (identical proposals => identical chains up to fp32-noise ties), which exercises the kind == 1 proposal branch.
 * the in-kernel Cholesky survives a rank-deficient covariance (first adaptation with fewer samples than parameters).
@@ -67,7 +67,7 @@ def test_amcmc_diag_adaptation_fp64_replayed_with_numpy_philox(seed, chain_offse
 
 @pytest.mark.parametrize('widths,tc_kind', [([3, 64, 64, 1], 'hot'), ([2, 32, 32, 1], 'general')])
 def test_tc_amcmc_replay_across_adaptation_points(widths, tc_kind):
-    """k_amcmc<float,1> / <float,2> with adapt='diag' in replay mode, 70 steps with t0=10, tadapt=20: decisions, chain and
+    """k_amcmc_tc3 / k_amcmc<float,2> with adapt='diag' in replay mode, 70 steps with t0=10, tadapt=20: decisions, chain and
     the adapted proposal scales against the oracle recursion."""
     from quinn_b200 import ops
     rs, layers, P, x, y, prob = _problem(widths, 300, 7, torch.float32)
@@ -107,8 +107,8 @@ def test_tc_amcmc_replay_across_adaptation_points(widths, tc_kind):
 
 @pytest.mark.parametrize('widths', [[3, 64, 64, 1], [2, 32, 32, 1]])
 def test_tc_amcmc_philox_adapted_proposals_equal_the_cuda_core_kernel(widths):
-    """Philox mode across adaptation points: the tensor-core kernel (kind == 1 branch of qb_amcmc_pre inside
-    k_amcmc<float,1|2>) and the CUDA-core kernel draw the same proposals, so states agree wherever decisions agree."""
+    """Philox mode across adaptation points: the tensor-core kernels (kind == 1 branch of the proposal in k_amcmc_tc3
+    and of qb_amcmc_pre in k_amcmc<float,2>) and the CUDA-core kernel draw the same proposals, so states agree wherever decisions agree."""
     from quinn_b200 import ops
     rs, layers, P, x, y, prob = _problem(widths, 400, 9, torch.float32, sigma=0.5)
     K, steps = 48, 70
