@@ -849,68 +849,128 @@ __device__ __forceinline__ void qb_bwd_gemm(const QbLayerPlan& L, const QbLayerP
     else qb_bwd_gemm_a<T, GLOBALW, TP, QB_ACT_IDENTITY>(L, Lm, sW, theta, R, D, lda, TM);
 }
 
-// value + gradient of the data term for one parameter vector over points [n0, n1):
-// returns sum of squared residuals; g[0..P) receives d/dtheta of  -0.5*ssq/sigma^2  (i.e. of lp's data term).
-// g must be addressable by this block only (one row per (chain, split)).
+// The tile of qb_backprop_tiles as its hooks see it: activation rows R (leading dimension lda) of TM points from p0 on,
+// the first `valid` of them below n1, o outputs from the top layer Ltop, and the pass over the tile.
+template <typename T>
+struct QbTile {
+    T* R;
+    const QbLayerPlan& Ltop;
+    int lda, TM, o;
+    int64_t p0;
+    int valid, pass;
+    // output j at tile point p
+    __device__ __forceinline__ T& top(int j, int p) const { return R[(size_t)(Ltop.row_out + j) * lda + p]; }
+};
+
+// The back-propagation tile loop of kernels 2, 6 and 7, for one parameter vector over points [n0, n1): stage the
+// weights, then per tile run the forward pass, set the top delta and walk the layers top-down.  At layer l's dW point
+// its input rows a_in are intact and delta_z has been written in place over its output rows; the backward GEMM then
+// overwrites layer l-1's output rows with its delta_z, so every activation above the input is gone after a pass.
+// What differs between the kernels is in the hooks H (all __forceinline__):
+//   zero()                          clears the block's output row before the first tile
+//   passes(o)                       forward + backward passes per tile
+//   after_forward(t)                after each forward pass; a hook that writes the tile adds its own barrier
+//   top_delta(t, j, p, ssq)         delta of output j at tile point p; also called for the padded points of a partial
+//                                   tile (p >= t.valid)
+//   at_dw(t, l)                     layer l's dW point
+//   sums_squares                    the loop returns the block sum of ssq (otherwise 0)
 // TPG = points per thread tile in the gradient kernel: 4 (twice the threads per tile, for layers >= 64 wide) or 8
-template <typename T, int TPG>
-__device__ double qb_eval_value_grad_t(const QbPlan& P, const QbSmem& S, const T* theta, const T* __restrict__ x,
-                                     const T* __restrict__ y, int64_t n0, int64_t n1, double inv_sigma2, T* g) {
+template <typename T, int TPG, typename H>
+__device__ double qb_backprop_tiles_t(const QbPlan& P, const QbSmem& S, const T* theta, const T* __restrict__ x,
+                                      int64_t n0, int64_t n1, H& h) {
     T* sW = reinterpret_cast<T*>(S.w);
     T* R = reinterpret_cast<T*>(S.act);
     const int lda = P.lda, TM = P.TM, o = P.out_dim, nl = P.n_layers;
     T* D = P.d_row >= 0 ? R + (size_t)P.d_row * lda : nullptr;
     __syncthreads();
     qb_stage_weights<T>(P, sW, theta);
-    for (int idx = threadIdx.x; idx < P.n_params; idx += blockDim.x) g[idx] = T(0);
+    h.zero();
     __syncthreads();
     T ssq = T(0);
-    const T is2 = T(inv_sigma2);
     const QbLayerPlan& Ltop = P.L[nl - 1];
     const QbScope bsc = qb_block_scope(TM);
     for (int64_t p0 = n0; p0 < n1; p0 += TM) {
+        const int valid = (int)min((int64_t)TM, n1 - p0);
         qb_load_x_tile<T>(x, P.in_dim, p0, n1, R, lda, bsc);
         __syncthreads();
-        for (int l = 0; l < nl; ++l) {
-            const QbLayerPlan& L = P.L[l];
-            qb_layer_forward<T, TPG>(L, sW, R + (size_t)L.row_in * lda, R + (size_t)L.row_out * lda, lda, bsc, false);
-        }
-        // residuals -> delta at the top
-        const int n = TM * o;
-        for (int idx = threadIdx.x; idx < n; idx += blockDim.x) {
-            const int j = idx / TM, p = idx - j * TM;
-            const int64_t gp = p0 + p;
-            T da = T(0);
-            if (gp < n1) {
-                T out = R[(size_t)(Ltop.row_out + j) * lda + p];
-                if (P.final_exp) out = qb_exp(out);
-                const T r = __ldg(y + gp * o + j) - out;
-                ssq = fma(r, r, ssq);
-                da = r * is2;
-                if (P.final_exp) da *= out;
+        for (int pass = 0; pass < h.passes(o); ++pass) {
+            const QbTile<T> t{R, Ltop, lda, TM, o, p0, valid, pass};
+            for (int l = 0; l < nl; ++l) {
+                const QbLayerPlan& L = P.L[l];
+                qb_layer_forward<T, TPG>(L, sW, R + (size_t)L.row_in * lda, R + (size_t)L.row_out * lda, lda, bsc, false);
             }
-            qb_finish_delta<T>(Ltop, R, D, lda, j, p, da);
-        }
-        __syncthreads();
-        for (int l = nl - 1; l >= 0; --l) {
-            const QbLayerPlan& L = P.L[l];
-            qb_dw_accumulate<T>(L, R, lda, TM, g);
+            h.after_forward(t);
+            const int n = TM * o;
+            for (int idx = threadIdx.x; idx < n; idx += blockDim.x) {
+                const int j = idx / TM, p = idx - j * TM;
+                const T da = h.top_delta(t, j, p, ssq);
+                qb_finish_delta<T>(Ltop, R, D, lda, j, p, da);
+            }
             __syncthreads();
-            if (l > 0) {
-                if (L.wr_off >= 0) qb_bwd_gemm<T, false, TPG>(L, P.L[l - 1], sW, theta, R, D, lda, TM);
-                else qb_bwd_gemm<T, true, TPG>(L, P.L[l - 1], sW, theta, R, D, lda, TM);
+            for (int l = nl - 1; l >= 0; --l) {
+                const QbLayerPlan& L = P.L[l];
+                h.at_dw(t, l);
                 __syncthreads();
+                if (l > 0) {
+                    if (L.wr_off >= 0) qb_bwd_gemm<T, false, TPG>(L, P.L[l - 1], sW, theta, R, D, lda, TM);
+                    else qb_bwd_gemm<T, true, TPG>(L, P.L[l - 1], sW, theta, R, D, lda, TM);
+                    __syncthreads();
+                }
             }
         }
     }
-    return qb_block_sum((double)ssq, S.red);
+    if (H::sums_squares) return qb_block_sum((double)ssq, S.red);
+    return 0.0;
 }
 
+template <typename T, typename H>
+__device__ double qb_backprop_tiles(const QbPlan& P, const QbSmem& S, const T* theta, const T* __restrict__ x,
+                                    int64_t n0, int64_t n1, H& h) {
+    if (sizeof(T) == 4 && P.tpg == 8) return qb_backprop_tiles_t<T, VT<T>::TP>(P, S, theta, x, n0, n1, h);
+    return qb_backprop_tiles_t<T, 4>(P, S, theta, x, n0, n1, h);
+}
+
+// kernel 2's hooks: g[0..n_params) receives d/dtheta of -0.5*ssq/sigma^2; delta at the top is r / sigma^2 (final_exp:
+// times e^u) and zero at padded points
+template <typename T>
+struct QbGradHooks {
+    static constexpr bool sums_squares = true;
+    const QbPlan& P;
+    const T* __restrict__ y;
+    int64_t n1;
+    double inv_sigma2;
+    T* g;
+    __device__ __forceinline__ void zero() const {
+        for (int idx = threadIdx.x; idx < P.n_params; idx += blockDim.x) g[idx] = T(0);
+    }
+    __device__ __forceinline__ int passes(int) const { return 1; }
+    __device__ __forceinline__ void after_forward(const QbTile<T>&) const {}
+    __device__ __forceinline__ T top_delta(const QbTile<T>& t, int j, int p, T& ssq) const {
+        const int64_t gp = t.p0 + p;
+        T da = T(0);
+        if (gp < n1) {
+            T out = t.top(j, p);
+            if (P.final_exp) out = qb_exp(out);
+            const T r = __ldg(y + gp * t.o + j) - out;
+            ssq = fma(r, r, ssq);
+            da = r * T(inv_sigma2);
+            if (P.final_exp) da *= out;
+        }
+        return da;
+    }
+    __device__ __forceinline__ void at_dw(const QbTile<T>& t, int l) const {
+        qb_dw_accumulate<T>(P.L[l], t.R, t.lda, t.TM, g);
+    }
+};
+
+// value + gradient of the data term for one parameter vector over points [n0, n1):
+// returns sum of squared residuals; g[0..P) receives d/dtheta of  -0.5*ssq/sigma^2  (i.e. of lp's data term).
+// g must be addressable by this block only (one row per (chain, split)).
 template <typename T>
 __device__ double qb_eval_value_grad(const QbPlan& P, const QbSmem& S, const T* theta, const T* __restrict__ x,
                                      const T* __restrict__ y, int64_t n0, int64_t n1, double inv_sigma2, T* g) {
-    if (sizeof(T) == 4 && P.tpg == 8) return qb_eval_value_grad_t<T, VT<T>::TP>(P, S, theta, x, y, n0, n1, inv_sigma2, g);
-    return qb_eval_value_grad_t<T, 4>(P, S, theta, x, y, n0, n1, inv_sigma2, g);
+    QbGradHooks<T> h{P, y, n1, inv_sigma2, g};
+    return qb_backprop_tiles<T>(P, S, theta, x, n0, n1, h);
 }
 
 // --------------------------------------------------------------------------------------------

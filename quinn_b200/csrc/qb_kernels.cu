@@ -379,14 +379,15 @@ template <typename T> struct KfacArgs {
     double inv_sigma2;
 };
 
-// fp32: one block per SM in the register budget (157 registers; at two, 128 registers spill the fp32 factor passes)
+// fp32: one block per SM in the register budget (163 registers; at two, 128 registers spill the fp32 factor passes)
 template <typename T>
 __global__ void __launch_bounds__(256, sizeof(T) == 8 ? 2 : 1) k_logpost_kfac(const __grid_constant__ QbKfacPlan K, const KfacArgs<T> a) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     const QbSmem S = qb_carve<T>(K.P, smem_raw);
     const long long s = blockIdx.x;
     const long long n0 = s * a.pps, n1 = min(a.N, n0 + a.pps);
-    qb_kfac_eval<T>(K, S, a.theta, a.x, a.y, n0, n1, a.inv_sigma2, a.part + s * K.n_factors);
+    QbKfacHooks<T> h{{K.P, a.y, n1, a.inv_sigma2, a.part + s * K.n_factors}, K};
+    qb_backprop_tiles<T>(K.P, S, a.theta, a.x, n0, n1, h);
 }
 
 // factors[e] = sum of the N-split rows in fixed order, in double
@@ -448,7 +449,8 @@ __global__ void __launch_bounds__(256, 2) k_predict_jac(const __grid_constant__ 
     const QbSmem S = qb_carve<T>(J.P, smem_raw);
     const long long s = blockIdx.x;
     const long long n0 = s * a.pps, n1 = min(a.N, n0 + a.pps);
-    qb_jac_eval<T>(J, S, a.theta, a.x, a.N, n0, n1, a.out, a.fac);
+    QbJacHooks<T> h{J, a.N, a.out, a.fac};
+    qb_backprop_tiles<T>(J.P, S, a.theta, a.x, n0, n1, h);
 }
 
 template <typename T>

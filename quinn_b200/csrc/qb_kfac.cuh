@@ -1,5 +1,5 @@
-// Kernel 6: Kronecker factors of the per-point empirical Fisher of every Linear layer, accumulated through kernel 2's
-// resident body.  sm_100a, CUDA cores (FFMA2 in fp32, DFMA in fp64).
+// Kernel 6: Kronecker factors of the per-point empirical Fisher of every Linear layer, accumulated in kernel 2's
+// back-propagation tile loop (qb_backprop_tiles) with the hooks below.  sm_100a, CUDA cores (FFMA2 in fp32, DFMA in fp64).
 //
 // For layer l with input activations a_i and pre-activation gradients delta_i = d log p_i / d z_l of point i:
 //   A_l = sum_i a_i a_i^T [n_in, n_in],   s_l = sum_i a_i [n_in] (layers with a bias),   G_l = sum_i delta_i delta_i^T
@@ -22,70 +22,32 @@ struct QbKfacPlan {
     int pad_;
 };
 
-// Factors of the points [n0, n1) added to g[0..n_factors) (zeroed first).  g must be addressable by this block only.
-template <typename T, int TPG>
-__device__ void qb_kfac_eval_t(const QbKfacPlan& K, const QbSmem& S, const T* theta, const T* __restrict__ x,
-                               const T* __restrict__ y, int64_t n0, int64_t n1, double inv_sigma2, T* g) {
-    const QbPlan& P = K.P;
-    T* sW = reinterpret_cast<T*>(S.w);
-    T* R = reinterpret_cast<T*>(S.act);
-    const int lda = P.lda, TM = P.TM, o = P.out_dim, nl = P.n_layers;
-    T* D = P.d_row >= 0 ? R + (size_t)P.d_row * lda : nullptr;
-    __syncthreads();
-    qb_stage_weights<T>(P, sW, theta);
-    for (int idx = threadIdx.x; idx < K.n_factors; idx += blockDim.x) g[idx] = T(0);
-    __syncthreads();
-    const T is2 = T(inv_sigma2);
-    const QbLayerPlan& Ltop = P.L[nl - 1];
-    const QbScope bsc = qb_block_scope(TM);
-    for (int64_t p0 = n0; p0 < n1; p0 += TM) {
-        qb_load_x_tile<T>(x, P.in_dim, p0, n1, R, lda, bsc);
-        __syncthreads();
-        for (int l = 0; l < nl; ++l) {
-            const QbLayerPlan& L = P.L[l];
-            qb_layer_forward<T, TPG>(L, sW, R + (size_t)L.row_in * lda, R + (size_t)L.row_out * lda, lda, bsc, false);
-        }
-        const int valid = (int)min((int64_t)TM, n1 - p0);
-        if (valid < TM) {
+// Kernel 2's top delta (its sum of squares is not returned); the factor row g[0..n_factors) is zeroed first, padded
+// activation columns are zeroed after each forward pass, and layer l's dW point accumulates its factors.
+// Inherited from QbGradHooks on purpose: top_delta and passes (one pass per tile).  Every other hook is defined here,
+// so a hook added to QbGradHooks must be checked for kernel 6 as well.
+template <typename T>
+struct QbKfacHooks : QbGradHooks<T> {
+    static constexpr bool sums_squares = false;
+    const QbKfacPlan& K;
+    __device__ __forceinline__ void zero() const {
+        for (int idx = threadIdx.x; idx < K.n_factors; idx += blockDim.x) this->g[idx] = T(0);
+    }
+    __device__ __forceinline__ void after_forward(const QbTile<T>& t) const {
+        // the value of t.valid, formed again here: reading t.valid instead costs the fp64 kernel 8 SASS instructions
+        const int valid = (int)min((int64_t)t.TM, this->n1 - t.p0);
+        if (valid < t.TM) {
             // padded points: every activation column zero (their delta is zero; their activations would enter A and s)
-            const int w = TM - valid;
-            for (int idx = threadIdx.x; idx < P.total_rows * w; idx += blockDim.x) {
+            const int w = t.TM - valid;
+            for (int idx = threadIdx.x; idx < K.P.total_rows * w; idx += blockDim.x) {
                 const int r = idx / w, p = valid + (idx - r * w);
-                R[(size_t)r * lda + p] = T(0);
+                t.R[(size_t)r * t.lda + p] = T(0);
             }
             __syncthreads();
-        }
-        // delta at the top: d lp_i / d out = r / sigma^2 (final_exp: times e^u), as in kernel 2
-        for (int idx = threadIdx.x; idx < TM * o; idx += blockDim.x) {
-            const int j = idx / TM, p = idx - j * TM;
-            const int64_t gp = p0 + p;
-            T da = T(0);
-            if (gp < n1) {
-                T out = R[(size_t)(Ltop.row_out + j) * lda + p];
-                if (P.final_exp) out = qb_exp(out);
-                da = (__ldg(y + gp * o + j) - out) * is2;
-                if (P.final_exp) da *= out;
-            }
-            qb_finish_delta<T>(Ltop, R, D, lda, j, p, da);
-        }
-        __syncthreads();
-        for (int l = nl - 1; l >= 0; --l) {
-            const QbLayerPlan& L = P.L[l];
-            qb_dw_accumulate<T>(K.LA[l], R, lda, TM, g);
-            qb_dw_accumulate<T>(K.LG[l], R, lda, TM, g);
-            __syncthreads();
-            if (l > 0) {
-                if (L.wr_off >= 0) qb_bwd_gemm<T, false, TPG>(L, P.L[l - 1], sW, theta, R, D, lda, TM);
-                else qb_bwd_gemm<T, true, TPG>(L, P.L[l - 1], sW, theta, R, D, lda, TM);
-                __syncthreads();
-            }
         }
     }
-}
-
-template <typename T>
-__device__ void qb_kfac_eval(const QbKfacPlan& K, const QbSmem& S, const T* theta, const T* __restrict__ x,
-                             const T* __restrict__ y, int64_t n0, int64_t n1, double inv_sigma2, T* g) {
-    if (sizeof(T) == 4 && K.P.tpg == 8) qb_kfac_eval_t<T, VT<T>::TP>(K, S, theta, x, y, n0, n1, inv_sigma2, g);
-    else qb_kfac_eval_t<T, 4>(K, S, theta, x, y, n0, n1, inv_sigma2, g);
-}
+    __device__ __forceinline__ void at_dw(const QbTile<T>& t, int l) const {
+        qb_dw_accumulate<T>(K.LA[l], t.R, t.lda, t.TM, this->g);
+        qb_dw_accumulate<T>(K.LG[l], t.R, t.lda, t.TM, this->g);
+    }
+};

@@ -613,6 +613,16 @@ extern "C" int qb_hvp_plan_info(const qb_net_t* net, int dtype, int64_t K, int64
     return 0;
 }
 
+// Kernels 6 and 7 run kernel 2's tile loop: kernel 2's resident CUDA-core plan for one theta, or `streamed_error` for a
+// net that kernel 2 evaluates layer-streamed.  The caller has checked the arguments.
+static int make_resident_plan(const qb_net_t* net, int dtype, long long N, const char* streamed_error, QbPlan* out) {
+    QbLaunch L;
+    if (make_launch(net, dtype, true, 1, N, true, &L)) return -1;
+    if (L.streamed) return qb_fail("%s", streamed_error);
+    *out = L.plan;
+    return 0;
+}
+
 // =================================================================================================
 // kernel 6: Kronecker factors of the per-point empirical Fisher (qb_kfac.cuh)
 // =================================================================================================
@@ -630,13 +640,11 @@ int make_kfac_launch(const qb_net_t* net, int dtype, long long N, QbKfacLaunch* 
                 return qb_fail("Kronecker factors: layer %s%lld shares its weights with an earlier layer; every layer must "
                                "own its weights", "", l);
     }
-    QbLaunch L;
-    if (make_launch(net, dtype, true, 1, N, true, &L)) return -1;
-    if (L.streamed)
-        return qb_fail("Kronecker factors: the network's weights do not fit in shared memory next to one tile of "
-                       "activations, and the layer-streamed path (plan code 5) has no factor kernel");
     memset(&out->K, 0, sizeof(out->K));
-    out->K.P = L.plan;
+    if (make_resident_plan(net, dtype, N, "Kronecker factors: the network's weights do not fit in shared memory next to "
+                           "one tile of activations, and the layer-streamed path (plan code 5) has no factor kernel",
+                           &out->K.P))
+        return -1;
     const QbPlan& P = out->K.P;
     const QbDt D = dt_of(dtype);
     int off = 0;
@@ -685,13 +693,11 @@ extern "C" int qb_kfac_plan_info(const qb_net_t* net, int dtype, int64_t N, int6
 // whole tiles.  Nothing is reduced over the points, so there are no partial rows to cap.
 int make_jac_launch(const qb_net_t* net, int dtype, long long N, QbJacLaunch* out) {
     if (check_args(net, dtype, 1, N)) return -1;
-    QbLaunch L;
-    if (make_launch(net, dtype, true, 1, N, true, &L)) return -1;
-    if (L.streamed)
-        return qb_fail("output Jacobians: the network's weights do not fit in shared memory next to one tile of "
-                       "activations, and the layer-streamed path (plan code 5) has no Jacobian kernel");
     memset(&out->J, 0, sizeof(out->J));
-    out->J.P = L.plan;
+    if (make_resident_plan(net, dtype, N, "output Jacobians: the network's weights do not fit in shared memory next to "
+                           "one tile of activations, and the layer-streamed path (plan code 5) has no Jacobian kernel",
+                           &out->J.P))
+        return -1;
     const QbPlan& P = out->J.P;
     int row = 0;
     for (int l = 0; l < P.n_layers; ++l) {
