@@ -296,6 +296,35 @@ int qb_nuts_run(const qb_net_t* net, int dtype, const qb_data_t* data, const qb_
                 double* log_eps_bar, double* h_bar, void* grad_cur, void* scratch, int32_t* rec_depth,
                 int32_t* rec_n_leapfrog, uint8_t* rec_diverging, double* rec_step_size, void* stream);
 
+/* Parallel tempering (replica exchange) on HMC / MALA: nsteps steps of K = T * n_groups chains from absolute step
+ * t_start, on the same kernel path qb_hmc_run takes for (net, dtype, K).  Chains are slot-major: chain k = i * n_groups
+ * + g is temperature slot i = k / n_groups of group g and targets exp(beta[i] * lp), lp the log-posterior of kernel 2
+ * (likelihood and prior).  hm->method and hm->L as qb_hmc_run; the step size of slot i is eps[i] (hm->epsilon is not
+ * read).  chain->lp, map_lp and hm->grad_cur hold tempered values (beta * lp, beta * grad); with beta == 1 every product
+ * is exact.
+ *   beta, eps: [T] device double.  They are NOT validated here (reading them would synchronise): the caller guarantees
+ *     beta[0] == 1, beta strictly decreasing and > 0, eps finite and > 0 (quinn_b200/ops.py PtState does).
+ * Swaps: after every absolute step t with (t + 1) % swap_every == 0, deterministic even-odd round r = (t + 1) /
+ * swap_every - 1 pairs slots (i, i + 1) with i = r (mod 2) in every group.  With U = lp / beta (untempered, double) a pair
+ * is accepted when u < exp((beta_i - beta_{i+1}) (U_{i+1} - U_i)) (strict <, NaN rejects), u = word 0 of Philox
+ * (seed, chain_offset + k_i, r, QB_STREAM_PT = 6, 0).  On accept the slots exchange their theta and grad_cur rows; the lp
+ * and gradient that move from slot j to slot i are multiplied by beta_i / beta_j (double, rounded once to dtype).
+ * naccept, map_theta and map_lp stay with their slot.
+ *   replica: [K] int32, which replica (initial row) is in each slot, swapped with the state.
+ *   last_end: [K] int8 by replica, +1 / -1 for the cold / hot end it visited last; round_trips: [n_groups] int64,
+ *     replicas that reached slot T - 1 and then slot 0 again.
+ *   swap_attempts, swap_accepts: [n_groups, T - 1] int64, per group and pair (i, i + 1).
+ * One call cuts the steps into launches at swap boundaries with a swap kernel after each, without host synchronisation.
+ * rec: scalars for all K chains (tempered values) and samples [n_groups, n_slots, P] for the cold rows, at the positions
+ * qb_hmc_run gives for the same call.  Momenta and MH uniforms as qb_hmc_run (Philox keyed by chain_offset + k).
+ * Refused (error text says why): REPLAY rng mode, NULL arrays, n_groups < 1, K not a multiple of n_groups,
+ * swap_every < 1, t_start % swap_every != 0, a store_every such that neither it nor swap_every divides the other.
+ * K == 0 or nsteps == 0 launches nothing. */
+int qb_pt_run(const qb_net_t* net, int dtype, const qb_data_t* data, const qb_lik_t* lik, qb_chain_t* chain, qb_hmc_t* hm,
+              const qb_rng_t* rng, const qb_record_t* rec, int64_t t_start, int64_t nsteps, int init_lp, int64_t n_groups,
+              const double* beta, const double* eps, int64_t swap_every, int32_t* replica, int8_t* last_end,
+              int64_t* round_trips, int64_t* swap_attempts, int64_t* swap_accepts, void* stream);
+
 /* ---- Kernel 4: posterior predictive -----------------------------------------------------------
  * Replaces the M sequential forwards of nn_p (quinn/nns/nnwrap.py:330-347), NN_MCMC.predict_ens
  * (nn_mcmc.py:180-200), NN_Ens.predict_ens (nn_ens.py:85-110), QUiNNBase.predict_ens /

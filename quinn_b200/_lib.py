@@ -102,6 +102,9 @@ SYMBOLS = {
     'qb_nuts_run': (C.c_int, [C.POINTER(qb_net_t), C.c_int, C.POINTER(qb_data_t), C.POINTER(qb_lik_t),
                               C.POINTER(qb_chain_t), C.POINTER(qb_rng_t), C.POINTER(qb_record_t), C.c_int64, C.c_int64,
                               C.c_int, C.c_double, C.c_int, C.c_int64, C.c_double, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
+    'qb_pt_run': (C.c_int, [C.POINTER(qb_net_t), C.c_int, C.POINTER(qb_data_t), C.POINTER(qb_lik_t), C.POINTER(qb_chain_t),
+                            C.POINTER(qb_hmc_t), C.POINTER(qb_rng_t), C.POINTER(qb_record_t), C.c_int64, C.c_int64, C.c_int,
+                            C.c_int64, _P, _P, C.c_int64, _P, _P, _P, _P, _P, _P]),
     'qb_predict': (C.c_int, [C.POINTER(qb_net_t), C.c_int, _P, C.c_int64, _P, C.c_int64, _P, _P, _P, _P]),
     'qb_vi_sample': (C.c_int, [C.c_int, _P, _P, _P, C.c_int64, C.c_int64, C.c_double, C.c_double, C.c_double,
                                C.c_uint64, C.c_uint64, _P, _P, _P, _P]),

@@ -9,6 +9,7 @@
 #include "qb_device.cuh"
 #include "qb_chain.cuh"
 #include "qb_nuts.cuh"
+#include "qb_pt.cuh"
 #include "qb_tc.cuh"
 #include "qb_tcg.cuh"
 #include "qb_grad_tc.h"
@@ -117,6 +118,18 @@ __global__ void __launch_bounds__(H * 8, H == 32 ? 2 : 1) k_nuts_tc(const __grid
     qb_tc_stop(cx.tmem, (uint32_t)tp.tmem_cols);
 }
 
+// parallel-tempering twin of k_hmc_tc (qb_pt.cuh)
+template <int H, int NI, int ACT>
+__global__ void __launch_bounds__(H * 8, H == 32 ? 2 : 1) k_pt_hmc_tc(const __grid_constant__ QbTcgPlan tp, const __grid_constant__ ChainArgs<float> c,
+                                                        const __grid_constant__ HmcArgs<float> h, const __grid_constant__ PtArgs a) {
+    extern __shared__ __align__(1024) unsigned char smem_g[];
+    QbTcgCtx cx;
+    qb_tcg_init(tp, smem_g, cx);
+    QbGradTc<H, NI, ACT> inner{tp, cx, smem_g, c, (long long)blockIdx.x};
+    qb_pt_hmc_body<float>(c, h, a, tp.n_params, reinterpret_cast<double*>(smem_g), inner);
+    qb_tc_stop(cx.tmem, (uint32_t)tp.tmem_cols);
+}
+
 template <int H, int NI, int ACT>
 static cudaError_t launch_eval_t(const QbTcgPlan& tp, const EvalArgs<float>& a, dim3 grid, cudaStream_t st) {
     cudaError_t e = cudaFuncSetAttribute(k_logpost_grad_tc<H, NI, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, tp.smem_bytes);
@@ -140,6 +153,15 @@ static cudaError_t launch_nuts_t(const QbTcgPlan& tp, const ChainArgs<float>& c,
     return cudaGetLastError();
 }
 
+template <int H, int NI, int ACT>
+static cudaError_t launch_pt_t(const QbTcgPlan& tp, const ChainArgs<float>& c, const HmcArgs<float>& h, const PtArgs& a, long long K,
+                               cudaStream_t st) {
+    cudaError_t e = cudaFuncSetAttribute(k_pt_hmc_tc<H, NI, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, tp.smem_bytes);
+    if (e != cudaSuccess) return e;
+    k_pt_hmc_tc<H, NI, ACT><<<(unsigned)K, tp.nthreads, tp.smem_bytes, st>>>(tp, c, h, a);
+    return cudaGetLastError();
+}
+
 #define QB_TCG_DISPATCH(FN, ...)                                                                          \
     do {                                                                                                  \
         const bool tanh_ = tp.act == QB_ACT_TANH;                                                         \
@@ -157,4 +179,8 @@ cudaError_t qb_tcg_launch_hmc(const QbTcgPlan& tp, const ChainArgs<float>& c, co
 }
 cudaError_t qb_tcg_launch_nuts(const QbTcgPlan& tp, const ChainArgs<float>& c, const NutsArgs<float>& a, long long K, cudaStream_t st) {
     QB_TCG_DISPATCH(launch_nuts_t, tp, c, a, K, st);
+}
+cudaError_t qb_tcg_launch_pt(const QbTcgPlan& tp, const ChainArgs<float>& c, const HmcArgs<float>& h, const PtArgs& a, long long K,
+                             cudaStream_t st) {
+    QB_TCG_DISPATCH(launch_pt_t, tp, c, h, a, K, st);
 }

@@ -13,6 +13,7 @@
 #include "qb_device.cuh"
 #include "qb_chain.cuh"
 #include "qb_nuts.cuh"
+#include "qb_pt.cuh"
 #include "qb_tc.cuh"
 #include "qb_tg8.cuh"
 #include "qb_grad_tc128.h"
@@ -134,6 +135,18 @@ __global__ void __launch_bounds__(4 * H + 32, 1) k_nuts_tc128(const __grid_const
     qb_tc_stop(tmem, (uint32_t)tp.tmem_cols);
 }
 
+// parallel-tempering twin of k_hmc_tc128 (qb_pt.cuh)
+template <int H>
+__global__ void __launch_bounds__(4 * H + 32, H == 64 ? 2 : 1) k_pt_hmc_tc128(const __grid_constant__ QbTg8Plan tp, const __grid_constant__ ChainArgs<float> c,
+                                                                              const __grid_constant__ HmcArgs<float> h, const __grid_constant__ PtArgs a,
+                                                                              const float* __restrict__ absmax) {
+    extern __shared__ __align__(1024) unsigned char smem_g[];
+    const uint32_t tmem = qb_tg8_init<H>(tp, smem_g);
+    QbGradTg8<H> inner{tp, tmem, smem_g, c, absmax, (long long)blockIdx.x};
+    qb_pt_hmc_body<float>(c, h, a, tp.n_params, reinterpret_cast<double*>(smem_g), inner);
+    qb_tc_stop(tmem, (uint32_t)tp.tmem_cols);
+}
+
 template <int H>
 static cudaError_t launch_eval_t(const QbTg8Plan& tp, const EvalArgs<float>& a, const float* absmax, dim3 grid, cudaStream_t st) {
     cudaError_t e = cudaFuncSetAttribute(k_logpost_grad_tc128<H>, cudaFuncAttributeMaxDynamicSharedMemorySize, tp.smem_bytes);
@@ -156,6 +169,15 @@ static cudaError_t launch_nuts_t(const QbTg8Plan& tp, const ChainArgs<float>& c,
     cudaError_t e = cudaFuncSetAttribute(k_nuts_tc128<H>, cudaFuncAttributeMaxDynamicSharedMemorySize, tp.smem_bytes);
     if (e != cudaSuccess) return e;
     k_nuts_tc128<H><<<(unsigned)K, tp.nthreads, tp.smem_bytes, st>>>(tp, c, a, absmax);
+    return cudaGetLastError();
+}
+
+template <int H>
+static cudaError_t launch_pt_t(const QbTg8Plan& tp, const ChainArgs<float>& c, const HmcArgs<float>& h, const PtArgs& a, long long K,
+                               const float* absmax, cudaStream_t st) {
+    cudaError_t e = cudaFuncSetAttribute(k_pt_hmc_tc128<H>, cudaFuncAttributeMaxDynamicSharedMemorySize, tp.smem_bytes);
+    if (e != cudaSuccess) return e;
+    k_pt_hmc_tc128<H><<<(unsigned)K, tp.nthreads, tp.smem_bytes, st>>>(tp, c, h, a, absmax);
     return cudaGetLastError();
 }
 
@@ -195,6 +217,18 @@ cudaError_t qb_tg8_launch_nuts(const QbTg8Plan& tp, const ChainArgs<float>& c, c
     cudaError_t e = tg8_absmax(c.x, c.N * tp.in_dim, c.y, c.N, scratch, st);
     if (e != cudaSuccess) return e;
     return tp.h == 64 ? launch_nuts_t<64>(tp, c, a, K, (const float*)scratch, st) : launch_nuts_t<128>(tp, c, a, K, (const float*)scratch, st);
+}
+
+cudaError_t qb_tg8_pt_absmax(const QbTg8Plan& tp, const ChainArgs<float>& c, cudaStream_t st, const float** absmax) {
+    void* scratch = tg8_stream_scratch(st);
+    if (!scratch) return cudaErrorMemoryAllocation;
+    *absmax = (const float*)scratch;
+    return tg8_absmax(c.x, c.N * tp.in_dim, c.y, c.N, scratch, st);
+}
+
+cudaError_t qb_tg8_launch_pt(const QbTg8Plan& tp, const ChainArgs<float>& c, const HmcArgs<float>& h, const PtArgs& a, long long K,
+                             const float* absmax, cudaStream_t st) {
+    return tp.h == 64 ? launch_pt_t<64>(tp, c, h, a, K, absmax, st) : launch_pt_t<128>(tp, c, h, a, K, absmax, st);
 }
 
 #ifdef QB_TG8_TRACE

@@ -10,6 +10,7 @@
 #include "qb_device.cuh"
 #include "qb_chain.cuh"
 #include "qb_nuts.cuh"
+#include "qb_pt.cuh"
 #include "qb_launch.h"
 #include "qb_value_tc3.h"
 #include "qb_grad_tc.h"
@@ -829,6 +830,26 @@ __global__ void __launch_bounds__(QS_THREADS, 1) k_nuts_stream(const __grid_cons
     qb_nuts_body<T>(c, a, P.n_params, reinterpret_cast<double*>(smem_raw), eval);
 }
 
+// parallel-tempering twins of k_hmc / k_hmc_stream (qb_pt.cuh): same evaluation functors, tempered
+template <typename T>
+__global__ void __launch_bounds__(256, 2) k_pt_hmc(const __grid_constant__ QbPlan plan, const ChainArgs<T> c, const HmcArgs<T> h,
+                                                   const PtArgs a) {
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    const QbSmem S = qb_carve<T>(plan, smem_raw);
+    QbGradSimt<T> inner{plan, S, c, (long long)blockIdx.x};
+    qb_pt_hmc_body<T>(c, h, a, plan.n_params, S.red, inner);
+}
+
+template <typename T>
+__global__ void __launch_bounds__(QS_THREADS, 1) k_pt_hmc_stream(const __grid_constant__ QbStreamPlan P, const ChainArgs<T> c,
+                                                                 const HmcArgs<T> h, const PtArgs a) {
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    QsRing rg;
+    qs_ring_init(P, smem_raw, rg);
+    QbGradStream<T> inner{P, smem_raw, rg, c, (long long)blockIdx.x};
+    qb_pt_hmc_body<T>(c, h, a, P.n_params, reinterpret_cast<double*>(smem_raw), inner);
+}
+
 template <typename T>
 static void fill_chain_args(ChainArgs<T>& c, const qb_data_t* data, const qb_lik_t* lik, const qb_chain_t* ch,
                             const qb_rng_t* rng, const qb_record_t* rec, int64_t t_start, int64_t nsteps, int init_lp) {
@@ -934,6 +955,128 @@ extern "C" int qb_hmc_run(const qb_net_t* net, int dtype, const qb_data_t* data,
     if (check_chain_common(data, lik, chain, rng) || !hm) return g_err[0] ? -1 : qb_fail("NULL hmc state");
     if (dtype == QB_F64) return run_hmc<double>(net, dtype, data, lik, chain, hm, rng, rec, t_start, nsteps, init_lp, (cudaStream_t)stream);
     return run_hmc<float>(net, dtype, data, lik, chain, hm, rng, rec, t_start, nsteps, init_lp, (cudaStream_t)stream);
+}
+
+template <typename T> static int launch_pt_tc128(const QbTg8Plan&, const ChainArgs<T>&, const HmcArgs<T>&, const PtArgs&, long long,
+                                                 const float*, cudaStream_t) { return qb_fail("tensor-core path is fp32 only"); }
+template <> int launch_pt_tc128<float>(const QbTg8Plan& tg, const ChainArgs<float>& c, const HmcArgs<float>& h, const PtArgs& a,
+                                       long long K, const float* absmax, cudaStream_t st) {
+    QB_CUDA(qb_tg8_launch_pt(tg, c, h, a, K, absmax, st));
+    return 0;
+}
+template <typename T> static int pt_absmax(const QbTg8Plan&, const ChainArgs<T>&, cudaStream_t, const float**) {
+    return qb_fail("tensor-core path is fp32 only");
+}
+template <> int pt_absmax<float>(const QbTg8Plan& tg, const ChainArgs<float>& c, cudaStream_t st, const float** absmax) {
+    QB_CUDA(qb_tg8_pt_absmax(tg, c, st, absmax));
+    return 0;
+}
+template <typename T> static int launch_pt_tc(const QbTcgPlan&, const ChainArgs<T>&, const HmcArgs<T>&, const PtArgs&, long long,
+                                              cudaStream_t) { return qb_fail("tensor-core path is fp32 only"); }
+template <> int launch_pt_tc<float>(const QbTcgPlan& tg, const ChainArgs<float>& c, const HmcArgs<float>& h, const PtArgs& a,
+                                    long long K, cudaStream_t st) {
+    QB_CUDA(qb_tcg_launch_pt(tg, c, h, a, K, st));
+    return 0;
+}
+
+// The local ChainArgs of the sub-launch [s, s + n) of a call: its t_start, step count and record positions.  Stored
+// draws keep the slots qb_hmc_run gives the whole call: slot (s + j + 1) / store_every - 1 after call step s + j.
+template <typename T>
+static void pt_sub_args(ChainArgs<T>& cs, const ChainArgs<T>& c, long long s, long long n, int P) {
+    cs = c;
+    cs.t_start = c.t_start + s; cs.nsteps = n; cs.init_lp = c.init_lp && s == 0;
+    if (c.rec_lp) cs.rec_lp = c.rec_lp + s;
+    if (c.rec_alpha) cs.rec_alpha = c.rec_alpha + s;
+    if (c.rec_acc) cs.rec_acc = c.rec_acc + s;
+    cs.samples = nullptr;
+    const long long se = c.store_every;
+    if (!c.samples || se <= 0) return;
+    long long slot0, every;
+    if (s % se == 0) { slot0 = s / se; every = se; }                  // stores at local steps j with (j + 1) % se == 0
+    else if ((s + n) % se == 0) { slot0 = (s + n) / se - 1; every = n; }   // one store, after the last step
+    else return;
+    if (slot0 >= c.n_slots) return;
+    cs.samples = c.samples + slot0 * P;          // row k stays at k * n_slots (the kernel's stride)
+    cs.store_every = every;
+}
+
+template <typename T>
+static int run_pt(const qb_net_t* net, int dtype, const qb_data_t* data, const qb_lik_t* lik, qb_chain_t* ch, qb_hmc_t* hm,
+                  const qb_rng_t* rng, const qb_record_t* rec, int64_t t_start, int64_t nsteps, int init_lp, int64_t G,
+                  const double* beta, const double* eps, int64_t swap_every, int32_t* replica, int8_t* last_end,
+                  int64_t* round_trips, int64_t* attempts, int64_t* accepts, cudaStream_t st) {
+    QbLaunch L;
+    if (plan_eval(net, dtype, true, ch->K, data->n, true, &L)) return -1;
+    if (!hm->grad_cur || !hm->mom || !hm->prop || !hm->grad_prop) return qb_fail("hmc state has NULL arrays");
+    if (hm->method == 0 && hm->L < 1) return qb_fail("HMC needs L >= 1");
+    const int P = net->n_params;
+    const long long K = ch->K, nT = K / G;
+    ChainArgs<T> c; fill_chain_args<T>(c, data, lik, ch, rng, rec, t_start, nsteps, init_lp);
+    HmcArgs<T> h;
+    h.method = hm->method; h.L = hm->L; h.eps = hm->epsilon;
+    h.gcur = (T*)hm->grad_cur; h.mom = (T*)hm->mom; h.prop = (T*)hm->prop; h.gprop = (T*)hm->grad_prop;
+    const PtArgs a{beta, eps, (long long)G};
+    PtSwapArgs sw{beta, (long long)G, (int)nT, rng->seed, rng->chain_offset, 0, ch->lp, replica, (signed char*)last_end,
+                  (long long*)round_trips, (long long*)attempts, (long long*)accepts};
+    const float* absmax = nullptr;
+    if (L.path == QB_PATH_TG8 && pt_absmax<T>(L.t8, c, st, &absmax)) return -2;      // once per call, not per launch
+    if (L.path == QB_PATH_STREAM && set_smem(k_pt_hmc_stream<T>, L.sp.smem_bytes)) return -2;
+    const bool simt = L.path != QB_PATH_STREAM && L.path != QB_PATH_TG8 && L.path != QB_PATH_TCG;
+    if (simt && set_smem(k_pt_hmc<T>, L.plan.smem_bytes)) return -2;
+    // sub-launches end at swap boundaries and, so that no store passes the last slot, at n_slots * store_every
+    const long long cut = (c.samples && c.store_every > 0) ? c.n_slots * c.store_every : -1;
+    for (long long s = 0; s < nsteps;) {
+        const long long t = t_start + s;
+        long long n = std::min<long long>(swap_every - t % swap_every, nsteps - s);
+        if (s < cut) n = std::min(n, cut - s);
+        ChainArgs<T> cs; pt_sub_args<T>(cs, c, s, n, P);
+        if (L.path == QB_PATH_STREAM) {
+            k_pt_hmc_stream<T><<<(unsigned)K, QS_THREADS, L.sp.smem_bytes, st>>>(L.sp, cs, h, a);
+        } else if (L.path == QB_PATH_TG8) {
+            if (launch_pt_tc128<T>(L.t8, cs, h, a, K, absmax, st)) return -2;
+        } else if (L.path == QB_PATH_TCG) {
+            if (launch_pt_tc<T>(L.tg, cs, h, a, K, st)) return -2;
+        } else {
+            k_pt_hmc<T><<<(unsigned)K, L.plan.nthreads, L.plan.smem_bytes, st>>>(L.plan, cs, h, a);
+        }
+        QB_CUDA(cudaGetLastError());
+        g_launches += 1;
+        s += n;
+        if ((t_start + s) % swap_every == 0 && nT > 1) {
+            sw.r = (t_start + s) / swap_every - 1;
+            const int npairs = (int)(nT / 2);
+            k_pt_swap<T><<<(unsigned)G, 256, std::max(npairs, 1) * (int)sizeof(int), st>>>(sw, (T*)ch->theta, h.gcur, P);
+            QB_CUDA(cudaGetLastError());
+            g_launches += 1;
+        }
+    }
+    if (L.path == QB_PATH_TG8) g_launches += 1;
+    return 0;
+}
+
+extern "C" int qb_pt_run(const qb_net_t* net, int dtype, const qb_data_t* data, const qb_lik_t* lik, qb_chain_t* chain,
+                         qb_hmc_t* hm, const qb_rng_t* rng, const qb_record_t* rec, int64_t t_start, int64_t nsteps,
+                         int init_lp, int64_t n_groups, const double* beta, const double* eps, int64_t swap_every,
+                         int32_t* replica, int8_t* last_end, int64_t* round_trips, int64_t* swap_attempts,
+                         int64_t* swap_accepts, void* stream) {
+    if (!net || !data || !lik || !chain || !rng || !hm) return qb_fail("NULL argument to chain run");
+    if (rng->mode == QB_RNG_REPLAY) return qb_fail("parallel tempering has no replay mode: its draws come from Philox");
+    if (!beta || !eps || !replica || !last_end || !round_trips || !swap_attempts || !swap_accepts)
+        return qb_fail("parallel-tempering state has NULL arrays");
+    if (n_groups < 1) return qb_fail("parallel tempering needs n_groups >= 1");
+    if (chain->K % n_groups != 0) return qb_fail("K must be a multiple of n_groups%s (K=%lld)", "", chain->K);
+    if (swap_every < 1) return qb_fail("parallel tempering needs swap_every >= 1");
+    if (nsteps < 0 || t_start < 0) return qb_fail("nsteps and t_start must be >= 0");
+    if (t_start % swap_every != 0) return qb_fail("t_start must be a multiple of swap_every%s (t_start=%lld)", "", t_start);
+    if (rec && rec->samples && rec->store_every > 0 && rec->store_every % swap_every != 0 && swap_every % rec->store_every != 0)
+        return qb_fail("store_every and swap_every must divide one another%s (store_every=%lld)", "", rec->store_every);
+    if (chain->K == 0 || nsteps == 0) return 0;
+    if (check_chain_common(data, lik, chain, rng)) return -1;
+    if (dtype == QB_F64)
+        return run_pt<double>(net, dtype, data, lik, chain, hm, rng, rec, t_start, nsteps, init_lp, n_groups, beta, eps,
+                              swap_every, replica, last_end, round_trips, swap_attempts, swap_accepts, (cudaStream_t)stream);
+    return run_pt<float>(net, dtype, data, lik, chain, hm, rng, rec, t_start, nsteps, init_lp, n_groups, beta, eps, swap_every,
+                         replica, last_end, round_trips, swap_attempts, swap_accepts, (cudaStream_t)stream);
 }
 
 template <typename T>

@@ -358,7 +358,8 @@ def _rng_struct(seed, chain_offset, incr, unif):
 class Recorder:
     """Per-step records of one run segment (qb_record_t)."""
 
-    def __init__(self, state: ChainState, nsteps, store_every=1, record_scalars=True):
+    def __init__(self, state: ChainState, nsteps, store_every=1, record_scalars=True, sample_rows=None):
+        """``sample_rows``: rows of ``samples`` (default K; parallel tempering stores the cold rows only)."""
         dev, K, P = state.prob.device, state.K, state.P
         self.nsteps = nsteps
         self.store_every = int(store_every)
@@ -366,7 +367,8 @@ class Recorder:
         self.logpost = torch.empty((K, nsteps), dtype=torch.float64, device=dev) if record_scalars else None
         self.alpha = torch.empty((K, nsteps), dtype=torch.float64, device=dev) if record_scalars else None
         self.accepted = torch.empty((K, nsteps), dtype=torch.uint8, device=dev) if record_scalars else None
-        self.samples = (torch.empty((K, self.n_slots, P), dtype=state.prob.dtype, device=dev)
+        rows = K if sample_rows is None else int(sample_rows)
+        self.samples = (torch.empty((rows, self.n_slots, P), dtype=state.prob.dtype, device=dev)
                         if self.n_slots > 0 else None)
         self.logpost0 = torch.empty(K, dtype=torch.float64, device=dev)     # filled by the first segment of a run
 
@@ -553,6 +555,117 @@ def nuts_run(state: ChainState, ns: NutsState, nsteps, rec: Recorder = None, nre
     _lib.check(rc, 'qb_nuts_run')
     state.t += nsteps
     state.initialised = True
+
+
+def pt_ladder(n_temps, beta_min):
+    """Geometric inverse temperatures 1 = beta_0 > ... > beta_{T-1} = beta_min (T = n_temps)."""
+    T = int(n_temps)
+    if T < 1:
+        raise ValueError('n_temps must be >= 1')
+    if T == 1:
+        return np.ones(1)
+    if not 0.0 < float(beta_min) < 1.0:
+        raise ValueError('beta_min must lie in (0, 1)')
+    b = float(beta_min) ** (np.arange(T) / (T - 1.0))
+    b[0] = 1.0
+    return b
+
+
+def pt_check_ladder(betas, epsilon):
+    """Validated float64 (betas [T], step sizes [T]): beta_0 == 1, strictly decreasing, all > 0; epsilon a scalar (slot i
+    uses epsilon * beta_i^-1/2) or [T], finite and > 0."""
+    b = np.asarray(betas, dtype=np.float64).reshape(-1)
+    if b.size < 1 or b[0] != 1.0:
+        raise ValueError('the ladder must start at beta_0 == 1.0')
+    if not np.all(np.isfinite(b)) or np.any(b <= 0.0):
+        raise ValueError('every beta must be finite and > 0')
+    if np.any(np.diff(b) >= 0.0):
+        raise ValueError('the betas must be strictly decreasing')
+    e = np.asarray(epsilon, dtype=np.float64).reshape(-1)
+    if e.size == 1:
+        e = e[0] / np.sqrt(b)
+    if e.size != b.size:
+        raise ValueError(f'epsilon must be a scalar or one step size per temperature ({b.size})')
+    if not np.all(np.isfinite(e)) or np.any(e <= 0.0):
+        raise ValueError('every step size must be finite and > 0')
+    return b, e
+
+
+class PtState:
+    """Parallel-tempering state of K = T * n_groups chains (qb_pt_run): the HMC / MALA arrays, the ladder beta [T] and
+    step sizes eps [T] on the device, which replica sits in each slot, the last ladder end each replica visited, round
+    trips per group and swap counters per group and pair."""
+
+    _FIELDS = ('replica', 'last_end', 'round_trips', 'swap_attempts', 'swap_accepts')
+
+    def __init__(self, state: ChainState, n_groups, betas, epsilon=0.05, L=3, method='hmc', swap_every=1):
+        if method not in ('hmc', 'mala'):
+            raise ValueError("method must be 'hmc' or 'mala'")
+        b, e = pt_check_ladder(betas, epsilon)
+        G, T = int(n_groups), b.size
+        if G < 1 or state.K != T * G:
+            raise ValueError(f'K = {state.K} chains must be n_temps ({T}) x n_groups ({n_groups})')
+        if int(swap_every) < 1:
+            raise ValueError('swap_every must be >= 1')
+        if method == 'hmc' and int(L) < 1:
+            raise ValueError('HMC needs L >= 1')
+        dev = state.prob.device
+        self.n_groups, self.n_temps, self.swap_every = G, T, int(swap_every)
+        self.betas, self.step_sizes = b, e
+        self.hmc = HmcState(state, epsilon=float(e[0]), L=L, method=method)
+        self.beta = torch.as_tensor(b, dtype=torch.float64).to(dev)
+        self.eps = torch.as_tensor(e, dtype=torch.float64).to(dev)
+        self.replica = torch.arange(state.K, dtype=torch.int32, device=dev)
+        le = torch.zeros(state.K, dtype=torch.int8)
+        le[:G] = 1
+        if T > 1:
+            le[(T - 1) * G:] = -1
+        self.last_end = le.to(dev)
+        self.round_trips = torch.zeros(G, dtype=torch.int64, device=dev)
+        # [G, T-1] views of a buffer that is never empty, so that qb_pt_run gets non-NULL counters also for T == 1
+        self._swap_buf = torch.zeros((2, G * max(T - 1, 1)), dtype=torch.int64, device=dev)
+        self.swap_attempts = self._swap_buf[0, :G * (T - 1)].view(G, T - 1)
+        self.swap_accepts = self._swap_buf[1, :G * (T - 1)].view(G, T - 1)
+
+    @property
+    def grad_cur(self):
+        return self.hmc.grad_cur
+
+    def state_dict(self):
+        d = {k: getattr(self, k).detach().cpu().clone() for k in self._FIELDS}
+        d.update(self.hmc.state_dict())
+        return d
+
+    def load_state_dict(self, d):
+        for k in self._FIELDS:
+            getattr(self, k).copy_(d[k])
+        self.hmc.load_state_dict(d)
+
+    def swap_rate(self):
+        """[n_groups, T-1] accepted / attempted swaps of each pair (0 where none was attempted)."""
+        return self.swap_accepts.double() / self.swap_attempts.clamp(min=1).double()
+
+
+def pt_run(state: ChainState, ps: PtState, nsteps, rec: Recorder = None, seed=0, chain_offset=0):
+    """qb_pt_run: advance all K = T * n_groups chains by nsteps tempered HMC / MALA steps with a DEO swap round after
+    every absolute step t with (t + 1) % swap_every == 0 (Philox draws; there is no replay mode).  rec.samples, if any,
+    must have n_groups rows (Recorder(..., sample_rows=n_groups)): draws are stored for the cold chains only."""
+    if rec is not None and rec.samples is not None and rec.samples.shape[0] != ps.n_groups:
+        raise ValueError('parallel tempering stores the cold chains only: use Recorder(..., sample_rows=n_groups)')
+    prob = state.prob
+    rng = _rng_struct(seed, chain_offset, None, None)
+    cch, chm = state.c(), ps.hmc.c()
+    crec = rec.c() if rec is not None else None
+    with torch.cuda.device(prob.device):
+        rc = _lib.load().qb_pt_run(C.byref(prob.cnet), prob.qdt, C.byref(prob.cdata), C.byref(prob.clik), C.byref(cch),
+                                   C.byref(chm), C.byref(rng), C.byref(crec) if crec is not None else None, state.t, nsteps,
+                                   0 if state.initialised else 1, ps.n_groups, _ptr(ps.beta), _ptr(ps.eps), ps.swap_every,
+                                   _ptr(ps.replica), _ptr(ps.last_end), _ptr(ps.round_trips), _ptr(ps._swap_buf[0]),
+                                   _ptr(ps._swap_buf[1]), _stream())
+    _lib.check(rc, 'qb_pt_run')
+    if nsteps > 0:
+        state.t += nsteps
+        state.initialised = True
 
 
 def vi_sample(mu, rho, nsam, pi, sigma1, sigma2, eps=None, seed=0, step=0):

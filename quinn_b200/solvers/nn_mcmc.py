@@ -13,6 +13,7 @@ from ..mcmc.admcmc import AMCMC
 from ..mcmc.hmc import HMC
 from ..mcmc.mala import MALA
 from ..mcmc.nuts import NUTS
+from ..mcmc.pt import PT
 from ..mcmc.mcmc import DeviceLogPost
 from ..netdesc import netdesc_from_module
 from ..nns.nnwrap import NNWrap, nn_p
@@ -78,6 +79,11 @@ class NN_MCMC(QUiNNBase):
         target_accept) in this process; its result dict adds ``tree_depth``, ``n_leapfrog``, ``diverging`` and
         ``step_size`` per transition.
 
+        ``sampler='pt'`` runs parallel tempering on HMC or MALA (quinn_b200.mcmc.PT, sampler_params: base, epsilon, L,
+        betas, n_temps, beta_min, swap_every) in this process.  ``nchains`` / the rows of ``param_ini`` count groups: each
+        runs T tempered chains, and the result dict (and so predict_* and diagnose()) holds the cold ones; it adds
+        ``betas``, ``step_sizes``, ``swap_rate`` and ``round_trips``.
+
         Extensions (keyword-only): ``nchains`` / a (K,P) ``param_ini`` run K chains at once (``samples``
         becomes (K, M+1, P)); ``seed``, ``store_every``, ``replay``, ``chain_offset`` are passed to the sampler.
         With ``zflag`` the start point is refined by BFGS on -logpost using the analytic gradient of kernel 2
@@ -94,6 +100,9 @@ class NN_MCMC(QUiNNBase):
         (and gradient) is the all-reduced sum of the per-rank partial sums (the N-sharded mode for data that exceed one
         GPU; propose / accept run redundantly and identically on every rank)."""
         assert xtrn.shape[0] == ytrn.shape[0]
+        if sampler == 'pt' and (data_sharded or distributed or replay is not None):
+            raise ValueError("sampler='pt' runs in a single process from Philox draws: distributed=True, "
+                             "data_sharded=True and replay are not supported with it")
         if sampler == 'nuts' and (data_sharded or distributed):
             raise ValueError("sampler='nuts' runs in a single process: distributed=True and data_sharded=True are not "
                              "supported with it")
@@ -123,8 +132,11 @@ class NN_MCMC(QUiNNBase):
         elif sampler == 'nuts':
             mymcmc = NUTS(**sampler_params)
             mymcmc.setLogPost(self.logpost, self.logpostgrad, lpinfo=self.lpinfo)
+        elif sampler == 'pt':
+            mymcmc = PT(**sampler_params)
+            mymcmc.setLogPost(self.logpost, self.logpostgrad, lpinfo=self.lpinfo)
         else:
-            raise ValueError(f"sampler {sampler!r} is not one of 'amcmc', 'hmc', 'mala', 'nuts'")
+            raise ValueError(f"sampler {sampler!r} is not one of 'amcmc', 'hmc', 'mala', 'nuts', 'pt'")
         res = mymcmc.run(param_ini=param_ini, nmcmc=nmcmc, seed=seed, store_every=store_every, replay=replay,
                          chain_offset=chain_offset, verbose=self.verbose, keep_on_device=keep_on_device)
         self.sampler_obj, self.mcmc_results = mymcmc, res
